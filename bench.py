@@ -1,8 +1,12 @@
 #!/usr/bin/env python
 """Benchmark of the self-play hot path: MCTS simulations/sec, network evaluation included.
 
-    python bench.py --gpus N --steps K --warmup W [--workload tictactoe|cartpole|gomoku|atari]
+    python bench.py --gpus N --steps K --warmup W [--workload tictactoe|cartpole|gomoku|atari] [--dump-outputs DIR]
     python bench.py --impl reference ...        # the CPU arm (oracle port of the reference path)
+
+--dump-outputs DIR writes what the last timed search returned (action, pi, root_value of rank 0's trees) and the
+last timed training step's loss / priorities as DIR/<name>.npy (float64), so that two builds run with the same
+arguments, hence the same inputs, weights and RNG seeds, can be compared output for output.
 
 A "step" is ONE batched search: B trees x S simulations, from observations to
 (action, pi, root value): initial inference, Dirichlet noise, S x (select, recurrent
@@ -403,6 +407,9 @@ def measure_workload(spec, args, dev, world, rank, steps, warmup, min_seconds=0.
     uuid = str(torch.cuda.get_device_properties(dev).uuid)
     sampler = ClockSampler(uuid if uuid.startswith('GPU-') else 'GPU-' + uuid) if rank == 0 else None
     ms_dev = timed(step_device, steps)
+    # what the last timed search returned, read before the e2e steps below overwrite the plan's output buffers
+    built['outputs'] = {'action': plan.action.cpu().numpy(), 'pi': plan.pi.cpu().numpy(),
+                        'root_value': plan.root_value.cpu().numpy()}
     stats1 = read_stats()
     ms_e2e = timed(step_e2e, steps)
     clocks = sampler.stop() if rank == 0 else None
@@ -628,11 +635,14 @@ def run_engine_arm(args):
     result, built = measure_workload(spec, args, dev, world, rank, args.steps, args.warmup, parts=args.parts,
                                      cta_limit=args.cta_limit)
     net = built['net']
+    outputs = dict(built['outputs'])
     if not args.no_train_step:
         try:
-            result['train_step'] = train_step_sample(net, spec, dev, world)
+            result['train_step'] = train_step_sample(net, spec, dev, world, outputs=outputs)
         except Exception as exc:                      # never lose the search line to the secondary measurement
             result['train_step'] = {'error': repr(exc)[:200]}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outputs)
     if spec['name'] in ('gomoku', 'tictactoe') and not args.no_self_play:
         try:
             result['self_play'] = self_play_sample(net, spec, dev, rank)
@@ -673,10 +683,11 @@ def run_engine_arm(args):
         dist.destroy_process_group()
 
 
-def train_step_sample(net, spec, dev, world, batch=128, unroll=5, warmup=6, steps=20):
+def train_step_sample(net, spec, dev, world, batch=128, unroll=5, warmup=6, steps=20, outputs=None):
     """BASELINE.json config 5's second half: the K=5-unroll training step, data-parallel, one flat
     NCCL all-reduce of the gradients; the towers' forward / dgrad / wgrad and train-mode BatchNorm run on the
-    hand-written tcgen05 kernels of csrc/train.cu (SURVEY.md section 8 e / f-2)."""
+    hand-written tcgen05 kernels of csrc/train.cu (SURVEY.md section 8 e / f-2).  The last timed step's loss and
+    priorities go into `outputs` when it is given."""
     import copy
     import torch
     import torch.distributed as dist
@@ -735,6 +746,8 @@ def train_step_sample(net, spec, dev, world, batch=128, unroll=5, warmup=6, step
         replay.update_priorities(idx, prio)
     e1.record()
     torch.cuda.synchronize(dev)
+    if outputs is not None:
+        outputs['train_loss'], outputs['train_priorities'] = np.array([loss]), prio
     sample_ms = s0.elapsed_time(s1)
     dp_only_ms = None
     if world > 1:                        # the data-parallel learner step on its own (fixed batch, no replay calls)
@@ -920,6 +933,27 @@ def cpu_baseline_sample(args, spec):
                       f'(oracle port of uct_search + fp32 torch network, 1 thread per process)'}
 
 
+DUMP_LIMIT_BYTES = 60 << 20         # under 64 MB in all, .npy headers included
+
+
+def dump_outputs(dirname: str, outputs: dict, limit: int = DUMP_LIMIT_BYTES) -> None:
+    """`outputs` as float64 arrays DIR/<name>.npy.  Past `limit` bytes in all, the per-tree arrays keep a fixed sample of
+    trees (seed 0; the tree indices go to DIR/sampled_trees.npy) so that the files stay small enough to keep and diff."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in outputs.items()}
+    per_tree = ('action', 'pi', 'root_value')
+    B = len(arrays['action'])
+    total = sum(a.nbytes for a in arrays.values())
+    if total > limit:
+        tree_bytes = sum(arrays[k].nbytes for k in per_tree)
+        keep = max(1, int(B * (limit - (total - tree_bytes) - 8 * B) / tree_bytes))
+        rows = np.sort(np.random.RandomState(0).choice(B, size=keep, replace=False))
+        arrays = {k: (a[rows] if k in per_tree else a) for k, a in arrays.items()}
+        arrays['sampled_trees'] = rows.astype(np.float64)
+    os.makedirs(dirname, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(dirname, f'{k}.npy'), a)
+
+
 _REAL_STDOUT = None
 
 
@@ -941,7 +975,7 @@ def main():
     os.dup2(2, 1)
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=10)
+    ap.add_argument('--steps', type=int, default=10, help='timed steps (searches) of the workload')
     ap.add_argument('--warmup', type=int, default=3)
     ap.add_argument('--workload', default=os.environ.get('MZ_BENCH_WORKLOAD', 'gomoku'))
     ap.add_argument('--trees', type=int, default=None, help='trees per GPU (default: the config size)')
@@ -955,7 +989,13 @@ def main():
     ap.add_argument('--no-configs', action='store_true', help='skip the sub-runs of the other configurations')
     ap.add_argument('--strong', action='store_true',
                     help="strong scaling: the configuration's trees in total, split over the ranks")
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help="write the last timed step's outputs to DIR/<name>.npy (engine arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs applies to the engine arm')
     if args.impl == 'reference':
         run_reference_arm(args)
     else:
