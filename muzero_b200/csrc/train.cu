@@ -18,8 +18,9 @@
 // K = consecutive 16-byte rows), so both operands are again plain 1-D bulk copies and a tap is a shifted start address.
 // Every plane has `front` zero rows before row 0 and a zero tail, so that no tile needs a special case.
 //
-// Precision: activations and weights fp16 (like the inference engine; MZ_TRAIN_FWD_BF16=1: bf16), gradients bf16
-// (fp32 range, no loss scaling), fp32 accumulation in TMEM, fp32 BatchNorm statistics and parameter gradients.
+// Precision: activations and weights fp16 (like the inference engine; with bf16 the towers are 7e-3 instead of 8e-4 from
+// fp32 at the same step time, DESIGN.md 4), gradients bf16 (fp32 range, no loss scaling), fp32 accumulation in TMEM,
+// fp32 BatchNorm statistics and parameter gradients.
 // kind::f16 MMAs take fp16 x fp16 or bf16 x bf16 but not a mix (an fp16 x bf16 descriptor raises an illegal-instruction
 // fault), so every activation a weight gradient needs is ALSO kept as a bf16 copy, written by the kernel that produces
 // it: the forward chain keeps fp16's three extra mantissa bits, dW = dY^T A runs bf16 x bf16.
@@ -28,6 +29,7 @@
 #include <cuda_fp16.h>
 #include <cuda_bf16.h>
 #include <cstdlib>
+#include <type_traits>
 #include <vector>
 
 namespace mz {
@@ -47,14 +49,16 @@ constexpr int kTimelineMax = 8192;
 constexpr int kDyRing = 6;         // dY buffers in flight between the dgrad / BatchNorm chain and the weight-gradient streams
 constexpr int kSideStreams = 3;    // weight-gradient launches alternate between these: consecutive ones may overlap
 
-// ---- 16-bit element helpers (runtime element type: 0 = fp16, 1 = bf16) -------------------------------------------
-__device__ __forceinline__ float2 unpack2(uint32_t v, int bf16) {
-  if (bf16) return __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&v));
-  return __half22float2(*reinterpret_cast<const __half2*>(&v));
+// ---- 16-bit element helpers: T = __half (forward tensors) or __nv_bfloat16 (gradients, wgrad operand copies) -------
+template <typename T>
+__device__ __forceinline__ float2 unpack2(uint32_t v) {
+  if constexpr (std::is_same_v<T, __nv_bfloat16>) return __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&v));
+  else return __half22float2(*reinterpret_cast<const __half2*>(&v));
 }
-__device__ __forceinline__ uint32_t pack2(float a, float b, int bf16) {
+template <typename T>
+__device__ __forceinline__ uint32_t pack2(float a, float b) {
   uint32_t d;
-  if (bf16) {
+  if constexpr (std::is_same_v<T, __nv_bfloat16>) {
     __nv_bfloat162 t = __floats2bfloat162_rn(a, b);
     d = *reinterpret_cast<uint32_t*>(&t);
   } else {
@@ -62,17 +66,18 @@ __device__ __forceinline__ uint32_t pack2(float a, float b, int bf16) {
   }
   return d;
 }
-__device__ __forceinline__ void unpack8(const int4& r, int bf16, float (&v)[8]) {
+template <typename T>
+__device__ __forceinline__ void unpack8(const int4& r, float (&v)[8]) {
   const uint32_t w[4] = {(uint32_t)r.x, (uint32_t)r.y, (uint32_t)r.z, (uint32_t)r.w};
 #pragma unroll
   for (int u = 0; u < 4; ++u) {
-    const float2 f = unpack2(w[u], bf16);
+    const float2 f = unpack2<T>(w[u]);
     v[2 * u] = f.x; v[2 * u + 1] = f.y;
   }
 }
-__device__ __forceinline__ int4 pack8(const float* v, int bf16) {
-  return make_int4((int)pack2(v[0], v[1], bf16), (int)pack2(v[2], v[3], bf16), (int)pack2(v[4], v[5], bf16),
-                   (int)pack2(v[6], v[7], bf16));
+template <typename T>
+__device__ __forceinline__ int4 pack8(const float* v) {
+  return make_int4((int)pack2<T>(v[0], v[1]), (int)pack2<T>(v[2], v[3]), (int)pack2<T>(v[4], v[5]), (int)pack2<T>(v[6], v[7]));
 }
 
 // kind::f16 instruction descriptor with explicit operand formats (0 = fp16, 1 = bf16) and majors (1 = MN-major)
@@ -152,10 +157,9 @@ struct TConvParams {
   // dZ = G * (A > 0) right here (that is all its consumers read) and the layer's BatchNorm-backward sums
   // (sum dZ, sum dZ * xhat) are taken from the fp32 values -- no separate reduction pass over the tensor
   const uint8_t* mask_bits; // the layer's ReLU mask [16][R128]: bit e of byte (g, row) = (A[row][8 g + e] > 0), or nullptr
-  const uint16_t* mask_y;   // its raw conv output Y (forward type)
+  const uint16_t* mask_y;   // its raw conv output Y (fp16)
   const float* mask_saved;  // its [128][2] (mean, invstd)
   long long* mask_sums;     // its [128][2] += fixed-point (sum dZ, sum dZ * xhat)
-  int fbf16;                // forward tensors are bf16
   int cg_in, stage_g, chunks;   // a weight stage = stage_g channel groups of one tap; chunks stages per tap
   int Ptot, PB, Wp, W, H, PR, R128;
   int TP, TPs;              // rows of a tile incl. halo / rows of a shared-memory plane (odd)
@@ -163,8 +167,7 @@ struct TConvParams {
                             // (floats) between consecutive calls' statistics records -- a tile belongs to call row0 / sub_rows
   int stages, nbuf;
   uint32_t idesc;
-  int out_bf16;
-  int ablate;               // measurement only (MZ_TRAIN_ABLATE): 1 no MMAs, 2 no epilogue loads / stores, 4 no column sums, 8 no weight copies
+  int dgrad;                // dgrad: bf16 operands and output; forward: fp16
   unsigned long long* tl;   // measurement only: timeline record or nullptr
 };
 
@@ -235,11 +238,8 @@ __global__ void __launch_bounds__(kTConvThreads) tconv_kernel(const __grid_const
     auto next_stage = [&](int it) {
       if (lane == 0) {
         if (wrapped) mbar_wait(&w_empty[s], ph);
-        if (p.ablate & 8) mbar_arrive(&w_full[s]);
-        else {
-          mbar_arrive_expect_tx(&w_full[s], stage_bytes);
-          bulk_g2s(sW + (size_t)s * stage_bytes, wsrc + (size_t)it * stage_bytes, stage_bytes, &w_full[s]);
-        }
+        mbar_arrive_expect_tx(&w_full[s], stage_bytes);
+        bulk_g2s(sW + (size_t)s * stage_bytes, wsrc + (size_t)it * stage_bytes, stage_bytes, &w_full[s]);
       }
       if (++s == p.stages) { s = 0; if (wrapped) ph ^= 1u; wrapped = true; }
     };
@@ -289,7 +289,7 @@ __global__ void __launch_bounds__(kTConvThreads) tconv_kernel(const __grid_const
       tc_fence_after();
       if (i == 0) tl_stamp_lane0(p.tl, 4);
       const uint32_t tm = tm0 + (uint32_t)buf * 128u, a_base = a_base0 + (uint32_t)buf * a_buf_units;
-      if (kChunks > 0 && !(p.ablate & 1)) {
+      if constexpr (kChunks > 0) {
         // 128-channel stages: eight K steps under two elections; kChunks stages per tap
         uint32_t a_tap = a_base - wp - 1u;      // tap (0, 0)
 #pragma unroll
@@ -312,7 +312,7 @@ __global__ void __launch_bounds__(kTConvThreads) tconv_kernel(const __grid_const
           a_tap += (tap % 3 == 2) ? wp - 2u : 1u;
         }
       } else {
-        // any other stage shape (the representation tower's first convolution), or the MMAs ablated
+        // any other stage shape (the representation tower's first convolution)
         const int ksteps = p.stage_g / 2;
         uint32_t acc = 0;
         uint32_t a_tap = a_base - wp - 1u;
@@ -321,11 +321,9 @@ __global__ void __launch_bounds__(kTConvThreads) tconv_kernel(const __grid_const
           for (int ch = 0; ch < p.chunks; ++ch) {
             mbar_wait(&w_full[s], ph);
             tc_fence_after();
-            if (!(p.ablate & 1)) {
-              for (int ks = 0; ks < ksteps; ++ks) {
-                mma_f16_elect(tm, d64(a_lo + (uint32_t)ks * a_step, a_hi), d64(b_lo + (uint32_t)ks * b_step, b_hi), idesc, acc);
-                acc = 1;
-              }
+            for (int ks = 0; ks < ksteps; ++ks) {
+              mma_f16_elect(tm, d64(a_lo + (uint32_t)ks * a_step, a_hi), d64(b_lo + (uint32_t)ks * b_step, b_hi), idesc, acc);
+              acc = 1;
             }
             commit_elect(&w_empty[s]);
             a_lo += a_chunk;
@@ -366,10 +364,10 @@ __global__ void __launch_bounds__(kTConvThreads) tconv_kernel(const __grid_const
       // this thread's row and 64 columns -- is requested NOW, while the MMAs run: no global round trip sits between the
       // last MMA and the stores.  Loads are UNCONDITIONAL per lane (every row of a plane up to its zero tail is readable;
       // halo rows are discarded by `valid` below): a predicate would turn each load into load + select.
-      const bool do_mask = mask && !(p.ablate & 2), do_add = p.add != nullptr && !(p.ablate & 2);
+      const bool do_add = p.add != nullptr;
       int4 py[8], pd[8];
       uint2 bits = make_uint2(0xffffffffu, 0xffffffffu);
-      if (do_mask) {
+      if (mask) {
         uint32_t bq[8];
 #pragma unroll
         for (int u = 0; u < 8; ++u) bq[u] = __ldcg(p.mask_bits + (size_t)(half * 8 + u) * p.R128 + P);
@@ -401,7 +399,7 @@ __global__ void __launch_bounds__(kTConvThreads) tconv_kernel(const __grid_const
 #pragma unroll
           for (int u = 0; u < 4; ++u) {
             float f[8];
-            unpack8(pd[c * 4 + u], 1, f);
+            unpack8<__nv_bfloat16>(pd[c * 4 + u], f);
 #pragma unroll
             for (int e = 0; e < 8; ++e) v[8 * u + e] = valid ? v[8 * u + e] + f[e] : 0.0f;
           }
@@ -413,11 +411,7 @@ __global__ void __launch_bounds__(kTConvThreads) tconv_kernel(const __grid_const
 #pragma unroll
           for (int u = 0; u < 4; ++u) {
             float y8[8];
-            if (do_mask) unpack8(py[c * 4 + u], p.fbf16, y8);
-            else {
-#pragma unroll
-              for (int e = 0; e < 8; ++e) y8[e] = 0.0f;
-            }
+            unpack8<__half>(py[c * 4 + u], y8);
 #pragma unroll
             for (int e = 0; e < 8; ++e) {
               const int col = half * 64 + c * 32 + 8 * u + e;
@@ -427,14 +421,15 @@ __global__ void __launch_bounds__(kTConvThreads) tconv_kernel(const __grid_const
             }
           }
         }
-        if (inr && !(p.ablate & 2)) {
+        if (inr) {
+          int4 o[4];                           // packed before the stores: one store sequence for either type, fewer spills
 #pragma unroll
-          for (int u = 0; u < 4; ++u)
-            reinterpret_cast<int4*>(p.out)[(size_t)(half * 8 + c * 4 + u) * p.PR + rowoff] = pack8(v + 8 * u, p.out_bf16);
+          for (int u = 0; u < 4; ++u) o[u] = p.dgrad ? pack8<__nv_bfloat16>(v + 8 * u) : pack8<__half>(v + 8 * u);
+#pragma unroll
+          for (int u = 0; u < 4; ++u) reinterpret_cast<int4*>(p.out)[(size_t)(half * 8 + c * 4 + u) * p.PR + rowoff] = o[u];
         }
         const int col0 = half * 64 + c * 32;
-        if (p.ablate & 4) {
-        } else if (mask) {
+        if (mask) {
           const float s1 = warp_colsum32(v, lane);
           const float s2 = warp_colsum32(zx, lane);
           st_buf[quad * 2 * kC + col0 + lane] = s1;
@@ -456,11 +451,9 @@ __global__ void __launch_bounds__(kTConvThreads) tconv_kernel(const __grid_const
         asm volatile("bar.sync 1, 256;" ::: "memory");
         const int which = et >> 7, col = et & (kC - 1);
         float a = 0.0f;
-        if (!(p.ablate & 4)) {
 #pragma unroll
-          for (int q = 0; q < 4; ++q) a += st_buf[q * 2 * kC + which * kC + col];
-        }
-        if (!(p.ablate & 32)) fix_add(sums + 2 * col + which, a, mask ? kFixGrad : (which ? kFixActSq : kFixAct));
+        for (int q = 0; q < 4; ++q) a += st_buf[q * 2 * kC + which * kC + col];
+        fix_add(sums + 2 * col + which, a, mask ? kFixGrad : (which ? kFixActSq : kFixAct));
       }
     }
   }
@@ -483,7 +476,6 @@ struct TWgradParams {
   int slices, slice0;       // slices of the tensor (calls x kSplits) / first slice of this call: every launch owns its slices,
                             // nothing is read back (a read-modify-write of 9.4 MB per launch cost more than the MMAs)
   uint32_t idesc;
-  int swap_strides;         // debug: exchange LBO / SBO of the MN-major descriptors
   unsigned long long* tl;   // measurement only
 };
 
@@ -546,11 +538,9 @@ __global__ void __launch_bounds__(kWgThreads) twgrad_kernel(const __grid_constan
     // LBO = distance between core matrices along K (128 B), SBO = distance between 8-channel groups (one plane).
     // Same issue-loop discipline as tconv_kernel: hoisted descriptor words, warp-uniform operands, a compile-time body
     // for full 128-row stages.
-    uint32_t a_lbo = 128, a_sbo = kWgStage * 16, b_lbo = 128, b_sbo = (kWgStage + 2) * 16;
-    if (p.swap_strides) { uint32_t t = a_lbo; a_lbo = a_sbo; a_sbo = t; t = b_lbo; b_lbo = b_sbo; b_sbo = t; }
     auto U = [](uint32_t x) { return __reduce_max_sync(0xffffffffu, x); };
     auto d64 = [](uint32_t lo, uint32_t hi) { return ((uint64_t)hi << 32) | lo; };
-    const uint64_t a_t = smem_desc(smem_u32(sS), a_lbo, a_sbo), b_t = smem_desc(smem_u32(sS) + dy_bytes, b_lbo, b_sbo);
+    const uint64_t a_t = smem_desc(smem_u32(sS), 128, kWgStage * 16), b_t = smem_desc(smem_u32(sS) + dy_bytes, 128, (kWgStage + 2) * 16);
     const uint32_t a_hi = U((uint32_t)(a_t >> 32)), b_hi = U((uint32_t)(b_t >> 32));
     const uint32_t a_first = U((uint32_t)a_t), b_first = U((uint32_t)b_t), st16 = U(st_bytes >> 4);
     const uint32_t tm = U(tmem), idesc = U(p.idesc), n_cols = U((uint32_t)N);
@@ -619,8 +609,8 @@ constexpr int kEwThreads = 256;
 constexpr int kEwRows = 1;           // rows per thread
 
 struct BnFwdParams {
-  const uint16_t* y;        // raw conv output (fwd type)
-  const uint16_t* res;      // residual (fwd type) or nullptr
+  const uint16_t* y;        // raw conv output (fp16)
+  const uint16_t* res;      // residual (fp16) or nullptr
   uint16_t* a;              // relu(bn(y) + res)
   uint16_t* a_b;            // optional bf16 copy (wgrad operand)
   uint8_t* bits;            // ReLU mask [16][R128]: bit e of byte (g, row) = (a[row][8 g + e] > 0): what the backward pass reads instead of a
@@ -628,10 +618,9 @@ struct BnFwdParams {
   float* saved;             // [128][2] (mean, invstd) for the backward pass
   const float *gamma, *beta;
   float *running_mean, *running_var;
-  int Ptot, PB, Wp, W, H, PR, R128, fbf16;
+  int Ptot, PB, Wp, W, H, PR, R128;
   int sub_rows, stat_sub, n_sub;   // stacked calls (blockIdx.z): rows per call, distance between their statistics records (floats)
   float inv_n, unbias;      // 1 / (B*H*W), n / (n - 1)
-  int ablate;               // measurement only: 16 skip the partial-sum pass
   unsigned long long* tl;
 };
 
@@ -693,22 +682,22 @@ __global__ void __launch_bounds__(kEwThreads) bn_fwd_kernel(const BnFwdParams p)
     uint32_t m = 0;
     if (P < p.Ptot && !is_halo(P, p.PB, p.Wp, p.W, p.H)) {
       float v[8];
-      unpack8(yr[k], p.fbf16, v);
+      unpack8<__half>(yr[k], v);
 #pragma unroll
       for (int e = 0; e < 8; ++e) v[e] = v[e] * sc[e] + sh[e];
       if (p.res) {
         float r[8];
-        unpack8(rr[k], p.fbf16, r);
+        unpack8<__half>(rr[k], r);
 #pragma unroll
         for (int e = 0; e < 8; ++e) v[e] += r[e];
       }
 #pragma unroll
       for (int e = 0; e < 8; ++e) v[e] = fmaxf(v[e], 0.0f);
-      o = pack8(v, p.fbf16);
-      if (p.a_b) ob = pack8(v, 1);
+      o = pack8<__half>(v);
+      if (p.a_b) ob = pack8<__nv_bfloat16>(v);
       // the mask is taken from the STORED value (what bn_bwd_reduce_kernel's `a > 0` sees)
       float w[8];
-      unpack8(o, p.fbf16, w);
+      unpack8<__half>(o, w);
 #pragma unroll
       for (int e = 0; e < 8; ++e) m |= (w[e] > 0.0f ? 1u : 0u) << e;
     }
@@ -721,15 +710,15 @@ __global__ void __launch_bounds__(kEwThreads) bn_fwd_kernel(const BnFwdParams p)
 
 struct BnBwdParams {
   const uint16_t* g;        // gradient w.r.t. the activated output (bf16); with a == nullptr it is already dZ
-  const uint16_t* a;        // the activated output (fwd type): ReLU mask, or nullptr
-  const uint16_t* y;        // raw conv output (fwd type)
+  const uint16_t* a;        // the activated output (fp16): ReLU mask, or nullptr
+  const uint16_t* y;        // raw conv output (fp16)
   const float* saved;       // [128][2] mean, invstd
   long long* sums;          // [128][2] fixed-point (sum dZ, sum dZ * xhat): from the reduce kernel / the dgrad epilogue
   const float* gamma;
   float *dgamma, *dbeta;    // += (apply kernel, blockIdx.x == 0)
   uint16_t* dy;             // gradient w.r.t. the raw conv output (bf16), zeros at halo rows
   uint16_t* dz;             // optional: the masked gradient itself (the residual branch's share), bf16
-  int Ptot, PB, Wp, W, H, PR, fbf16;
+  int Ptot, PB, Wp, W, H, PR;
   int sub_rows, stat_sub, n_sub;   // stacked calls (blockIdx.z), as in BnFwdParams
   float inv_n;
   int rows_per_cta;         // reduce kernel
@@ -751,9 +740,9 @@ __global__ void __launch_bounds__(kEwThreads) bn_bwd_reduce_kernel(const BnBwdPa
   for (int L = r_begin + threadIdx.x; L < r_end; L += kEwThreads) {
     // halo rows: G is zero there, so they add nothing
     float gv[8], av[8], yv[8];
-    unpack8(__ldcg(reinterpret_cast<const int4*>(p.g) + plane + L), 1, gv);
-    unpack8(__ldcg(reinterpret_cast<const int4*>(p.a) + plane + L), p.fbf16, av);
-    unpack8(__ldcg(reinterpret_cast<const int4*>(p.y) + plane + L), p.fbf16, yv);
+    unpack8<__nv_bfloat16>(__ldcg(reinterpret_cast<const int4*>(p.g) + plane + L), gv);
+    unpack8<__half>(__ldcg(reinterpret_cast<const int4*>(p.a) + plane + L), av);
+    unpack8<__half>(__ldcg(reinterpret_cast<const int4*>(p.y) + plane + L), yv);
 #pragma unroll
     for (int e = 0; e < 8; ++e) {
       const float dz = av[e] > 0.0f ? gv[e] : 0.0f;
@@ -833,17 +822,17 @@ __global__ void __launch_bounds__(kEwThreads) bn_bwd_apply_kernel(const BnBwdPar
     int4 o = make_int4(0, 0, 0, 0), oz = make_int4(0, 0, 0, 0);
     if (P < p.Ptot && !is_halo(P, p.PB, p.Wp, p.W, p.H)) {
       float gv[8], av[8], yv[8], dzv[8], dyv[8];
-      unpack8(gr[k], 1, gv);
-      if (p.a) unpack8(ar[k], p.fbf16, av);
-      unpack8(yr[k], p.fbf16, yv);
+      unpack8<__nv_bfloat16>(gr[k], gv);
+      if (p.a) unpack8<__half>(ar[k], av);
+      unpack8<__half>(yr[k], yv);
 #pragma unroll
       for (int e = 0; e < 8; ++e) {
         dzv[e] = (!p.a || av[e] > 0.0f) ? gv[e] : 0.0f;
         const float xh = (yv[e] - mean[e]) * is[e];
         dyv[e] = gi[e] * (dzv[e] - m1[e] - xh * m2[e]);
       }
-      o = pack8(dyv, 1);
-      oz = pack8(dzv, 1);
+      o = pack8<__nv_bfloat16>(dyv);
+      oz = pack8<__nv_bfloat16>(dzv);
     }
     reinterpret_cast<int4*>(p.dy)[plane + L] = o;
     if (p.dz) reinterpret_cast<int4*>(p.dz)[plane + L] = oz;
@@ -851,9 +840,9 @@ __global__ void __launch_bounds__(kEwThreads) bn_bwd_apply_kernel(const BnBwdPar
   tl_end(p.tl, 4);
 }
 
-// float32 [B][C][H][W] -> planes (zeros at halo positions and channels >= C); cg planes are written
+// float32 [B][C][H][W] -> fp16 planes and their bf16 copy (zeros at halo positions and channels >= C); cg planes are written
 __global__ void nchw_to_planes_kernel(const float* __restrict__ src, uint16_t* __restrict__ dst, uint16_t* __restrict__ dst_b, int C,
-                                      int cg, int Ptot, int PB, int Wp, int W, int H, int PR, int bf16) {
+                                      int cg, int Ptot, int PB, int Wp, int W, int H, int PR) {
   const int g = blockIdx.y;
   const int P = blockIdx.x * blockDim.x + threadIdx.x;
   if (P >= Ptot) return;
@@ -867,20 +856,20 @@ __global__ void nchw_to_planes_kernel(const float* __restrict__ src, uint16_t* _
   }
 #pragma unroll
   for (int e = 0; e < 8; ++e) v[e] = (g * 8 + e < C && y < H && x < W) ? v[e] : 0.0f;
-  reinterpret_cast<int4*>(dst)[(size_t)g * PR + kFront + P] = pack8(v, bf16);
-  if (dst_b) reinterpret_cast<int4*>(dst_b)[(size_t)g * PR + kFront + P] = pack8(v, 1);
+  reinterpret_cast<int4*>(dst)[(size_t)g * PR + kFront + P] = pack8<__half>(v);
+  reinterpret_cast<int4*>(dst_b)[(size_t)g * PR + kFront + P] = pack8<__nv_bfloat16>(v);
 }
 
-// planes -> float32 [B][C][H][W]; `mask`: optional planes (fwd type) whose sign gates nothing here (kept simple)
+// bf16 gradient planes -> float32 [B][C][H][W]
 __global__ void planes_to_nchw_kernel(const uint16_t* __restrict__ src, float* __restrict__ dst, int C, int Ptot, int PB, int Wp,
-                                      int W, int H, int PR, int bf16) {
+                                      int W, int H, int PR) {
   const int g = blockIdx.y;
   const int P = blockIdx.x * blockDim.x + threadIdx.x;
   if (P >= Ptot) return;
   const int b = P / PB, q = P - b * PB, y = q / Wp, x = q - y * Wp;
   if (y >= H || x >= W) return;
   float v[8];
-  unpack8(__ldcg(reinterpret_cast<const int4*>(src) + (size_t)g * PR + kFront + P), bf16, v);
+  unpack8<__nv_bfloat16>(__ldcg(reinterpret_cast<const int4*>(src) + (size_t)g * PR + kFront + P), v);
 #pragma unroll
   for (int e = 0; e < 8; ++e) {
     const int c = g * 8 + e;
@@ -897,14 +886,14 @@ constexpr int kTowerIoThreads = 512;
 
 __global__ void __launch_bounds__(kTowerIoThreads) tower_out_kernel(const uint16_t* __restrict__ src, float* __restrict__ raw,
                                                                     float* __restrict__ norm, int Ptot, int PB, int Wp, int W, int H,
-                                                                    int PR, int bf16) {
+                                                                    int PR) {
   __shared__ float s_lo[16][33], s_hi[16][33];
   const int g = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int P = blockIdx.x * 32 + lane;
   const int b = P / PB, q = P - b * PB, y = q / Wp, x = q - y * Wp;
   const bool real = P < Ptot && y < H && x < W;
   float v[8];
-  unpack8(__ldcg(reinterpret_cast<const int4*>(src) + (size_t)g * PR + kFront + P), bf16, v);      // rows past Ptot: the zero tail
+  unpack8<__half>(__ldcg(reinterpret_cast<const int4*>(src) + (size_t)g * PR + kFront + P), v);      // rows past Ptot: the zero tail
   float lo = v[0], hi = v[0];
 #pragma unroll
   for (int e = 1; e < 8; ++e) { lo = fminf(lo, v[e]); hi = fmaxf(hi, v[e]); }
@@ -932,7 +921,7 @@ __global__ void __launch_bounds__(kTowerIoThreads) tower_out_kernel(const uint16
 // row-wide quantities (lo, hi, their positions, the two sums) are combined over the 16 warps through shared memory.
 __global__ void __launch_bounds__(kTowerIoThreads) tower_gradin_kernel(const float* __restrict__ g_raw, const float* __restrict__ g_norm,
                                                                        const uint16_t* __restrict__ h, uint16_t* __restrict__ dst,
-                                                                       int Ptot, int PB, int Wp, int W, int H, int PR, int hbf16) {
+                                                                       int Ptot, int PB, int Wp, int W, int H, int PR) {
   __shared__ float s_lo[16][33], s_hi[16][33], s_1[16][33], s_2[16][33];
   __shared__ int s_amin[16][33], s_amax[16][33];
   const int g = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -945,7 +934,7 @@ __global__ void __launch_bounds__(kTowerIoThreads) tower_gradin_kernel(const flo
   for (int e = 0; e < 8; ++e) o[e] = (real && g_raw) ? __ldg(g_raw + base + e * cs) : 0.0f;
   if (g_norm) {
     float v[8], gn[8];
-    unpack8(__ldcg(reinterpret_cast<const int4*>(h) + (size_t)g * PR + kFront + P), hbf16, v);
+    unpack8<__half>(__ldcg(reinterpret_cast<const int4*>(h) + (size_t)g * PR + kFront + P), v);
 #pragma unroll
     for (int e = 0; e < 8; ++e) gn[e] = real ? __ldg(g_norm + base + e * cs) : 0.0f;
     float lo = v[0], hi = v[0];
@@ -981,13 +970,13 @@ __global__ void __launch_bounds__(kTowerIoThreads) tower_gradin_kernel(const flo
       if (c == amax) o[e] += dhi;
     }
   }
-  if (P < Ptot) reinterpret_cast<int4*>(dst)[(size_t)g * PR + kFront + P] = real ? pack8(o, 1) : make_int4(0, 0, 0, 0);
+  if (P < Ptot) reinterpret_cast<int4*>(dst)[(size_t)g * PR + kFront + P] = real ? pack8<__nv_bfloat16>(o) : make_int4(0, 0, 0, 0);
 }
 
 // the action "planes" of DynamicsConvNet.forward (network.py:440-444, quirk C of DESIGN.md): flat element f of the
 // [A*h*w] block is 1 iff f % A == action.  Written as channels 128.. of the dynamics' first-conv input (planes 16..31).
 __global__ void action_planes_kernel(const int64_t* __restrict__ action, uint16_t* __restrict__ dst, uint16_t* __restrict__ dst_b, int A,
-                                     int Ptot, int PB, int Wp, int W, int H, int PR, int bf16) {
+                                     int Ptot, int PB, int Wp, int W, int H, int PR) {
   const int g = blockIdx.y;                       // 0..15 -> plane 16 + g
   const int P = blockIdx.x * blockDim.x + threadIdx.x;
   if (P >= Ptot) return;
@@ -1001,8 +990,8 @@ __global__ void action_planes_kernel(const int64_t* __restrict__ action, uint16_
     if (c < A && y < H && x < W) f = ((c * H * W + y * W + x) % A == a) ? 1.0f : 0.0f;
     v[e] = f;
   }
-  reinterpret_cast<int4*>(dst)[(size_t)(16 + g) * PR + kFront + P] = pack8(v, bf16);
-  if (dst_b) reinterpret_cast<int4*>(dst_b)[(size_t)(16 + g) * PR + kFront + P] = pack8(v, 1);
+  reinterpret_cast<int4*>(dst)[(size_t)(16 + g) * PR + kFront + P] = pack8<__half>(v);
+  reinterpret_cast<int4*>(dst_b)[(size_t)(16 + g) * PR + kFront + P] = pack8<__nv_bfloat16>(v);
 }
 
 // ---- weights ---------------------------------------------------------------------------------------------------
@@ -1015,7 +1004,7 @@ struct ConvDesc {
   int ci_total, cg_in, chunk_g, n_groups, ci_blocks, slices, tower;
 };
 
-__global__ void pack_weights_kernel(const ConvDesc* __restrict__ descs, int fbf16) {
+__global__ void pack_weights_kernel(const ConvDesc* __restrict__ descs) {
   const ConvDesc d = descs[blockIdx.y];
   const int chunks = d.cg_in / d.chunk_g;
   const size_t nf = (size_t)9 * d.cg_in * kC * 8;
@@ -1030,8 +1019,7 @@ __global__ void pack_weights_kernel(const ConvDesc* __restrict__ descs, int fbf1
       const int tap = (int)(r / chunks);
       const int c = (ch * d.chunk_g + gl) * 8 + e;
       const float v = c < d.ci_total ? d.w[((size_t)n * d.ci_total + c) * 9 + tap] : 0.0f;
-      if (fbf16) reinterpret_cast<__nv_bfloat16*>(d.wf)[i] = __float2bfloat16_rn(v);
-      else reinterpret_cast<__half*>(d.wf)[i] = __float2half_rn(fminf(fmaxf(v, -65504.0f), 65504.0f));
+      reinterpret_cast<__half*>(d.wf)[i] = __float2half_rn(fminf(fmaxf(v, -65504.0f), 65504.0f));
     } else {
       const size_t j = i - nf;
       const int e = (int)(j % 8);
@@ -1078,10 +1066,6 @@ __global__ void wgrad_finalize_kernel(const ConvDesc* __restrict__ descs, int ca
 // ---------------------------------------------------------------------------------------------------------------
 struct BnPtrs { float *gamma, *dgamma, *beta, *dbeta, *rmean, *rvar; };
 
-struct Layer {              // one conv + BatchNorm of a tower
-  int conv;                 // index into convs[]
-};
-
 }  // namespace
 }  // namespace mz
 
@@ -1090,8 +1074,6 @@ using namespace mz;
 struct mz_train {
   mz_train_config cfg;
   Geom g;
-  int fbf16;                               // forward tensors are bf16 (else fp16)
-  int swap_strides;
   int nconv;                               // convs: rep0, rep blocks (2 each), dyn0, dyn blocks, pred blocks
   int rep_first, dyn_first, pred_first;    // index of each tower's first conv
   std::vector<ConvDesc> convs;
@@ -1109,7 +1091,7 @@ struct mz_train {
   int stat_stride;
   int n_calls[3];
   // saved activations: slot(tower, call) -> X, then (Y, A) per layer
-  std::vector<uint16_t*> slot_x, slot_xb;                    // xb / ab: bf16 copies for wgrad (== x / a when the forward type is bf16)
+  std::vector<uint16_t*> slot_x, slot_xb;                    // xb / ab: bf16 copies for wgrad (ab == a for a tower's last layer: no copy)
   std::vector<std::vector<uint16_t*>> slot_y, slot_a, slot_ab;
   std::vector<std::vector<uint8_t*>> slot_m;                 // ReLU masks [R128][16] per layer
   // weight gradients run on streams of their own, beside the dgrad / BatchNorm chain (nothing on the chain reads them):
@@ -1126,7 +1108,6 @@ struct mz_train {
   const Geom* cur_g;
   int cur_nsub, cur_sub_rows, cur_stat_sub;
   int num_sms;
-  bool no_persist;                         // MZ_TRAIN_NO_PERSIST=1: one tile per CTA also for the stacked launches
   bool group_ok;                           // rows of one call are a multiple of 128 and of 16 * kSplits: tiles and weight-gradient splits never straddle calls
   Geom gg;                                 // geometry of the stacked buffers (plane stride for unroll_steps calls)
   uint16_t* ggrad_buf[4 + kDyRing];
@@ -1178,38 +1159,31 @@ size_t wgrad_smem_bytes(int n_groups) {
 
 struct MaskArgs { const uint8_t* bits; const uint16_t* y; float* stat; };      // the layer whose ReLU / BatchNorm-backward sums a dgrad folds in
 
-template <typename... KArgs, typename... Args>
-cudaError_t launch_chain(mz_train* t, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
-  // programmatic dependent launch along the chain: the kernel may start as soon as its predecessor has called
-  // griddepcontrol.launch_dependents (the chain kernels do so at once; after an ordinary kernel -- weight packing, layout
-  // conversion -- it starts when that kernel has completed); everything that touches the predecessor's data sits behind
-  // griddepcontrol.wait, what does not (barrier set-up, TMEM allocation, the weight ring's first fill) runs before it.
-  (void)t;
-  return launch_pdl(true, kernel, grid, block, smem, st, args...);
-}
+// The conv and BatchNorm kernels of a tower form a chain launched with programmatic dependent launch (launch_pdl): a
+// kernel may start as soon as its predecessor has called griddepcontrol.launch_dependents (the chain kernels do so at
+// once; after an ordinary kernel -- weight packing, layout conversion -- it starts when that kernel has completed);
+// everything that touches the predecessor's data sits behind griddepcontrol.wait, what does not (barrier set-up, TMEM
+// allocation, the weight ring's first fill) runs before it.
 
+// forward: fp16 operands and output; dgrad: bf16
 int launch_conv(mz_train* t, const uint16_t* in, int cg_in, const uint16_t* w, uint16_t* out, const uint16_t* add,
-                float* stats, int a_bf16, int w_bf16, int out_bf16, cudaStream_t st, const MaskArgs* mask = nullptr) {
+                float* stats, bool dgrad, cudaStream_t st, const MaskArgs* mask = nullptr) {
   TConvParams p;
   const Geom& g = *t->cur_g;
   p.sub_rows = t->cur_nsub > 1 ? t->cur_sub_rows : g.R128; p.stat_sub = t->cur_stat_sub;
   p.in = in; p.w = w; p.out = out; p.add = add; p.stats = reinterpret_cast<long long*>(stats);
   p.mask_bits = mask ? mask->bits : nullptr; p.mask_y = mask ? mask->y : nullptr;
   p.mask_saved = mask ? mask->stat + 512 : nullptr; p.mask_sums = mask ? reinterpret_cast<long long*>(mask->stat + 768) : nullptr;
-  p.fbf16 = t->fbf16;
   p.cg_in = cg_in; p.stage_g = cg_in < 16 ? cg_in : 16; p.chunks = cg_in / p.stage_g;
   p.Ptot = g.Ptot; p.PB = g.PB; p.Wp = g.Wp; p.W = g.W; p.H = g.H; p.PR = g.PR; p.R128 = g.R128;
   const int tiles = g.R128 / 128;
-  p.nbuf = (tiles > t->num_sms && cg_in == 16 && !t->no_persist) ? 2 : 1;
+  p.nbuf = (tiles > t->num_sms && cg_in == 16) ? 2 : 1;
   const size_t smem = conv_smem_bytes(g, cg_in, p.nbuf, &p.stages, &p.TP, &p.TPs);
-  p.idesc = idesc_of(128, kC, (uint32_t)a_bf16, (uint32_t)w_bf16, 0);
-  p.out_bf16 = out_bf16;
-  static const int ablate = getenv("MZ_TRAIN_ABLATE") ? atoi(getenv("MZ_TRAIN_ABLATE")) : 0;
-  p.ablate = ablate;
+  p.idesc = idesc_of(128, kC, dgrad ? 1 : 0, dgrad ? 1 : 0, 0);
+  p.dgrad = dgrad;
   p.tl = t->timeline && t->tl_next < kTimelineMax ? t->timeline + 10 * (size_t)t->tl_next++ : nullptr;
-  if (ablate & 128) return MZ_OK;          // measurement only: no conv launches at all
   void (*kern)(TConvParams) = p.stage_g == 16 ? (p.chunks == 1 ? tconv_kernel<1> : (p.chunks == 2 ? tconv_kernel<2> : tconv_kernel<0>)) : tconv_kernel<0>;
-  cudaError_t e = launch_chain(t, kern, dim3(p.nbuf == 2 ? t->num_sms : tiles), dim3(kTConvThreads), smem, st, p);
+  cudaError_t e = launch_pdl(true, kern, dim3(p.nbuf == 2 ? t->num_sms : tiles), dim3(kTConvThreads), smem, st, p);
   if (e != cudaSuccess) { set_error("tconv_kernel launch: %s", cudaGetErrorString(e)); return MZ_ECUDA; }
   count_launch();
   return MZ_OK;
@@ -1232,10 +1206,7 @@ int launch_wgrad(mz_train* t, int conv, int call, int k, const uint16_t* dy, con
   p.Wp = g.Wp; p.PR = g.PR;
   p.slices = d.slices; p.slice0 = call * kSplits;
   p.idesc = idesc_of(128, (uint32_t)d.n_groups * 8, 1, 1, 1);
-  p.swap_strides = t->swap_strides;
   p.tl = t->timeline && t->tl_next < kTimelineMax ? t->timeline + 10 * (size_t)t->tl_next++ : nullptr;
-  static const int ablate = getenv("MZ_TRAIN_ABLATE") ? atoi(getenv("MZ_TRAIN_ABLATE")) : 0;
-  if (!(ablate & 256))                     // measurement only: 256 = no weight-gradient launches
   twgrad_kernel<<<dim3(kSplits * nsub, 3, d.ci_blocks), kWgThreads, wgrad_smem_bytes(d.n_groups), st>>>(p);
   MZ_LAUNCH_CHECK("twgrad_kernel");
   MZ_CUDA(cudaEventRecord(t->ev_wg[k], st));
@@ -1266,14 +1237,11 @@ int launch_bn_fwd(mz_train* t, int conv, const uint16_t* y, const uint16_t* res,
   p.n_sub = t->cur_nsub; p.sub_rows = t->cur_nsub > 1 ? t->cur_sub_rows : g.Ptot; p.stat_sub = t->cur_stat_sub;
   p.y = y; p.res = res; p.a = a; p.a_b = (a_b && a_b != a) ? a_b : nullptr; p.bits = bits; p.sums = reinterpret_cast<const long long*>(stat); p.saved = stat + 512;
   p.gamma = b.gamma; p.beta = b.beta; p.running_mean = b.rmean; p.running_var = b.rvar;
-  p.Ptot = g.Ptot; p.PB = g.PB; p.Wp = g.Wp; p.W = g.W; p.H = g.H; p.PR = g.PR; p.R128 = g.R128; p.fbf16 = t->fbf16;
+  p.Ptot = g.Ptot; p.PB = g.PB; p.Wp = g.Wp; p.W = g.W; p.H = g.H; p.PR = g.PR; p.R128 = g.R128;
   const double n = (double)g.B * g.H * g.W;
   p.inv_n = (float)(1.0 / n); p.unbias = (float)(n / (n - 1.0));
-  static const int ablate = getenv("MZ_TRAIN_ABLATE") ? atoi(getenv("MZ_TRAIN_ABLATE")) : 0;
-  p.ablate = ablate;
   p.tl = t->timeline && t->tl_next < kTimelineMax ? t->timeline + 10 * (size_t)t->tl_next++ : nullptr;
-  if (ablate & 64) return MZ_OK;           // measurement only: no BatchNorm launches at all
-  cudaError_t e = launch_chain(t, bn_fwd_kernel, ew_grid(t, 16), dim3(kEwThreads), 0, st, p);
+  cudaError_t e = launch_pdl(true, bn_fwd_kernel, ew_grid(t, 16), dim3(kEwThreads), 0, st, p);
   if (e != cudaSuccess) { set_error("bn_fwd_kernel launch: %s", cudaGetErrorString(e)); return MZ_ECUDA; }
   count_launch();
   return MZ_OK;
@@ -1289,7 +1257,7 @@ int launch_bn_bwd(mz_train* t, int conv, const uint16_t* gin, const uint16_t* a,
   p.n_sub = t->cur_nsub; p.sub_rows = t->cur_nsub > 1 ? t->cur_sub_rows : g.Ptot; p.stat_sub = t->cur_stat_sub;
   p.g = gin; p.a = a; p.y = y; p.saved = stat + 512; p.sums = reinterpret_cast<long long*>(stat + 768); p.gamma = b.gamma; p.dgamma = b.dgamma; p.dbeta = b.dbeta;
   p.dy = dy; p.dz = dz;
-  p.Ptot = g.Ptot; p.PB = g.PB; p.Wp = g.Wp; p.W = g.W; p.H = g.H; p.PR = g.PR; p.fbf16 = t->fbf16;
+  p.Ptot = g.Ptot; p.PB = g.PB; p.Wp = g.Wp; p.W = g.W; p.H = g.H; p.PR = g.PR;
   p.inv_n = (float)(1.0 / ((double)g.B * g.H * g.W));
   p.tl = nullptr;
   const int nchunk = 9;
@@ -1298,10 +1266,8 @@ int launch_bn_bwd(mz_train* t, int conv, const uint16_t* gin, const uint16_t* a,
     bn_bwd_reduce_kernel<<<dim3(nchunk, 16, t->cur_nsub), kEwThreads, 0, st>>>(p);
     MZ_LAUNCH_CHECK("bn_bwd_reduce_kernel");
   }
-  static const int ablate = getenv("MZ_TRAIN_ABLATE") ? atoi(getenv("MZ_TRAIN_ABLATE")) : 0;
-  if (ablate & 64) return MZ_OK;
   p.tl = t->timeline && t->tl_next < kTimelineMax ? t->timeline + 10 * (size_t)t->tl_next++ : nullptr;
-  cudaError_t e = launch_chain(t, bn_bwd_apply_kernel, ew_grid(t, 16), dim3(kEwThreads), 0, st, p);
+  cudaError_t e = launch_pdl(true, bn_bwd_apply_kernel, ew_grid(t, 16), dim3(kEwThreads), 0, st, p);
   if (e != cudaSuccess) { set_error("bn_bwd_apply_kernel launch: %s", cudaGetErrorString(e)); return MZ_ECUDA; }
   count_launch();
   return MZ_OK;
@@ -1375,21 +1341,19 @@ static int train_layout(const mz_train_config* c, Geom* g, size_t* bytes, mz_tra
   }
   // saved activations
   const int nslots = 1 + 2 * T;
-  const bool fb = getenv("MZ_TRAIN_FWD_BF16") ? atoi(getenv("MZ_TRAIN_FWD_BF16")) != 0 : false;
   if (t) { t->slot_x.resize(nslots); t->slot_xb.resize(nslots); t->slot_y.resize(nslots); t->slot_a.resize(nslots); t->slot_ab.resize(nslots); t->slot_m.resize(nslots); }
   int s = 0;
   for (int tower = 0; tower < 3; ++tower)
     for (int call = 0; call < calls[tower]; ++call, ++s) {
       const int xg = tower == 0 ? in_cg : (tower == 1 ? 32 : 16);
-      const size_t ox = take((size_t)xg * plane);
-      const size_t oxb = fb ? ox : take((size_t)xg * plane);
+      const size_t ox = take((size_t)xg * plane), oxb = take((size_t)xg * plane);
       if (t) { t->slot_x[s] = reinterpret_cast<uint16_t*>(t->arena + ox); t->slot_xb[s] = reinterpret_cast<uint16_t*>(t->arena + oxb); }
       const int layers = (tower == 2 ? 0 : 1) + 2 * nb;
       if (t) { t->slot_y[s].resize(layers); t->slot_a[s].resize(layers); t->slot_ab[s].resize(layers); t->slot_m[s].resize(layers); }
       for (int l = 0; l < layers; ++l) {
         const size_t oy = take(16 * plane), oa = take(16 * plane);
         // the tower's last activation feeds no convolution of this tower: no bf16 copy
-        const size_t oab = (fb || l == layers - 1) ? oa : take(16 * plane);
+        const size_t oab = l == layers - 1 ? oa : take(16 * plane);
         const size_t om = take((size_t)g->R128 * 16);
         if (t) {
           t->slot_m[s][l] = t->arena + om;
@@ -1399,7 +1363,7 @@ static int train_layout(const mz_train_config* c, Geom* g, size_t* bytes, mz_tra
       }
     }
   // stacked prediction calls: their own activation slots and gradient buffers with a plane stride for T calls
-  const bool group_ok = T > 1 && g->Ptot % 128 == 0 && g->Ptot % (16 * kSplits) == 0 && !(getenv("MZ_TRAIN_NO_STACK") && atoi(getenv("MZ_TRAIN_NO_STACK")));
+  const bool group_ok = T > 1 && g->Ptot % 128 == 0 && g->Ptot % (16 * kSplits) == 0;
   if (t) t->group_ok = group_ok;
   if (group_ok) {
     Geom gg = *g;
@@ -1411,15 +1375,14 @@ static int train_layout(const mz_train_config* c, Geom* g, size_t* bytes, mz_tra
       if (t) t->ggrad_buf[k] = reinterpret_cast<uint16_t*>(t->arena + o);
     }
     const int layers = 2 * nb;
-    const size_t ox = take(16 * gplane);
-    const size_t oxb = fb ? ox : take(16 * gplane);
+    const size_t ox = take(16 * gplane), oxb = take(16 * gplane);
     if (t) {
       t->gslot_x = reinterpret_cast<uint16_t*>(t->arena + ox); t->gslot_xb = reinterpret_cast<uint16_t*>(t->arena + oxb);
       t->gslot_y.resize(layers); t->gslot_a.resize(layers); t->gslot_ab.resize(layers); t->gslot_m.resize(layers);
     }
     for (int l = 0; l < layers; ++l) {
       const size_t oy = take(16 * gplane), oa = take(16 * gplane);
-      const size_t oab = (fb || l == layers - 1) ? oa : take(16 * gplane);
+      const size_t oab = l == layers - 1 ? oa : take(16 * gplane);
       const size_t om = take((size_t)gg.R128 * 16);
       if (t) {
         t->gslot_y[l] = reinterpret_cast<uint16_t*>(t->arena + oy); t->gslot_a[l] = reinterpret_cast<uint16_t*>(t->arena + oa);
@@ -1448,8 +1411,6 @@ int mz_train_create(const mz_train_config* cfg, void* arena_dev, size_t arena_by
   t->cfg = *cfg; t->g = g;
   t->arena = static_cast<unsigned char*>(arena_dev); t->arena_bytes = arena_bytes;
   t->plane_bytes = (size_t)g.PR * 16;
-  t->fbf16 = getenv("MZ_TRAIN_FWD_BF16") ? atoi(getenv("MZ_TRAIN_FWD_BF16")) != 0 : 0;
-  t->swap_strides = getenv("MZ_TRAIN_WGRAD_SWAP") ? atoi(getenv("MZ_TRAIN_WGRAD_SWAP")) != 0 : 0;
   t->bound = false;
   rc = train_layout(cfg, &t->g, &need, t);
   if (rc) { delete t; return rc; }
@@ -1461,7 +1422,6 @@ int mz_train_create(const mz_train_config* cfg, void* arena_dev, size_t arena_by
   for (int k = 0; k < 3; ++k) { const size_t s = conv_smem_bytes(t->g, cgs[k], 1, nullptr, nullptr, nullptr); if (s > max_smem) max_smem = s; }
   { const size_t s = conv_smem_bytes(t->g, 16, 2, nullptr, nullptr, nullptr); if (s > max_smem) max_smem = s; }
   { int dev = 0, sms = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev); t->num_sms = sms > 0 ? sms : 148; }
-  t->no_persist = getenv("MZ_TRAIN_NO_PERSIST") && atoi(getenv("MZ_TRAIN_NO_PERSIST"));
   e = cudaFuncSetAttribute(tconv_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)max_smem);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(tconv_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)max_smem);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(tconv_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)max_smem);
@@ -1470,13 +1430,11 @@ int mz_train_create(const mz_train_config* cfg, void* arena_dev, size_t arena_by
   // its defaults the driver re-partitions L1 / shared memory at every such boundary, which drains the SMs (measured:
   // 15 us per conv + BatchNorm pair with every instruction of the conv kernel ablated).  Everything asks for the
   // maximum carve-out instead.
-  if (!getenv("MZ_TRAIN_NO_CARVEOUT")) {
-    const void* ks[] = {(const void*)tconv_kernel<0>, (const void*)tconv_kernel<1>, (const void*)tconv_kernel<2>, (const void*)twgrad_kernel, (const void*)bn_fwd_kernel, (const void*)bn_bwd_apply_kernel,
-                        (const void*)bn_bwd_reduce_kernel, (const void*)nchw_to_planes_kernel, (const void*)planes_to_nchw_kernel,
-                        (const void*)action_planes_kernel};
-    for (const void* k : ks)
-      if (e == cudaSuccess) e = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-  }
+  const void* ks[] = {(const void*)tconv_kernel<0>, (const void*)tconv_kernel<1>, (const void*)tconv_kernel<2>, (const void*)twgrad_kernel, (const void*)bn_fwd_kernel, (const void*)bn_bwd_apply_kernel,
+                      (const void*)bn_bwd_reduce_kernel, (const void*)nchw_to_planes_kernel, (const void*)planes_to_nchw_kernel,
+                      (const void*)action_planes_kernel};
+  for (const void* k : ks)
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   if (e != cudaSuccess) { delete t; set_error("cudaFuncSetAttribute: %s", cudaGetErrorString(e)); return MZ_ECUDA; }
   for (int k = 0; k < kSideStreams; ++k) t->side[k] = nullptr;
   for (int k = 0; k < kDyRing; ++k) { t->ev_dy[k] = nullptr; t->ev_wg[k] = nullptr; }
@@ -1533,7 +1491,7 @@ int mz_train_begin_step(mz_train* t, mz_stream stream) {
   if (!t->bound) { set_error("mz_train_begin_step: mz_train_bind has not been called"); return MZ_ESTATE; }
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   MZ_CUDA(cudaMemsetAsync(t->stats, 0, t->stats_floats * 4, st));
-  pack_weights_kernel<<<dim3(32, t->nconv), 256, 0, st>>>(t->d_convs, t->fbf16);
+  pack_weights_kernel<<<dim3(32, t->nconv), 256, 0, st>>>(t->d_convs);
   MZ_LAUNCH_CHECK("pack_weights_kernel");
   std::fill(t->touched.begin(), t->touched.end(), 0);
   t->dy_turn = 0;                          // (pending weight-gradient launches keep their events: mz_train_join / next_dy wait for them)
@@ -1580,33 +1538,32 @@ int mz_train_tower_forward_calls(mz_train* t, int32_t tower, int32_t call, int32
   const int c_in = tower == 0 ? t->cfg.in_channels : kC;
   const dim3 cgrid((g.Ptot + 255) / 256, tower == 1 ? 16 : xg);
   uint16_t* X = cb.x;
-  uint16_t* Xb = cb.xb != X ? cb.xb : nullptr;
-  nchw_to_planes_kernel<<<cgrid, 256, 0, st>>>(x, X, Xb, c_in, tower == 1 ? 16 : xg, g.Ptot, g.PB, g.Wp, g.W, g.H, g.PR, t->fbf16);
+  nchw_to_planes_kernel<<<cgrid, 256, 0, st>>>(x, X, cb.xb, c_in, tower == 1 ? 16 : xg, g.Ptot, g.PB, g.Wp, g.W, g.H, g.PR);
   MZ_LAUNCH_CHECK("nchw_to_planes_kernel");
   if (tower == 1) {
-    action_planes_kernel<<<dim3((g.Ptot + 255) / 256, 16), 256, 0, st>>>(action, X, Xb, t->cfg.num_actions, g.Ptot, g.PB, g.Wp, g.W,
-                                                                       g.H, g.PR, t->fbf16);
+    action_planes_kernel<<<dim3((g.Ptot + 255) / 256, 16), 256, 0, st>>>(action, X, cb.xb, t->cfg.num_actions, g.Ptot, g.PB, g.Wp,
+                                                                       g.W, g.H, g.PR);
     MZ_LAUNCH_CHECK("action_planes_kernel");
   }
   int conv = tower_first_conv(t, tower), layer = 0, rc;
   const uint16_t* cur = X;
   auto stat = [&](int l) { return t->stats + (size_t)stat_slot(t, tower, call, l) * t->stat_stride; };
   if (tower != 2) {
-    if ((rc = launch_conv(t, X, xg, t->convs[conv].wf, cb.y[0], nullptr, stat(0), t->fbf16, t->fbf16, t->fbf16, st))) return rc;
+    if ((rc = launch_conv(t, X, xg, t->convs[conv].wf, cb.y[0], nullptr, stat(0), false, st))) return rc;
     if ((rc = launch_bn_fwd(t, conv, cb.y[0], nullptr, cb.a[0], cb.ab[0], cb.m[0], stat(0), st))) return rc;
     cur = cb.a[0];
     ++conv; ++layer;
   }
   for (int b = 0; b < nb; ++b) {
     uint16_t *y1 = cb.y[layer], *a1 = cb.a[layer], *y2 = cb.y[layer + 1], *a2 = cb.a[layer + 1];
-    if ((rc = launch_conv(t, cur, 16, t->convs[conv].wf, y1, nullptr, stat(layer), t->fbf16, t->fbf16, t->fbf16, st))) return rc;
+    if ((rc = launch_conv(t, cur, 16, t->convs[conv].wf, y1, nullptr, stat(layer), false, st))) return rc;
     if ((rc = launch_bn_fwd(t, conv, y1, nullptr, a1, cb.ab[layer], cb.m[layer], stat(layer), st))) return rc;
-    if ((rc = launch_conv(t, a1, 16, t->convs[conv + 1].wf, y2, nullptr, stat(layer + 1), t->fbf16, t->fbf16, t->fbf16, st))) return rc;
+    if ((rc = launch_conv(t, a1, 16, t->convs[conv + 1].wf, y2, nullptr, stat(layer + 1), false, st))) return rc;
     if ((rc = launch_bn_fwd(t, conv + 1, y2, cur, a2, cb.ab[layer + 1], cb.m[layer + 1], stat(layer + 1), st))) return rc;
     cur = a2;
     conv += 2; layer += 2;
   }
-  tower_out_kernel<<<dim3((g.Ptot + 31) / 32), kTowerIoThreads, 0, st>>>(cur, out, out_norm, g.Ptot, g.PB, g.Wp, g.W, g.H, g.PR, t->fbf16);
+  tower_out_kernel<<<dim3((g.Ptot + 31) / 32), kTowerIoThreads, 0, st>>>(cur, out, out_norm, g.Ptot, g.PB, g.Wp, g.W, g.H, g.PR);
   MZ_LAUNCH_CHECK("tower_out_kernel");
   return MZ_OK;
 }
@@ -1638,7 +1595,7 @@ int mz_train_tower_backward_calls(mz_train* t, int32_t tower, int32_t call, int3
   bool masked = false;
   auto other = [&](int a, int b, int c) { for (int i = 0; i < 4; ++i) if (i != a && i != b && i != c) return i; return -1; };
   tower_gradin_kernel<<<dim3((g.Ptot + 31) / 32), kTowerIoThreads, 0, st>>>(grad_out, grad_norm, cb.a[first + 2 * nb - 1], G[cur], g.Ptot, g.PB,
-                                                                  g.Wp, g.W, g.H, g.PR, t->fbf16);
+                                                                  g.Wp, g.W, g.H, g.PR);
   MZ_LAUNCH_CHECK("tower_gradin_kernel");
   for (int b = nb - 1; b >= 0; --b) {
     const int l1 = first + 2 * b, l2 = l1 + 1;
@@ -1656,7 +1613,7 @@ int mz_train_tower_backward_calls(mz_train* t, int32_t tower, int32_t call, int3
     if ((rc = launch_wgrad(t, c2, call, k, dYb[k], cb.ab[l1], st))) return rc;
     const int f1 = other(cur, -1, -1);
     const MaskArgs m1{cb.m[l1], cb.y[l1], stat(l1)};
-    if ((rc = launch_conv(t, dYb[k], 16, t->convs[c2].wd, G[f1], nullptr, nullptr, 1, 1, 1, st, &m1))) return rc;
+    if ((rc = launch_conv(t, dYb[k], 16, t->convs[c2].wd, G[f1], nullptr, nullptr, true, st, &m1))) return rc;
     // first conv: a1 = relu(bn1(conv1(a_in)))
     if ((rc = next_dy(t, st, &k))) return rc;
     if ((rc = launch_bn_bwd(t, c1, G[f1], nullptr, cb.y[l1], stat(l1), dYb[k], nullptr, st))) return rc;
@@ -1664,10 +1621,10 @@ int mz_train_tower_backward_calls(mz_train* t, int32_t tower, int32_t call, int3
     const int f2 = other(cur, f1, -1);
     if (l1 > 0) {                          // a_in is the output of layer l1 - 1 of this tower: fold its ReLU mask and sums in
       const MaskArgs m0{cb.m[l1 - 1], cb.y[l1 - 1], stat(l1 - 1)};
-      if ((rc = launch_conv(t, dYb[k], 16, t->convs[c1].wd, G[f2], G[cur], nullptr, 1, 1, 1, st, &m0))) return rc;
+      if ((rc = launch_conv(t, dYb[k], 16, t->convs[c1].wd, G[f2], G[cur], nullptr, true, st, &m0))) return rc;
       masked = true;
     } else {                               // a_in is the tower's input: the plain gradient
-      if ((rc = launch_conv(t, dYb[k], 16, t->convs[c1].wd, G[f2], G[cur], nullptr, 1, 1, 1, st))) return rc;
+      if ((rc = launch_conv(t, dYb[k], 16, t->convs[c1].wd, G[f2], G[cur], nullptr, true, st))) return rc;
       masked = false;
     }
     cur = f2;
@@ -1678,12 +1635,12 @@ int mz_train_tower_backward_calls(mz_train* t, int32_t tower, int32_t call, int3
     if ((rc = launch_wgrad(t, conv0, call, k, dYb[k], cb.xb, st))) return rc;
     if (tower == 1) {
       const int f = other(cur, -1, -1);
-      if ((rc = launch_conv(t, dYb[k], 16, t->convs[conv0].wd, G[f], nullptr, nullptr, 1, 1, 1, st))) return rc;
+      if ((rc = launch_conv(t, dYb[k], 16, t->convs[conv0].wd, G[f], nullptr, nullptr, true, st))) return rc;
       cur = f;
     }
   }
   if (tower != 0) {
-    planes_to_nchw_kernel<<<cgrid, 256, 0, st>>>(G[cur], grad_in, kC, g.Ptot, g.PB, g.Wp, g.W, g.H, g.PR, 1);
+    planes_to_nchw_kernel<<<cgrid, 256, 0, st>>>(G[cur], grad_in, kC, g.Ptot, g.PB, g.Wp, g.W, g.H, g.PR);
     MZ_LAUNCH_CHECK("planes_to_nchw_kernel");
   }
   return MZ_OK;

@@ -159,7 +159,7 @@ class _HeadConv1x1(torch.autograd.Function):
 
 def _head_conv(x: torch.Tensor, weight: torch.Tensor) -> torch.Tensor:
     if (x.is_cuda and x.dtype == torch.float32 and weight.shape[0] <= 4 and weight.shape[1] <= 256
-            and tuple(weight.shape[2:]) == (1, 1) and os.environ.get('MZ_HEAD_CONV', '1') != '0'):
+            and tuple(weight.shape[2:]) == (1, 1)):
         return _HeadConv1x1.apply(x, weight)
     return F.conv2d(x, weight)
 

@@ -189,9 +189,8 @@ class TowerTrainEngine:
         raw = self.arena[off:off + n.value]
         if which == 3:
             return raw.view(torch.float32).reshape(128, 2).clone()
-        dt = torch.bfloat16 if os.environ.get('MZ_TRAIN_FWD_BF16', '0') not in ('', '0') else torch.float16
         _, h, w = self.input_shape
-        planes = raw.view(dt).reshape(-1, pr.value, 8)[:, fr.value:fr.value + self.batch * (h + 1) * (w + 1)]
+        planes = raw.view(torch.float16).reshape(-1, pr.value, 8)[:, fr.value:fr.value + self.batch * (h + 1) * (w + 1)]
         g = planes.shape[0]
         x = planes.reshape(g, self.batch, h + 1, w + 1, 8)[:, :, :h, :w]
         return x.permute(1, 0, 4, 2, 3).reshape(self.batch, g * 8, h, w).float()

@@ -217,12 +217,12 @@ class DataParallelLearner:
         self.network, self.config, self.device = network, config, torch.device(device)
         # conv nets on CUDA train with NHWC weights / activations: same fp32 (TF32) cuDNN arithmetic without the layout
         # transposes around every convolution (24.8 -> 20.7 ms per 128 x K=5 Gomoku step).  state_dict shapes, the
-        # engine's weight packing and checkpoints are unaffected (memory format only).  MZ_TRAIN_CHANNELS_LAST=0: NCHW.
+        # engine's weight packing and checkpoints are unaffected (memory format only).
         # Networks the hand-written tower kernels cover (train_engine.py) keep NCHW parameters: the kernels read them.
         from . import train_engine
         self.native_towers = (self.device.type == 'cuda' and train_engine._enabled() and train_engine.supported(network))
-        self.channels_last = (os.environ.get('MZ_TRAIN_CHANNELS_LAST', '1') != '0' and self.device.type == 'cuda'
-                              and getattr(network, 'latent_hw', (0, 0)) != (0, 0) and not self.native_towers)
+        self.channels_last = (self.device.type == 'cuda' and getattr(network, 'latent_hw', (0, 0)) != (0, 0)
+                              and not self.native_towers)
         if self.channels_last:
             network.to(memory_format=torch.channels_last)
         self.group = process_group
