@@ -376,7 +376,9 @@ int mz_train_join(mz_train* t, mz_stream stream);
 int mz_train_end_step(mz_train* t, mz_stream stream);
 /* parity tests: which = 0 tower input planes, 1 raw conv output of `layer`, 2 its activated output, 3 its
  * batch statistics f32 [128][2] (mean, 1/sqrt(var + eps)).  Planes are 16-bit [groups][plane_rows][8],
- * row P of the padded (H+1)x(W+1) grid at plane row front_rows + P.                                                */
+ * row P of the padded (H+1)x(W+1) grid at plane row front_rows + P.  A prediction call that ran stacked in this
+ * step's forward returns the stacked buffers (plane_rows of unroll_steps calls, front_rows past the earlier calls
+ * of its stack): the same values a separate forward of that call stores.                                           */
 int mz_train_debug_view(mz_train* t, int32_t tower, int32_t call, int32_t layer, int32_t which, void** ptr, size_t* bytes,
                         int32_t* plane_rows, int32_t* front_rows);
 

@@ -1114,7 +1114,8 @@ struct mz_train {
   uint16_t *gslot_x, *gslot_xb;
   std::vector<uint16_t*> gslot_y, gslot_a, gslot_ab;
   std::vector<uint8_t*> gslot_m;
-  unsigned long long* timeline;            // MZ_TRAIN_TIMELINE=1: [kTimelineMax][10] stamps, one record per chain launch
+  std::vector<int> pred_stack_first;       // per prediction call of this step: first call of the stacked forward it ran in, or -1
+  unsigned long long* timeline;           // MZ_TRAIN_TIMELINE=1: [kTimelineMax][10] stamps, one record per chain launch
   int tl_next;
 };
 
@@ -1338,6 +1339,7 @@ static int train_layout(const mz_train_config* c, Geom* g, size_t* bytes, mz_tra
   if (t) {
     t->stats = reinterpret_cast<float*>(t->arena + o_stats); t->stats_floats = nstat * stat_stride; t->stat_stride = stat_stride;
     for (int k = 0; k < 3; ++k) t->n_calls[k] = calls[k];
+    t->pred_stack_first.assign(T, -1);
   }
   // saved activations
   const int nslots = 1 + 2 * T;
@@ -1496,6 +1498,7 @@ int mz_train_begin_step(mz_train* t, mz_stream stream) {
   std::fill(t->touched.begin(), t->touched.end(), 0);
   t->dy_turn = 0;                          // (pending weight-gradient launches keep their events: mz_train_join / next_dy wait for them)
   t->fwd_calls[0] = t->fwd_calls[1] = t->fwd_calls[2] = 0;
+  std::fill(t->pred_stack_first.begin(), t->pred_stack_first.end(), -1);
   t->tl_next = 0;
   return MZ_OK;
 }
@@ -1534,6 +1537,8 @@ int mz_train_tower_forward_calls(mz_train* t, int32_t tower, int32_t call, int32
   const Geom& g = *t->cur_g;
   const int nb = t->cfg.num_res_blocks;
   if (call + ncalls > t->fwd_calls[tower]) t->fwd_calls[tower] = call + ncalls;
+  if (tower == 2)                          // where mz_train_debug_view finds these calls' saved tensors
+    for (int c = call; c < call + ncalls; ++c) t->pred_stack_first[c] = ncalls > 1 ? call : -1;
   const int xg = tower_in_groups(t, tower);
   const int c_in = tower == 0 ? t->cfg.in_channels : kC;
   const dim3 cgrid((g.Ptot + 255) / 256, tower == 1 ? 16 : xg);
@@ -1687,17 +1692,24 @@ int mz_train_debug_view(mz_train* t, int32_t tower, int32_t call, int32_t layer,
   MZ_CHECK_ARG(tower >= 0 && tower < 3 && call >= 0 && call < t->n_calls[tower], "mz_train_debug_view: tower %d call %d out of range", tower, call);
   const int slot = slot_of(t, tower, call);
   const int layers = tower_layers(t, tower);
-  if (plane_rows) *plane_rows = t->g.PR;
-  if (front_rows) *front_rows = kFront;
+  // a prediction call that ran stacked saved its tensors in the stacked buffers, at row (call - first) * Ptot of them
+  const int first = tower == 2 ? t->pred_stack_first[call] : -1;
+  const size_t plane_bytes = first >= 0 ? (size_t)t->gg.PR * 16 : t->plane_bytes;
+  if (plane_rows) *plane_rows = first >= 0 ? t->gg.PR : t->g.PR;
+  if (front_rows) *front_rows = kFront + (first >= 0 ? (call - first) * t->g.Ptot : 0);
   if (which == 4) {
     if (!t->timeline) { set_error("mz_train_debug_view: no timeline (MZ_TRAIN_TIMELINE=1 at creation)"); return MZ_ESTATE; }
     *ptr = t->timeline; *bytes = (size_t)t->tl_next * 10 * sizeof(unsigned long long);
     return MZ_OK;
   }
-  if (which == 0) { *ptr = t->slot_x[slot]; *bytes = (size_t)tower_in_groups(t, tower) * t->plane_bytes; return MZ_OK; }
+  if (which == 0) {
+    *ptr = first >= 0 ? t->gslot_x : t->slot_x[slot];
+    *bytes = (size_t)tower_in_groups(t, tower) * plane_bytes;
+    return MZ_OK;
+  }
   MZ_CHECK_ARG(layer >= 0 && layer < layers, "mz_train_debug_view: layer %d out of range", layer);
-  if (which == 1) { *ptr = t->slot_y[slot][layer]; *bytes = 16 * t->plane_bytes; return MZ_OK; }
-  if (which == 2) { *ptr = t->slot_a[slot][layer]; *bytes = 16 * t->plane_bytes; return MZ_OK; }
+  if (which == 1) { *ptr = first >= 0 ? t->gslot_y[layer] : t->slot_y[slot][layer]; *bytes = 16 * plane_bytes; return MZ_OK; }
+  if (which == 2) { *ptr = first >= 0 ? t->gslot_a[layer] : t->slot_a[slot][layer]; *bytes = 16 * plane_bytes; return MZ_OK; }
   if (which == 3) { *ptr = t->stats + (size_t)stat_slot(t, tower, call, layer) * t->stat_stride + 512; *bytes = 256 * 4; return MZ_OK; }
   set_error("mz_train_debug_view: unknown view %d", which);
   return MZ_EINVAL;
