@@ -2,15 +2,11 @@
 // Blackwell tensor cores (fp16 x fp16 -> fp32).
 //
 // Data layout ("channel-group planes"): a board is a grid of
-//   PB = (H+pad)*(W+pad) positions,  position q = y*(W+pad) + x,          pad = grid_pad(), 0 by default.
+//   PB = H*W positions,  position q = y*W + x.
 // Flattening boards back to back (row P = b*PB + q) makes every 3x3 tap a constant row offset: tap (ky,kx) of
-// output row P reads input row P + (ky-1)*(W+pad) + (kx-1).
-//   pad == 0: no row is padding; a tap whose neighbour lies across a board edge is switched off for that output row
-//             by the disable-output-lane vector of the tap's tcgen05.mma (edge masks per tile from the loader warp,
-//             centre tap first so that it initialises the accumulator).
-//   pad == 1 (MZ_CONV_PAD=1, the first version): column x == W and row y == H are a ZERO halo shared with the next
-//             row / the next board, every tap is unmasked, every writer of an activation buffer writes zeros at halo
-//             positions.  19 % (9x9) / 27 % (6x6) of all MMA rows are halo.
+// output row P reads input row P + (ky-1)*W + (kx-1).  No row is padding: a tap whose neighbour lies across a board
+// edge is switched off for that output row by the disable-output-lane vector of the tap's tcgen05.mma (edge masks
+// per tile from the loader warp, centre tap first so that it initialises the accumulator).
 // An activation tensor is stored as C/8 PLANES of [rows][8 channels] fp16 (16 bytes per row):
 //   contiguous buffer:  element (P, c) at ((c/8) * plane_rows + P) * 8 + c%8
 //   hidden-state slot:  element (q, c) of slot s at ((s * C/8 + c/8) * PB + q) * 8 + c%8
@@ -81,10 +77,10 @@ struct ConvParams {
   int rot;                        // tile t of layer l belongs to CTA (t + l*rot) % grid: rotates who gets the odd tile
   unsigned int* flags;            // [num_layers][num_tiles], zeroed before the launch (nullptr for one layer)
   int* err;                       // dependency wait timed out (should never happen)
-  int Ptot, PB, Wp, W, H, B;
+  int Ptot, PB, W, H, B;
   int plane_rows;                 // rows per plane of the contiguous buffers of this launch
   int sub;                        // stride-2 layer: only rows with even (y, x) are stored, on the half-size grid
-  int out_plane_rows, out_PB, out_Wp;   // geometry of the output buffer when sub is set
+  int out_plane_rows, out_PB, out_W;    // geometry of the output buffer when sub is set
   int cg;                         // input channel groups of 8 (Cin_pad / 8), even
   int N;                          // output channels of one layer of this launch (multiple of 32, <= 128); wider convs
                                   // run as several 128-column passes, each its own LayerDesc
@@ -100,15 +96,11 @@ struct ConvParams {
   int khalf;                      // resident 256-row launches with two 64-channel K chunks: the K loop runs chunk by chunk
                                   // and the epilogue hands the low / high 64 channels of the next tile over separately
   int resident;                   // every CTA owns ONE board-aligned tile for all layers; activations stay in shared memory
-  int masked;                     // halo-free grid: edge taps are masked per output row (disable-output-lane)
-  int ablate;                     // debug only (MZ_CONV_ABLATE): 1 skip epilogue work, 2 skip tile loads, 4 skip weight copies, 512 epilogue without global loads/stores
 };
 
-__device__ __forceinline__ void split_pos(int P, const ConvParams& p, int& b, int& q, bool& halo) {
+__device__ __forceinline__ void split_pos(int P, const ConvParams& p, int& b, int& q) {
   b = P / p.PB;
   q = P - b * p.PB;
-  const int y = q / p.Wp, x = q - y * p.Wp;
-  halo = (x == p.W) || (y == p.H);
 }
 
 __device__ __forceinline__ uint32_t pack2(float a, float b) {
@@ -187,7 +179,7 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
   constexpr bool kSplitK = (kRows == 128);
   extern __shared__ __align__(1024) unsigned char smem[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int halo = p.Wp + 1;
+  const int halo = p.W + 1;
   const int TP = p.TP;
   const int chunk_g = p.cg < 8 ? p.cg : 8;              // channel groups per weight stage
   const int chunks_tap = p.cg / chunk_g;                // weight stages per tap
@@ -265,7 +257,6 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
             const long long tw = dbg ? clock64() : 0;
             mbar_wait(&w_empty[s], ph ^ 1);
             if (dbg) t_wait += clock64() - tw;
-            if (p.ablate & 4) { mbar_arrive(&w_full[s]); continue; }
             mbar_arrive_expect_tx(&w_full[s], stage_bytes);
             // taps are consumed centre first (kTapOrder): the centre tap is the one no edge mask applies to, so it is
             // the MMA that initialises every row of the accumulator
@@ -324,11 +315,8 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
       uint32_t acc = 0;
       uint32_t stage_no = 0;                    // weight stage within the tile (split-K: stage s belongs to warp s & 1)
       // rows of this accumulator that sit on a board edge (left / right column, top / bottom row), from the loader
-      uint4 eL = make_uint4(0, 0, 0, 0), eR = eL, eT = eL, eB = eL;
-      if (p.masked) {
-        const uint4* em = reinterpret_cast<const uint4*>(s_mask + (buf * 2 + (kSplitK ? 0 : (int)mhalf)) * 16);
-        eL = em[0]; eR = em[1]; eT = em[2]; eB = em[3];
-      }
+      const uint4* em = reinterpret_cast<const uint4*>(s_mask + (buf * 2 + (kSplitK ? 0 : (int)mhalf)) * 16);
+      const uint4 eL = em[0], eR = em[1], eT = em[2], eB = em[3];
       // one weight stage (a 64-channel K chunk of one tap): wait for it, issue its MMAs, release it, step the ring
       auto run_stage = [&](uint32_t a_lo, uint32_t m0, uint32_t m1, uint32_t m2, uint32_t m3) {
         if (kSplitK && (stage_no & 1u) != mhalf) {       // the other warp's stage: just step the ring
@@ -370,7 +358,7 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
         for (int ti = 0; ti < 9; ++ti) {
           const int tap = ti == 0 ? 4 : (ti <= 4 ? ti - 1 : ti);
           const int ky = tap / 3, kx = tap - 3 * ky;
-          const uint32_t a_tap = a_tile + (uint32_t)((ky - 1) * p.Wp + (kx - 1));   // wraps correctly: the shift may be negative
+          const uint32_t a_tap = a_tile + (uint32_t)((ky - 1) * p.W + (kx - 1));   // wraps correctly: the shift may be negative
           // output rows whose (y + ky - 1, x + kx - 1) neighbour is across a board edge take no part in this tap
           const uint32_t m0 = (kx == 0 ? eL.x : 0u) | (kx == 2 ? eR.x : 0u) | (ky == 0 ? eT.x : 0u) | (ky == 2 ? eB.x : 0u);
           const uint32_t m1 = (kx == 0 ? eL.y : 0u) | (kx == 2 ? eR.y : 0u) | (ky == 0 ? eT.y : 0u) | (ky == 2 ? eB.y : 0u);
@@ -435,20 +423,18 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
           *reinterpret_cast<float4*>(s_bias + (l & 3) * kN + c4 * 4) = __ldg(reinterpret_cast<const float4*>(L.bias) + c4);
         bias_layer = l;
       }
-      if (p.masked) {
-        // which rows of this tile are a board's left / right column or top / bottom row: one ballot per 32 rows
-        for (int h = 0; h < kRows / 128; ++h)
-          for (int w = 0; w < 4; ++w) {
-            const int P = tile * p.tile_stride + h * 128 + w * 32 + lane;
-            const int q = P % p.PB, y = q / p.Wp, x = q - y * p.Wp;
-            const unsigned mL = __ballot_sync(0xffffffffu, x == 0), mR = __ballot_sync(0xffffffffu, x == p.W - 1);
-            const unsigned mT = __ballot_sync(0xffffffffu, y == 0), mB = __ballot_sync(0xffffffffu, y == p.H - 1);
-            if (lane == 0) {
-              uint32_t* m = s_mask + (buf * 2 + h) * 16;
-              m[w] = mL; m[4 + w] = mR; m[8 + w] = mT; m[12 + w] = mB;
-            }
+      // which rows of this tile are a board's left / right column or top / bottom row: one ballot per 32 rows
+      for (int h = 0; h < kRows / 128; ++h)
+        for (int w = 0; w < 4; ++w) {
+          const int P = tile * p.tile_stride + h * 128 + w * 32 + lane;
+          const int q = P % p.PB, y = q / p.W, x = q - y * p.W;
+          const unsigned mL = __ballot_sync(0xffffffffu, x == 0), mR = __ballot_sync(0xffffffffu, x == p.W - 1);
+          const unsigned mT = __ballot_sync(0xffffffffu, y == 0), mB = __ballot_sync(0xffffffffu, y == p.H - 1);
+          if (lane == 0) {
+            uint32_t* m = s_mask + (buf * 2 + h) * 16;
+            m[w] = mL; m[4 + w] = mR; m[8 + w] = mT; m[12 + w] = mB;
           }
-      }
+        }
       const uint32_t dst0 = smem_u32(sA) + (uint32_t)buf * a_bytes;
       if (handed_over) {          // nothing to load: bias and masks are staged, tell the MMA warps
         __syncwarp();
@@ -470,25 +456,21 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
         fence_proxy_async();
       }
       __syncwarp();
-      if (p.ablate & 2) {
-        if (lane == 0) mbar_arrive(&a_full[buf]);
+      if (lane == 0) mbar_arrive_expect_tx(&a_full[buf], (uint32_t)(hi - lo) * 16u * (uint32_t)cg);
+      __syncwarp();
+      if (!L.in_slots) {
+        for (int g = lane; g < cg; g += 32)
+          bulk_g2s_u32(dst0 + (uint32_t)(g * TP + (lo - r0)) * 16, L.in + ((size_t)g * p.plane_rows + lo) * 8,
+                       (uint32_t)(hi - lo) * 16u, &a_full[buf]);
       } else {
-        if (lane == 0) mbar_arrive_expect_tx(&a_full[buf], (uint32_t)(hi - lo) * 16u * (uint32_t)cg);
-        __syncwarp();
-        if (!L.in_slots) {
-          for (int g = lane; g < cg; g += 32)
-            bulk_g2s_u32(dst0 + (uint32_t)(g * TP + (lo - r0)) * 16, L.in + ((size_t)g * p.plane_rows + lo) * 8,
-                         (uint32_t)(hi - lo) * 16u, &a_full[buf]);
-        } else {
-          const int b_lo = lo / p.PB, nb = (hi - 1) / p.PB - b_lo + 1;
-          for (int k = lane; k < nb * cg; k += 32) {
-            const int bi = k / cg, g = k - bi * cg, b = b_lo + bi;
-            const int s0 = b * p.PB > lo ? b * p.PB : lo, s1 = (b + 1) * p.PB < hi ? (b + 1) * p.PB : hi;
-            const size_t slot = L.in_index ? (size_t)L.in_index[b] : (size_t)b;
-            bulk_g2s_u32(dst0 + (uint32_t)(g * TP + (s0 - r0)) * 16,
-                         L.in + ((slot * cg + g) * p.PB + (size_t)(s0 - b * p.PB)) * 8, (uint32_t)(s1 - s0) * 16u,
-                         &a_full[buf]);
-          }
+        const int b_lo = lo / p.PB, nb = (hi - 1) / p.PB - b_lo + 1;
+        for (int k = lane; k < nb * cg; k += 32) {
+          const int bi = k / cg, g = k - bi * cg, b = b_lo + bi;
+          const int s0 = b * p.PB > lo ? b * p.PB : lo, s1 = (b + 1) * p.PB < hi ? (b + 1) * p.PB : hi;
+          const size_t slot = L.in_index ? (size_t)L.in_index[b] : (size_t)b;
+          bulk_g2s_u32(dst0 + (uint32_t)(g * TP + (s0 - r0)) * 16,
+                       L.in + ((slot * cg + g) * p.PB + (size_t)(s0 - b * p.PB)) * 8, (uint32_t)(s1 - s0) * 16u,
+                       &a_full[buf]);
         }
       }
     }
@@ -529,26 +511,26 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
         constexpr int STEPS = NJ * NCW;
         int Pj[2];
         size_t Dj[2];                        // destination row of the output buffer
-        bool vj[2], inr[2];                  // real (non-halo) row / row that is stored at all
+        bool vj[2], inr[2];                  // row in range (of the batch and of this tile) / row that is stored
 #pragma unroll
         for (int j = 0; j < NJ; ++j) {
           Pj[j] = tile * p.tile_stride + j * 128 + quad * 32 + lane;
-          int b = 0, pos = 0; bool hl = true;
-          inr[j] = Pj[j] < p.Ptot && j * 128 + quad * 32 + lane < p.tile_stride;
-          if (inr[j]) split_pos(Pj[j], p, b, pos, hl);
-          vj[j] = !hl;
+          vj[j] = Pj[j] < p.Ptot && j * 128 + quad * 32 + lane < p.tile_stride;
+          inr[j] = vj[j];
           Dj[j] = (size_t)Pj[j];
+          int b, pos;                        // only used under p.sub; split here, ptxas then spills less at 128 registers
+          split_pos(Pj[j], p, b, pos);
           if (p.sub) {
             // stride-2 convolution (padding 1) == the stride-1 result at the even positions: store those rows
-            // on the half-size grid, drop the rest (the destination's halo is zeroed by the caller)
-            const int y = pos / p.Wp, x = pos - y * p.Wp;
+            // on the half-size grid, drop the rest
+            const int y = pos / p.W, x = pos - y * p.W;
             inr[j] = vj[j] && !((y | x) & 1);
-            Dj[j] = (size_t)b * p.out_PB + (size_t)(y >> 1) * p.out_Wp + (x >> 1);
+            Dj[j] = (size_t)b * p.out_PB + (size_t)(y >> 1) * p.out_W + (x >> 1);
           }
         }
         const size_t PRo = p.sub ? (size_t)p.out_plane_rows : PR;
         const int4* resp = reinterpret_cast<const int4*>(L.residual);
-        const bool has_res = resp != nullptr && !(p.ablate & 512);
+        const bool has_res = resp != nullptr;
         int4 ring[3][4];
         // step t of this warp -> (row half j, 32-column chunk c).  khalf: low 64 channels (chunks 0, 1 across the two
         // column-half warps) of every row first, so that they can be handed to the next layer's first K chunk early
@@ -576,7 +558,7 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
         mbar_wait(&mma_done[buf], (uint32_t)((k >> 1) & 1));
         if (dbg) t_wait += clock64() - tw;
         tc_fence_after();
-        if (has_cols && !(p.ablate & 1)) {
+        if (has_cols) {
           int4* outp = reinterpret_cast<int4*>(L.out);
 #pragma unroll
           for (int t = 0; t < STEPS; ++t) {
@@ -596,13 +578,10 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
             float v[32];
             finish32(r, s_bias_l + c0, ring[t % 3], v);
             // ReLU (every conv of these nets is followed by one) and fp16 saturation ride on the fp32 -> fp16
-            // conversion; halo rows are stored as ZERO
-            if (pick(inr, j) && !(p.ablate & 512)) {
+            // conversion
+            if (pick(inr, j)) {
 #pragma unroll
-              for (int u = 0; u < 4; ++u) {
-                const int4 o4 = pack8_relu(v + 8 * u);
-                outp[(size_t)(c * 4 + u) * PRo + pick(Dj, j)] = pick(vj, j) ? o4 : make_int4(0, 0, 0, 0);
-              }
+              for (int u = 0; u < 4; ++u) outp[(size_t)(c * 4 + u) * PRo + pick(Dj, j)] = pack8_relu(v + 8 * u);
             }
             if (hand == 1) {
 #pragma unroll
@@ -622,15 +601,13 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
         if (dbg) t_wait += clock64() - tw;
         tc_fence_after();
 #pragma unroll 1
-        for (int j = 0; j < kRows / 128 && !(p.ablate & 1); ++j) {
+        for (int j = 0; j < kRows / 128; ++j) {
           const int P = tile * p.tile_stride + j * 128 + quad * 32 + lane;
-          int b = 0, pos = 0; bool hl = true;
+          int b = 0, pos = 0;
           const bool inrange = P < p.Ptot && j * 128 + quad * 32 + lane < p.tile_stride;
-          if (inrange) split_pos(P, p, b, pos, hl);
-          const bool valid = !hl;
-          const float top = valid ? 65504.0f : 0.0f;
-          const float* tab = (L.tab && valid) ? L.tab + ((size_t)L.action[b] * p.tab_groups * p.PB + pos) * 8 : nullptr;
-          const int4* resp = (L.residual && valid) ? reinterpret_cast<const int4*>(L.residual) + P : nullptr;
+          if (inrange) split_pos(P, p, b, pos);
+          const float* tab = (L.tab && inrange) ? L.tab + ((size_t)L.action[b] * p.tab_groups * p.PB + pos) * 8 : nullptr;
+          const int4* resp = (L.residual && inrange) ? reinterpret_cast<const int4*>(L.residual) + P : nullptr;
           // conv + bias (+ table) (+ residual) + ReLU of one 32-column chunk of this row (one chunk live at a
           // time keeps the register count of the whole kernel low; the normalising layers read TMEM twice)
           auto chunk = [&](int c, float (&v)[32]) {
@@ -659,9 +636,10 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
               }
             }
 #pragma unroll
-            for (int e = 0; e < 32; ++e) v[e] = fminf(fmaxf(v[e], 0.0f), top);
+            for (int e = 0; e < 32; ++e) v[e] = fminf(fmaxf(v[e], 0.0f), inrange ? 65504.0f : 0.0f);
           };
           float mn = INFINITY, mx = -INFINITY;
+          int4* o = (L.out && inrange) ? reinterpret_cast<int4*>(L.out) + P : nullptr;
           if (has_cols) {
 #pragma unroll 1
             for (int cc = 0; cc < NCW; ++cc) {
@@ -671,8 +649,7 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
 #pragma unroll
               for (int e = 0; e < 32; ++e)
                 if (c * 32 + e < p.n_real) { mn = fminf(mn, v[e]); mx = fmaxf(mx, v[e]); }
-              if (L.out && inrange) {
-                int4* o = reinterpret_cast<int4*>(L.out) + P;
+              if (o) {
 #pragma unroll
                 for (int u = 0; u < 4; ++u) o[(size_t)(c * 4 + u) * PR] = pack8(v + 8 * u);
               }
@@ -690,7 +667,7 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
             const float2 o = s_mm[(chalf ^ 1) * 128 + quad * 32 + lane];
             quad_bar_sync(quad);
             mn = fminf(mn, o.x); mx = fmaxf(mx, o.y);
-            const float inv = valid ? 1.0f / ((mx - mn) + 1e-8f) : 0.0f;
+            const float inv = inrange ? 1.0f / ((mx - mn) + 1e-8f) : 0.0f;
             if (has_cols) {             // warp-uniform: the TMEM loads inside chunk() are warp-collective
               int4* on = (L.out_norm && inrange) ? reinterpret_cast<int4*>(L.out_norm) + P : nullptr;
               int4* os = nullptr;
@@ -744,23 +721,22 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
 // ---------------------------------------------------------------------------
 // small SIMT kernels: observation packing, heads, weight repacking
 // ---------------------------------------------------------------------------
-// obs f32 [B][C][H][W] -> fp16 planes [cpad/8][plane_rows][8] (zeros at halo positions and padded channels)
+// obs f32 [B][C][H][W] -> fp16 planes [cpad/8][plane_rows][8] (zeros at padded channels)
 __global__ void pack_obs_kernel(const float* __restrict__ obs, act_t* __restrict__ out, int B, int C, int H,
-                                int W, int cpad, int plane_rows, int pad) {
+                                int W, int cpad, int plane_rows) {
   // one thread per (channel group, row): 8 plane reads that are each coalesced across the threads of a warp
   // (consecutive x), one 16-byte store
-  const int Wp = W + pad, PB = (H + pad) * Wp;
+  const int PB = H * W;
   const size_t rows = (size_t)B * PB, n = rows * (cpad / 8);
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
     const size_t P = i % rows;
     const int g = (int)(i / rows);
     const int pos = (int)(P % PB), b = (int)(P / PB);
-    const int y = pos / Wp, x = pos % Wp;
     float v[8];
 #pragma unroll
     for (int e = 0; e < 8; ++e) {
       const int c = g * 8 + e;
-      v[e] = (c < C && y < H && x < W) ? obs[(((size_t)b * C + c) * H + y) * W + x] : 0.0f;
+      v[e] = c < C ? obs[((size_t)b * C + c) * PB + pos] : 0.0f;
       v[e] = fminf(fmaxf(v[e], -65504.0f), 65504.0f);
     }
     reinterpret_cast<int4*>(out)[(size_t)g * plane_rows + P] = pack8(v);
@@ -771,38 +747,23 @@ __global__ void pack_obs_kernel(const float* __restrict__ obs, act_t* __restrict
 // then k constant action planes): frames u8 [B][K][H][W] + plane values f32 [B][K] -> the planes pack_obs_kernel would
 // produce from the float32 [B][2K][H][W] observation (0..255 are exact in fp16), at a quarter of the bytes.
 __global__ void pack_frames_kernel(const uint8_t* __restrict__ frames, const float* __restrict__ planes,
-                                   act_t* __restrict__ out, int B, int K, int H, int W, int cpad, int plane_rows, int pad) {
-  const int Wp = W + pad, PB = (H + pad) * Wp;
+                                   act_t* __restrict__ out, int B, int K, int H, int W, int cpad, int plane_rows) {
+  const int PB = H * W;
   const size_t rows = (size_t)B * PB, n = rows * (cpad / 8);
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
     const size_t P = i % rows;
     const int g = (int)(i / rows);
     const int pos = (int)(P % PB), b = (int)(P / PB);
-    const int y = pos / Wp, x = pos % Wp;
-    const bool real = y < H && x < W;
     float v[8];
 #pragma unroll
     for (int e = 0; e < 8; ++e) {
       const int c = g * 8 + e;
       float f = 0.0f;
-      if (real && c < K) f = (float)frames[(((size_t)b * K + c) * H + y) * W + x];
-      else if (real && c < 2 * K) f = fminf(fmaxf(planes[(size_t)b * K + (c - K)], -65504.0f), 65504.0f);
+      if (c < K) f = (float)frames[((size_t)b * K + c) * PB + pos];
+      else if (c < 2 * K) f = fminf(fmaxf(planes[(size_t)b * K + (c - K)], -65504.0f), 65504.0f);
       v[e] = f;
     }
     reinterpret_cast<int4*>(out)[(size_t)g * plane_rows + P] = pack8(v);
-  }
-}
-
-// zeros at the halo positions of a planar buffer (after the SIMT kernels that only write real positions)
-__global__ void zero_halo_kernel(act_t* __restrict__ buf, int B, int H, int W, int cg, int plane_rows) {
-  const int Wp = W + 1, PB = (H + 1) * Wp, nh = H + Wp;       // (padded layout only)       // halo positions per board: column W of rows 0..H-1, row H
-  const size_t n = (size_t)cg * B * nh;
-  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
-    const int k = (int)(i % nh);
-    const size_t r = i / nh;
-    const int b = (int)(r % B), g = (int)(r / B);
-    const int pos = k < H ? k * Wp + W : H * Wp + (k - H);
-    reinterpret_cast<int4*>(buf)[(size_t)g * plane_rows + (size_t)b * PB + pos] = make_int4(0, 0, 0, 0);
   }
 }
 
@@ -817,7 +778,7 @@ struct HeadParams {
   const float* w2;            // [out][mid*hw]
   const float* b2;            // [out]
   float* dst;                 // [B] or [B][out]
-  int C, H, W, pad, mid, out, kind;
+  int C, H, W, mid, out, kind;
 };
 
 __device__ __forceinline__ float signed_parabolic_f(float x) {
@@ -840,15 +801,14 @@ struct HeadsParams {
 __global__ void __launch_bounds__(128) head_kernel(const __grid_constant__ HeadsParams hp) {
   const HeadParams& p = hp.h[blockIdx.y];
   extern __shared__ float hs[];            // f[mid*hw] | logits[out]
-  const int hw = p.H * p.W, Wp = p.W + p.pad, PB = (p.H + p.pad) * Wp;
+  const int hw = p.H * p.W;
   float* f = hs;
   float* lg = hs + p.mid * hw;
   const int b = blockIdx.x;
-  const int4* a = reinterpret_cast<const int4*>(p.act) + (size_t)b * PB;
+  const int4* a = reinterpret_cast<const int4*>(p.act) + (size_t)b * hw;
   for (int i = threadIdx.x; i < p.mid * hw; i += blockDim.x) {
     const int m = i / hw, q = i % hw;
-    const int y = q / p.W, x = q % p.W;
-    const int4* row = a + (y * Wp + x);
+    const int4* row = a + q;
     const float* w = p.w1 + (size_t)m * p.C;
     float acc = 0.0f;
     for (int c = 0; c < p.C; c += 8) {
@@ -954,8 +914,8 @@ __global__ void scale_rows_kernel(const float* w, const float* scale, float* out
 // 1 iff f % A == action), so their contribution is tab[a][pos][n] = scale[n] * sum over
 // (plane c, tap) of w[n][C + c][tap] * E_a[c][y+ky-1][x+kx-1].
 __global__ void action_table_kernel(const float* __restrict__ w, const float* __restrict__ scale,
-                                    float* __restrict__ tab, int A, int C, int N, int n_real, int H, int W, int pad) {
-  const int Wp = W + pad, PB = (H + pad) * Wp, hw = H * W;
+                                    float* __restrict__ tab, int A, int C, int N, int n_real, int H, int W) {
+  const int PB = H * W;
   const size_t total = (size_t)A * PB * N;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
     // table layout [A][N/8][PB][8]: the epilogue (lane = row) reads 32 contiguous bytes per channel group
@@ -964,15 +924,15 @@ __global__ void action_table_kernel(const float* __restrict__ w, const float* __
     const int g = (int)((i / ((size_t)8 * PB)) % (N / 8));
     const int a = (int)(i / ((size_t)N * PB));
     const int n = g * 8 + e;
-    const int y = pos / Wp, x = pos % Wp;
+    const int y = pos / W, x = pos % W;
     float acc = 0.0f;
-    if (y < H && x < W && n < n_real) {
+    if (n < n_real) {
       for (int c = 0; c < A; ++c)
         for (int ky = 0; ky < 3; ++ky)
           for (int kx = 0; kx < 3; ++kx) {
             const int yy = y + ky - 1, xx = x + kx - 1;
             if (yy < 0 || yy >= H || xx < 0 || xx >= W) continue;
-            const int fidx = c * hw + yy * W + xx;
+            const int fidx = c * PB + yy * W + xx;
             if (fidx % A == a) acc += w[(((size_t)n * (C + A) + C + c) * 3 + ky) * 3 + kx];
           }
       acc *= scale[n];
@@ -994,52 +954,50 @@ __global__ void action_table_kernel(const float* __restrict__ w, const float* __
 __global__ void __launch_bounds__(256) avgpool_kernel(const act_t* __restrict__ in, act_t* __restrict__ out,
                                                       act_t* __restrict__ slots, const int32_t* __restrict__ out_index,
                                                       int B, int Hi, int Wi, int normalise, int rows_in, int rows_out,
-                                                      int pad, int C) {
-  const int Ho = Hi / 2, Wo = Wi / 2, Wpi = Wi + pad, PBi = (Hi + pad) * Wpi, Wpo = Wo + pad, PBo = (Ho + pad) * Wpo;
+                                                      int C) {
+  const int Ho = Hi / 2, Wo = Wi / 2, PBi = Hi * Wi, PBo = Ho * Wo;
   const int lane = threadIdx.x & 31;
   const int g0 = lane >> 1, off = (lane & 1) * 4;     // channel-group plane and offset of this lane's 4 channels
   const int nblk = C / 128;                           // 128-channel blocks (<= 2)
-  const long long total = (long long)B * PBo;         // halo positions included: they are written as zeros
+  const long long total = (long long)B * PBo;
   for (long long i = (long long)blockIdx.x * 8 + (threadIdx.x >> 5); i < total; i += (long long)gridDim.x * 8) {
-    const int b = (int)(i / PBo), pos = (int)(i % PBo), oy = pos / Wpo, ox = pos % Wpo;
+    const int b = (int)(i / PBo), pos = (int)(i % PBo), oy = pos / Wo, ox = pos % Wo;
     float s[2][4] = {{0.f, 0.f, 0.f, 0.f}, {0.f, 0.f, 0.f, 0.f}};
-    if (oy < Ho && ox < Wo) {
-      for (int ky = 0; ky < 3; ++ky)
-        for (int kx = 0; kx < 3; ++kx) {
-          const int iy = 2 * oy + ky - 1, ix = 2 * ox + kx - 1;
-          if (iy < 0 || iy >= Hi || ix < 0 || ix >= Wi) continue;
+    for (int ky = 0; ky < 3; ++ky)
+      for (int kx = 0; kx < 3; ++kx) {
+        const int iy = 2 * oy + ky - 1, ix = 2 * ox + kx - 1;
+        if (iy < 0 || iy >= Hi || ix < 0 || ix >= Wi) continue;
 #pragma unroll
-          for (int k = 0; k < 2; ++k) {
-            if (k >= nblk) break;
-            const int g = g0 + 16 * k;
-            const uint2 v = *reinterpret_cast<const uint2*>(in + ((size_t)g * rows_in + (size_t)b * PBi + (size_t)iy * Wpi + ix) * 8 + off);
-            const float2 f0 = __half22float2(*reinterpret_cast<const act2_t*>(&v.x));
-            const float2 f1 = __half22float2(*reinterpret_cast<const act2_t*>(&v.y));
-            s[k][0] += f0.x; s[k][1] += f0.y; s[k][2] += f1.x; s[k][3] += f1.y;
-          }
+        for (int k = 0; k < 2; ++k) {
+          if (k >= nblk) break;
+          const int g = g0 + 16 * k;
+          const uint2 v = *reinterpret_cast<const uint2*>(in + ((size_t)g * rows_in + (size_t)b * PBi + (size_t)iy * Wi + ix) * 8 + off);
+          const float2 f0 = __half22float2(*reinterpret_cast<const act2_t*>(&v.x));
+          const float2 f1 = __half22float2(*reinterpret_cast<const act2_t*>(&v.y));
+          s[k][0] += f0.x; s[k][1] += f0.y; s[k][2] += f1.x; s[k][3] += f1.y;
         }
+      }
+#pragma unroll
+    for (int k = 0; k < 2; ++k)
+#pragma unroll
+      for (int j = 0; j < 4; ++j) s[k][j] *= (1.0f / 9.0f);
+    if (normalise) {
+      float mn = INFINITY, mx = -INFINITY;
+#pragma unroll
+      for (int k = 0; k < 2; ++k)
+        if (k < nblk)
+#pragma unroll
+          for (int j = 0; j < 4; ++j) { mn = fminf(mn, s[k][j]); mx = fmaxf(mx, s[k][j]); }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) {
+        mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, o));
+        mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+      }
+      const float inv = 1.0f / ((mx - mn) + 1e-8f);
 #pragma unroll
       for (int k = 0; k < 2; ++k)
 #pragma unroll
-        for (int j = 0; j < 4; ++j) s[k][j] *= (1.0f / 9.0f);
-      if (normalise) {
-        float mn = INFINITY, mx = -INFINITY;
-#pragma unroll
-        for (int k = 0; k < 2; ++k)
-          if (k < nblk)
-#pragma unroll
-            for (int j = 0; j < 4; ++j) { mn = fminf(mn, s[k][j]); mx = fmaxf(mx, s[k][j]); }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-          mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, o));
-          mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-        }
-        const float inv = 1.0f / ((mx - mn) + 1e-8f);
-#pragma unroll
-        for (int k = 0; k < 2; ++k)
-#pragma unroll
-          for (int j = 0; j < 4; ++j) s[k][j] = (s[k][j] - mn) * inv;
-      }
+        for (int j = 0; j < 4; ++j) s[k][j] = (s[k][j] - mn) * inv;
     }
 #pragma unroll
     for (int k = 0; k < 2; ++k) {
@@ -1115,18 +1073,10 @@ struct Head {
   const float *w1, *b1, *w2, *b2;
   int mid, out, kind;
 };
-// Grid padding.  0 (default): boards are stored without halo, H*W rows each, and the conv kernel masks the taps that
-// would reach over a board edge with tcgen05.mma's disable-output-lane vector (no MMA row is spent on padding).
-// 1: the first layout of this kernel -- one zero column / row shared between neighbours, (H+1)*(W+1) rows per board,
-// every tap unmasked (19 % of the rows of a 9x9 board, 27 % of a 6x6 latent, are halo).  MZ_CONV_PAD=1 selects it.
-static int grid_pad() {
-  static const int pad = getenv("MZ_CONV_PAD") ? (atoi(getenv("MZ_CONV_PAD")) != 0) : 0;
-  return pad;
-}
+// A board grid: H*W rows per board (the layout at the top of this file).
 struct Geo {
   int H, W;
-  int Wp() const { return W + grid_pad(); }
-  int PB() const { return (H + grid_pad()) * (W + grid_pad()); }
+  int PB() const { return H * W; }
 };
 // channels as the kernels see them: num_planes rounded up to a multiple of 32 (the reference's ResNet Tic-Tac-Toe
 // variant has 16, config.py:126-127); the extra channels have zero weights and zero bias everywhere
@@ -1152,7 +1102,7 @@ struct ConvNet : NetImpl {
   size_t flags_cap;
   int* err_flag;
 
-  static int tp_of(const Geo& g, int rows = kTileM) { return (rows + 2 * (g.Wp() + 1)) | 1; }
+  static int tp_of(const Geo& g, int rows = kTileM) { return (rows + 2 * (g.W + 1)) | 1; }
   // rows of one channel-group plane of a contiguous activation buffer holding `batch` boards of grid g
   static int plane_rows_of(const Geo& g, int batch) {
     return (batch * g.PB() + kTileM - 1) / kTileM * kTileM + kPlaneSlack;
@@ -1168,9 +1118,7 @@ struct ConvNet : NetImpl {
     const size_t stage = (size_t)chunk_g * n * 16;
     const size_t fixed = conv_fixed_smem(g, cg, n, rows);
     if (fixed + 2 * stage > 227 * 1024) return 0;
-    int s = (int)((227 * 1024 - fixed) / stage);
-    static const int cap = getenv("MZ_CONV_MAX_STAGES") ? atoi(getenv("MZ_CONV_MAX_STAGES")) : kMaxStages;
-    if (s > cap && cap >= 2) s = cap;
+    const int s = (int)((227 * 1024 - fixed) / stage);
     return s > kMaxStages ? kMaxStages : s;
   }
   static size_t conv_smem(const Geo& g, int cg, int n, int rows) {
@@ -1246,13 +1194,13 @@ struct ConvNet : NetImpl {
     const Geo g = pend_geo;
     const int batch = pend_batch, cg = pend_cg, nl = p.num_layers, N = p.N;
     const bool multi_pass = p.tab_groups * 8 > 128;
-    p.PB = g.PB(); p.Wp = g.Wp(); p.W = g.W; p.H = g.H; p.B = batch;
+    p.PB = g.PB(); p.W = g.W; p.H = g.H; p.B = batch;
     p.Ptot = batch * p.PB;
     p.plane_rows = plane_rows_of(g, batch);
     p.sub = pend_sub ? 1 : 0;
     {
       const Geo go{g.H / 2, g.W / 2};
-      p.out_plane_rows = plane_rows_of(go, batch); p.out_PB = go.PB(); p.out_Wp = go.Wp();
+      p.out_plane_rows = plane_rows_of(go, batch); p.out_PB = go.PB(); p.out_W = go.W;
     }
     p.cg = cg; p.relu = 1;
     // Few tiles per SM (small batches / small grids): a multi-layer launch is bound by the dependency chain between
@@ -1262,23 +1210,21 @@ struct ConvNet : NetImpl {
     const int force_rows = force_env ? atoi(force_env) : 0;
     int rows = (nl > 1 && (p.Ptot + kTileM - 1) / kTileM < 2 * num_sms) ? 128 : kTileM;
     if (force_rows == 128 || force_rows == 256) rows = force_rows;
-    p.masked = grid_pad() == 0;
     // split-K tiles give the second MMA warp the odd weight stages; with one stage per tap its first MMA would be a
     // masked (non-centre) tap and could not initialise its accumulator
-    if (p.masked && cg <= 8) rows = kTileM;
+    if (cg <= 8) rows = kTileM;
     // 256 input channels: two 256-row activation buffers do not fit shared memory
     if (!fits(g, cg, N, rows)) rows = rows == kTileM ? 128 : kTileM;
     // RESIDENT launch: when every CTA can own one tile of whole boards for all layers, nothing a tile needs comes from
-    // another tile (the halo-free layout masks every tap that leaves a board), so the layers of a tower hand their
-    // activations over in shared memory -- no tile flags, no tile loads, no waiting for neighbours after layer 0.
+    // another tile (every tap that leaves a board is masked), so the layers of a tower hand their activations over
+    // in shared memory -- no tile flags, no tile loads, no waiting for neighbours after layer 0.
     // This is the regime of small batches and small grids (single-tree searches, the 6x6 Atari latent), where a
     // launch is bound by the chain flag -> load -> MMA -> epilogue -> publish of every layer, not by throughput.
     const int sm_cap0 = (cta_limit > 0 && cta_limit < num_sms) ? cta_limit : num_sms;
     p.resident = 0;
     p.khalf = 0;
     p.tile_stride = rows;
-    static const bool no_resident = getenv("MZ_CONV_NO_RESIDENT") != nullptr;
-    if (p.masked && nl > 1 && !p.sub && !no_resident && !multi_pass) {
+    if (nl > 1 && !p.sub && !multi_pass) {
       bool chain = true;
       for (int i = 0; i + 1 < nl && chain; ++i) {
         LayerDesc& a = pend.L[i];
@@ -1297,8 +1243,7 @@ struct ConvNet : NetImpl {
           if (bpt < 1) continue;
           if ((batch + bpt - 1) / bpt > sm_cap0) continue;
           p.resident = 1; rows = rr; p.tile_stride = bpt * p.PB;
-          static const bool no_khalf = getenv("MZ_CONV_NO_KHALF") != nullptr;
-          p.khalf = (rr == kTileM && cg == 16 && !no_khalf) ? 1 : 0;
+          p.khalf = (rr == kTileM && cg == 16) ? 1 : 0;
         }
       }
     }
@@ -1319,8 +1264,6 @@ struct ConvNet : NetImpl {
       if (e != cudaSuccess) { reset_pending(); set_error("cudaMemsetAsync: %s", cudaGetErrorString(e)); return MZ_ECUDA; }
     }
     p.dbg = nullptr;
-    static const int ablate = getenv("MZ_CONV_ABLATE") ? atoi(getenv("MZ_CONV_ABLATE")) : 0;
-    p.ablate = ablate;
     static const bool debug = getenv("MZ_CONV_DEBUG") != nullptr;
     if (debug) cudaMalloc(&p.dbg, (size_t)grid * 16 * sizeof(long long));
     prof_mark(kProfConv, st, multi_pass ? (nl + 1) / 2 : nl);       // counted in convolutions, not passes
@@ -1332,8 +1275,7 @@ struct ConvNet : NetImpl {
       lc.gridDim = dim3((unsigned)grid); lc.blockDim = dim3(kConvThreads); lc.dynamicSmemBytes = smem; lc.stream = st;
       cudaLaunchAttribute at[1];
       at[0].id = cudaLaunchAttributeCooperative;
-      static const bool noncoop = getenv("MZ_CONV_NONCOOP") != nullptr;     // scheduling experiments only
-      at[0].val.cooperative = (nl > 1 && !noncoop) ? 1 : 0;
+      at[0].val.cooperative = nl > 1 ? 1 : 0;
       lc.attrs = at; lc.numAttrs = 1;
       cudaError_t le;
       if (rows == 256) {
@@ -1372,7 +1314,7 @@ struct ConvNet : NetImpl {
     HeadParams& p = pend_heads.h[num_pend_heads++];
     p.act = act; p.w1 = h.w1; p.b1 = h.b1; p.w2 = h.w2; p.b2 = h.b2; p.dst = dst;
     p.plane_rows = plane_rows_of(lat, batch);
-    p.C = Creal; p.H = lat.H; p.W = lat.W; p.pad = grid_pad(); p.mid = h.mid; p.out = h.out; p.kind = h.kind;
+    p.C = Creal; p.H = lat.H; p.W = lat.W; p.mid = h.mid; p.out = h.out; p.kind = h.kind;
     const size_t smem = ((size_t)h.mid * lat.H * lat.W + h.out) * 4;
     if (smem > pend_heads_smem) pend_heads_smem = smem;
   }
@@ -1425,10 +1367,9 @@ struct ConvNet : NetImpl {
       // contents (the block's first conv, tiles t-1..t+1) has published before this tile starts.  Two live buffers per
       // tower instead of three: two engines' activations (2 x 2 x 21 MB for 1024 Gomoku boards) then fit the 126 MB L2,
       // where three per engine (126 MB + weights + trees) were evicted to DRAM between a layer's write and its rewrite.
-      static const bool no_inplace = getenv("MZ_CONV_NO_INPLACE") != nullptr;
       act_t* dst = pp[which];
       if (dst == cur) dst = pp[which ^ 1];
-      if (!no_inplace && (cur == b0 || cur == b1 || cur == b3)) dst = const_cast<act_t*>(cur);
+      if (cur == b0 || cur == b1 || cur == b3) dst = const_cast<act_t*>(cur);
       if (last && raw_dst) dst = raw_dst;
       rc = add_conv(blk[2 * i + 1], g, b2, nullptr, false, batch, nullptr, nullptr, cur,
                     (last && normalise && !keep_raw) ? nullptr : dst, (last && !late_norm) ? norm_out : nullptr,
@@ -1456,42 +1397,35 @@ struct ConvNet : NetImpl {
     prof_mark(kProfPack, st);
     if (frames)
       pack_frames_kernel<<<num_sms * 8, 256, 0, st>>>(frames, plane_values, xobs, batch, cfg.in_channels / 2, Hin, Win, 16,
-                                                      plane_rows_of(g0, batch), grid_pad());
+                                                      plane_rows_of(g0, batch));
     else
-      pack_obs_kernel<<<num_sms * 8, 256, 0, st>>>(obs, xobs, batch, cfg.in_channels, Hin, Win, 16, plane_rows_of(g0, batch), grid_pad());
+      pack_obs_kernel<<<num_sms * 8, 256, 0, st>>>(obs, xobs, batch, cfg.in_channels, Hin, Win, 16, plane_rows_of(g0, batch));
     prof_mark(-1, st);
     MZ_LAUNCH_CHECK("pack_obs_kernel");
     // stride-2 conv + ReLU: one tcgen05 launch at the input resolution whose epilogue stores the even positions on
-    // the half-size grid; then the halo of that grid is zeroed
-    auto s2 = [&](const ConvLayer& L, const act_t* in, act_t* out, const Geo& gi, const Geo& go) -> int {
+    // the half-size grid
+    auto s2 = [&](const ConvLayer& L, const act_t* in, act_t* out, const Geo& gi) -> int {
       int rc2 = add_conv(L, gi, in, nullptr, false, batch, nullptr, nullptr, nullptr, out, nullptr, nullptr, nullptr, st, true);
       if (rc2) return rc2;
-      if ((rc2 = flush(st))) return rc2;
-      if (grid_pad()) {
-        prof_mark(kProfPack, st);
-        zero_halo_kernel<<<num_sms * 4, 256, 0, st>>>(out, batch, go.H, go.W, L.n_out / 8, plane_rows_of(go, batch));
-        prof_mark(-1, st);
-        MZ_LAUNCH_CHECK("zero_halo_kernel");
-      }
-      return MZ_OK;
+      return flush(st);
     };
     auto pool = [&](const act_t* in, act_t* out, act_t* sl, const int32_t* idx, const Geo& gi, const Geo& go, int norm) -> int {
       prof_mark(kProfPack, st);
       avgpool_kernel<<<num_sms * 8, 256, 0, st>>>(in, out, sl, idx, batch, gi.H, gi.W, norm, plane_rows_of(gi, batch),
-                                                  plane_rows_of(go, batch), grid_pad(), C);
+                                                  plane_rows_of(go, batch), C);
       prof_mark(-1, st);
       MZ_LAUNCH_CHECK("avgpool_kernel");
       return MZ_OK;
     };
     act_t* fin;
     int rc;
-    // every writer rewrites the halo of the grid it produces, so grids of different sizes can reuse the same buffers
-    if ((rc = s2(s2_1, xobs, b0, g0, g1))) return rc;                                          // relu(conv_1)
+    // every writer writes every row of the grid it produces, so grids of different sizes can reuse the same buffers
+    if ((rc = s2(s2_1, xobs, b0, g0))) return rc;                                              // relu(conv_1)
     if ((rc = tower(nullptr, at_blocks[0], 2, g1, b0, nullptr, false, nullptr, nullptr, batch, true, nullptr, nullptr,
                     nullptr, st, &fin))) return rc;
     if ((rc = flush(st))) return rc;
     act_t* nxt = (fin == b0) ? b1 : b0;
-    if ((rc = s2(s2_2, fin, nxt, g1, g2))) return rc;                                          // relu(conv_2)
+    if ((rc = s2(s2_2, fin, nxt, g1))) return rc;                                              // relu(conv_2)
     if ((rc = tower(nullptr, at_blocks[1], 2, g2, nxt, nullptr, false, nullptr, nullptr, batch, true, nullptr, nullptr,
                     nullptr, st, &fin))) return rc;
     if ((rc = flush(st))) return rc;
@@ -1511,7 +1445,7 @@ struct ConvNet : NetImpl {
     } else {
       prof_mark(kProfPack, st);
       pack_obs_kernel<<<num_sms * 4, 256, 0, st>>>(obs, xobs, batch, cfg.in_channels, lat.H, lat.W, in_cg * 8,
-                                                   plane_rows_of(lat, batch), grid_pad());
+                                                   plane_rows_of(lat, batch));
       prof_mark(-1, st);
       MZ_LAUNCH_CHECK("pack_obs_kernel");
       act_t* fin;
@@ -1592,13 +1526,14 @@ int conv_hidden_bytes(const mz_net_config& c, int32_t* bytes) {
   int H, W;
   int rc = conv_geometry(c, &H, &W);
   if (rc) return rc;
-  *bytes = (H + grid_pad()) * (W + grid_pad()) * padded_planes(c.num_planes) * 2;
+  *bytes = H * W * padded_planes(c.num_planes) * 2;
   return MZ_OK;
 }
 
 static size_t conv_w_bytes(int cg, int N) { return align_up((size_t)9 * cg * N * 16, 256); }
 static int obs_cg(int cin) { return ((cin + 15) / 16) * 2; }
 
+// An upper bound on what conv_create takes: its grids are sized (H+1)(W+1), more than the H*W rows a board uses.
 int conv_arena_bytes(const mz_net_config& c, int max_batch, size_t* bytes) {
   int H, W;
   int rc = conv_geometry(c, &H, &W);
@@ -1740,7 +1675,7 @@ int conv_create(const mz_net_config& c, const float* const* w, int nw, int max_b
     float* scale = nullptr;
     MZ_TRY(fold_conv(Nreal, Nreal + A, N / 8, Nreal, N, &net->dyn0, &scale));
     float* tab = (float*)take((size_t)A * PB * N * 4);
-    action_table_kernel<<<512, 256>>>(dyn_w, scale, tab, A, Nreal, N, Nreal, H, W, grid_pad());
+    action_table_kernel<<<512, 256>>>(dyn_w, scale, tab, A, Nreal, N, Nreal, H, W);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) { set_error("action_table_kernel: %s", cudaGetErrorString(e)); delete net; return MZ_ECUDA; }
     count_launch();

@@ -7,7 +7,7 @@
 // and backward.  The heads (1x1 convolution, BatchNorm, ReLU, Linear) and the optimizer step are in optim.cu; the losses
 // and the two gradient-scale hooks stay PyTorch autograd (muzero_b200/train_engine.py, training.py).
 //
-// Layout: the padded channel-group planes of conv.cu (pad == 1): a board is (H+1)*(W+1) positions, column W and row H
+// Layout: padded channel-group planes: a board is (H+1)*(W+1) positions, position q = y*(W+1) + x, column W and row H
 // are a ZERO halo shared with the next row / board, an activation tensor is C/8 planes of [rows][8 channels] 16-bit.
 // With zeros at the halo every 3x3 tap is an unmasked constant row offset in all three GEMMs:
 //   forward   Y[P][co]    = sum_tap sum_ci  A[P + off(tap)][ci]  * W[co][ci][tap]          M = rows, N = co, K = 9*ci

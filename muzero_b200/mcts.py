@@ -556,7 +556,7 @@ def pipeline_shape(network, B: int):
     if network.kind == _lib.MZ_NET_MLP or B % 2:
         return 1, 0
     h, w = network.latent_hw
-    if (B // 2) * (h + network.grid_pad) * (w + network.grid_pad) >= 2 * 148 * 256:
+    if (B // 2) * h * w >= 2 * 148 * 256:
         return 2, 0
     return 1, 0
 

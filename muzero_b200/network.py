@@ -533,8 +533,7 @@ class _ConvNet(MuZeroNet):
                                '(self-play always does, pipeline.py:79-80)')
         return super()._engine_tensors()
 
-    # engine layout: fp16 planes of 8 channels, [Cp/8][(H+pad)*(W+pad)][8], pad = grid_pad, Cp = padded_planes
-    # (see csrc/conv.cu)
+    # engine layout: fp16 planes of 8 channels, [Cp/8][H*W][8], Cp = padded_planes (see csrc/conv.cu)
     @property
     def padded_planes(self) -> int:
         """Channels of a hidden-state slot: num_planes rounded up to a multiple of 32 (the kernels' minimum tile
@@ -544,24 +543,18 @@ class _ConvNet(MuZeroNet):
     def hidden_to_reference(self, slots):
         h, w = self.latent_hw
         c, cp = self.num_planes, self.padded_planes
-        pad = self.grid_pad
-        x = slots.view(torch.float16).reshape(slots.shape[0], cp // 8, h + pad, w + pad, 8)[:, :, :h, :w, :]
+        x = slots.view(torch.float16).reshape(slots.shape[0], cp // 8, h, w, 8)
         return x.permute(0, 1, 4, 2, 3).reshape(slots.shape[0], cp, h, w)[:, :c].to(torch.float32).contiguous()
 
-    @property
-    def grid_pad(self) -> int:
-        """0: boards stored without halo (the conv kernel masks the edge taps); 1: the padded (H+1)x(W+1) layout
-        (MZ_CONV_PAD=1).  Read off the engine's slot size so that this module never disagrees with the library."""
-        h, w = self.latent_hw
-        return 1 if self.hidden_bytes == (h + 1) * (w + 1) * self.padded_planes * 2 else 0
+    # Rows of padding around each board in the engine layout: none.  Kept because bench.py reads it.
+    grid_pad = 0
 
     def hidden_from_reference(self, hid):
         h, w = self.latent_hw
         c, cp = self.num_planes, self.padded_planes
         hid = hid.reshape(-1, c // 8, 8, h, w)
-        pad = self.grid_pad
-        out = torch.zeros((hid.shape[0], cp // 8, h + pad, w + pad, 8), dtype=torch.float16, device=hid.device)
-        out[:, :c // 8, :h, :w, :] = hid.permute(0, 1, 3, 4, 2).to(torch.float16)
+        out = torch.zeros((hid.shape[0], cp // 8, h, w, 8), dtype=torch.float16, device=hid.device)
+        out[:, :c // 8] = hid.permute(0, 1, 3, 4, 2).to(torch.float16)
         return out.reshape(hid.shape[0], -1).view(torch.uint8)
 
     # -- training: the towers run on the hand-written kernels of csrc/train.cu where they apply (train_engine.py) ------

@@ -147,17 +147,16 @@ def test_fma_division_sequence_is_correctly_rounded(tmp_path):
 
 
 def test_conv_hidden_slot_layout_round_trip_on_cpu():
-    """The engine's hidden-state slot of a conv net is [C/8][(H+pad)(W+pad)][8] fp16 with pad read off the library
-    (0: halo-free boards, the default; 1 under MZ_CONV_PAD=1): reference layout -> slot -> reference layout."""
+    """The engine's hidden-state slot of a conv net is [C/8][H*W][8] fp16, no padding around the board:
+    reference layout -> slot -> reference layout."""
     import muzero_b200 as mz
     net = mz.MuZeroBoardGameNet((9, 9, 9), 82, 1, 32)
-    pad = net.grid_pad
-    assert pad == (1 if os.environ.get('MZ_CONV_PAD', '0') not in ('', '0') else 0)
-    assert net.hidden_bytes == (9 + pad) * (9 + pad) * 32 * 2
+    assert net.grid_pad == 0
+    assert net.hidden_bytes == 9 * 9 * 32 * 2
     h = (torch.arange(2 * 32 * 81, dtype=torch.float32).reshape(2, 32, 9, 9) % 251) / 256.0    # fp16-exact values
     slots = net.hidden_from_reference(h)
     assert slots.dtype == torch.uint8 and tuple(slots.shape) == (2, net.hidden_bytes)
     assert torch.equal(net.hidden_to_reference(slots), h)
-    # element (q = y*(W+pad) + x, c) of a slot lives at ((c/8) * PB + q) * 8 + c % 8
-    v = slots.view(torch.float16).reshape(2, 4, (9 + pad) * (9 + pad), 8)
-    assert float(v[1, 2, 3 * (9 + pad) + 5, 7]) == float(h[1, 2 * 8 + 7, 3, 5])
+    # element (q = y*W + x, c) of a slot lives at ((c/8) * PB + q) * 8 + c % 8, PB = 81
+    v = slots.view(torch.float16).reshape(2, 4, 81, 8)
+    assert float(v[1, 2, 3 * 9 + 5, 7]) == float(h[1, 2 * 8 + 7, 3, 5])

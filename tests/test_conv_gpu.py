@@ -439,7 +439,7 @@ def test_new_board_shapes_batched_vs_torch_fp32(name, batch, nref, TOL_PV=TOL_PV
     report(f'{name} pi1', pi2[rows].cpu().numpy(), pi2_ref.numpy(), 0.05 if kw['num_res_blocks'] >= 16 else TOL_PV)
     assert (out.view(torch.float16)[0::2] == 0).all()        # untouched slots stay untouched
     if name == 'ttt_resnet':                                 # channels 16..31 of a slot are the zero padding
-        pb = (3 + net.grid_pad) ** 2
+        pb = 9
         raw = out.view(torch.float16).reshape(2 * batch + 1, 4, pb, 8)
         assert (raw[1::2, 2:] == 0).all()
 

@@ -6,8 +6,6 @@ timeout 1200 python -m pytest tests -m gpu -x -q 2>&1 | tail -15 > $O/${TAG}_pyt
 cat $O/${TAG}_pytest_gpu.log
 timeout 900 python bench.py --steps 5 --warmup 3 --no-cpu-baseline > $O/${TAG}_bench.json 2> $O/${TAG}_bench.err
 tail -2 $O/${TAG}_bench.err; python tools/show_bench.py $O/${TAG}_bench.json
-MZ_CONV_NO_INPLACE=1 timeout 600 python bench.py --steps 5 --warmup 3 --no-cpu-baseline --no-configs --no-train-step --no-self-play > $O/${TAG}_bench_noinplace.json 2>/dev/null
-python tools/show_bench.py $O/${TAG}_bench_noinplace.json
 timeout 600 ncu --set full --clock-control none --import-source on -k regex:backup_select_kernel -s 150 -c 1 -f -o $O/${TAG}_tree_gomoku \
     python tools/profile_target.py gomoku 200 1024 > $O/${TAG}_ncu_tree_gomoku.log 2>&1
 timeout 600 ncu --set full --clock-control none --import-source on -k regex:backup_select_kernel -s 20 -c 1 -f -o $O/${TAG}_tree_ttt262144 \

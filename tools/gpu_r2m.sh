@@ -1,11 +1,9 @@
 #!/bin/bash
-# full validation: GPU suite (+ layout / kernel variants), smoke, default bench, reference arm, sanitizer, launch list
+# full validation: GPU suite (+ kernel variants), smoke, default bench, reference arm, sanitizer, launch list
 TAG=${1:-r2m}
 O=gpurun_out; mkdir -p $O
 L=$O/${TAG}_pytest_gpu.log
 timeout 1500 python -m pytest tests -m gpu -x -q > $L 2>&1; echo "pytest exit $?" >> $L
-MZ_CONV_PAD=1 timeout 600 python -m pytest tests/test_conv_gpu.py -m gpu -x -q 2>&1 | tail -2 | sed 's/^/padded layout (MZ_CONV_PAD=1): /' >> $L
-MZ_CONV_NO_RESIDENT=1 timeout 600 python -m pytest tests/test_conv_gpu.py -m gpu -x -q 2>&1 | tail -2 | sed 's/^/no resident launches (MZ_CONV_NO_RESIDENT=1): /' >> $L
 MZ_TREE_THREAD=1 timeout 600 python -m pytest tests/test_mcts_gpu.py -m gpu -x -q 2>&1 | tail -2 | sed 's/^/thread-per-tree kernels forced for A <= 4 (MZ_TREE_THREAD=1): /' >> $L
 MZ_FUSED_SEARCH=0 MZ_NO_PDL=1 MZ_NO_FUSED_ROOT=1 timeout 600 python -m pytest tests/test_network_gpu.py tests/test_mcts_gpu.py -m gpu -x -q 2>&1 | tail -2 | sed 's/^/launch chain, no PDL, separate root launches: /' >> $L
 timeout 300 python -c "import __graft_entry__ as g; g.smoke()" >> $L 2>&1; echo "smoke exit $?" >> $L

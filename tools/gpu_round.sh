@@ -6,8 +6,6 @@ O=gpurun_out
 mkdir -p $O
 nvidia-smi --query-gpu=name,clocks.max.sm,power.limit --format=csv > $O/${TAG}_gpu.txt 2>&1
 timeout 600 python -m pytest tests -m gpu -x -q > $O/${TAG}_pytest_gpu.log 2>&1
-MZ_CONV_PAD=1 timeout 300 python -m pytest tests/test_conv_gpu.py -m gpu -x -q 2>&1 | tail -2 | sed 's/^/padded layout (MZ_CONV_PAD=1): /' >> $O/${TAG}_pytest_gpu.log
-MZ_CONV_NO_RESIDENT=1 timeout 300 python -m pytest tests/test_conv_gpu.py -m gpu -x -q 2>&1 | tail -2 | sed 's/^/no resident launches (MZ_CONV_NO_RESIDENT=1): /' >> $O/${TAG}_pytest_gpu.log
 MZ_TREE_THREAD=1 timeout 300 python -m pytest tests/test_mcts_gpu.py -m gpu -x -q 2>&1 | tail -2 | sed 's/^/thread-per-tree kernels forced for A <= 4 (MZ_TREE_THREAD=1): /' >> $O/${TAG}_pytest_gpu.log
 timeout 120 python -c "import __graft_entry__ as g; g.smoke()" >> $O/${TAG}_pytest_gpu.log 2>&1
 echo "pytest exit $?" >> $O/${TAG}_pytest_gpu.log
