@@ -82,6 +82,22 @@ inline cudaError_t launch_pdl(bool allow, void (*kernel)(KArgs...), dim3 grid, d
   lc.attrs = at; lc.numAttrs = 1;
   return cudaLaunchKernelEx(&lc, kernel, static_cast<KArgs>(args)...);
 }
+// the same with the grid launched as 2-CTA clusters when it has an even number of CTAs: a 2-CTA cluster is placed on
+// the two SMs of one TPC, so such a grid holds whole SM pairs and leaves every other pair to an SM-pair launch (the
+// conv towers) running beside it
+template <typename... KArgs, typename... Args>
+inline cudaError_t launch_pdl_pairs(bool allow, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem,
+                                    cudaStream_t st, Args... args) {
+  cudaLaunchConfig_t lc = {};
+  lc.gridDim = grid; lc.blockDim = block; lc.dynamicSmemBytes = smem; lc.stream = st;
+  cudaLaunchAttribute at[2];
+  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  at[0].val.programmaticStreamSerializationAllowed = (allow && pdl_enabled()) ? 1 : 0;
+  at[1].id = cudaLaunchAttributeClusterDimension;
+  at[1].val.clusterDim.x = 2; at[1].val.clusterDim.y = 1; at[1].val.clusterDim.z = 1;
+  lc.attrs = at; lc.numAttrs = grid.x % 2 == 0 ? 2 : 1;
+  return cudaLaunchKernelEx(&lc, kernel, static_cast<KArgs>(args)...);
+}
 
 }  // namespace mz
 

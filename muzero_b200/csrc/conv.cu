@@ -45,6 +45,7 @@ constexpr int kConvThreads = 384;   // w0 weights, w1 MMA (rows 0-127), w2 tile 
 constexpr int kEpiThreads = 256;
 constexpr int kTileM = 256;     // rows per tile (two M=128 accumulators)
 constexpr int kMaxStages = 6;
+constexpr int kMaxPairStages = 12;   // SM-pair launches: a ring slot holds half a stage
 constexpr int kPlaneSlack = 64; // rows allocated past the last tile of every plane (>= the widest halo)
 
 constexpr int kMaxLayers = 34;   // one launch runs up to a whole recurrent inference: 1 + 16 + 16 convs
@@ -56,6 +57,7 @@ struct LayerDesc {
   const act_t* in;        // planes [Cin/8][plane_rows][8], or the slot array when in_slots is set
   const int32_t* in_index;        // slot input: board b lives in slot in_index[b] (nullptr: slot b)
   const act_t* w;         // packed [9][chunks][chunk_g][N][8]
+  const act_t* w_pair;    // the same weights for SM-pair launches: [9][chunks][half][chunk_g][N/2][8]
   const float* bias;              // [N]
   const float* tab;               // [A][N/8][PB][8] per-action bias (dynamics conv0) or nullptr
   const int32_t* action;          // [B]
@@ -97,6 +99,13 @@ struct ConvParams {
                                   // and the epilogue hands the low / high 64 channels of the next tile over separately
   int resident;                   // every CTA owns ONE board-aligned tile for all layers; activations stay in shared memory
 };
+// SM-pair launches (kPair: 256-row dataflow launches of more than one stride-1 layer) run as 2-CTA clusters.  The
+// unit of work is a tile PAIR: pair item j of a layer is tiles 2j (even CTA) and 2j+1 (odd CTA; past the last tile it
+// is a null tile whose rows are neither read nor written, nor published), and pair items rotate over the clusters
+// per layer as tiles rotate over CTAs otherwise.  The even CTA issues tcgen05.mma.cta_group::2 M = 256 for both:
+// each SM reads its own 128 activation rows and HALF of the weight operand (6 KB instead of 8 KB of shared memory
+// per M128-equivalent MMA), and each SM streams only its half of every weight stage (half the ring fills and the L2
+// weight traffic).  Arithmetic and summation order are those of the single-CTA form.
 
 __device__ __forceinline__ void split_pos(int P, const ConvParams& p, int& b, int& q) {
   b = P / p.PB;
@@ -174,25 +183,32 @@ __device__ __forceinline__ void st_tile(uint32_t addr, const int4& v) {
 
 __device__ __constant__ int kTapOrder[9] = {4, 0, 1, 2, 3, 5, 6, 7, 8};
 
-template <int kN, int kRows>
+template <int kN, int kRows, bool kPair = false>
 __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvParams p) {
+  static_assert(!kPair || kRows == 256, "SM-pair launches use 256-row tiles");
   constexpr bool kSplitK = (kRows == 128);
+  constexpr int kRing = kPair ? kMaxPairStages : kMaxStages;
   extern __shared__ __align__(1024) unsigned char smem[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int halo = p.W + 1;
   const int TP = p.TP;
   const int chunk_g = p.cg < 8 ? p.cg : 8;              // channel groups per weight stage
   const int chunks_tap = p.cg / chunk_g;                // weight stages per tap
-  const uint32_t stage_bytes = (uint32_t)chunk_g * p.N * 16;
+  // a ring slot: the whole stage [chunk_g][N][8], or (pair) this CTA's half of its N rows, [chunk_g][N/2][8]
+  const uint32_t half_rows = kPair ? (uint32_t)p.N / 2 : (uint32_t)p.N;
+  const uint32_t stage_bytes = (uint32_t)chunk_g * half_rows * 16;
   const uint32_t a_bytes = (uint32_t)p.cg * TP * 16;
+  // pair launches: this CTA's rank in its cluster; the even CTA (rank 0) issues the MMAs of both
+  const uint32_t rank = kPair ? cluster_ctarank() : 0u;
+  const bool resident = !kPair && p.resident, khalf = !kPair && p.khalf;
 
   unsigned char* sA = smem;                                              // [2][cg][TP][16]
   unsigned char* sW = smem + (((size_t)2 * a_bytes + 127) & ~(size_t)127);   // [kStages][stage_bytes]
   const uint32_t kStages = (uint32_t)p.stages;
   uint64_t* bars = reinterpret_cast<uint64_t*>(sW + (size_t)kStages * stage_bytes);
   uint64_t* w_full = bars;                 // [kStages]
-  uint64_t* w_empty = bars + kMaxStages;   // [kStages]
-  uint64_t* a_full = bars + 2 * kMaxStages;   // [2]
+  uint64_t* w_empty = bars + kRing;        // [kStages]
+  uint64_t* a_full = bars + 2 * kRing;     // [2]
   uint64_t* mma_done = a_full + 2;         // [2]
   uint64_t* acc_empty = mma_done + 2;      // [2]
   uint64_t* a_ready = acc_empty + 2;       // [2 tiles][low, high channels] resident launches: the epilogue has written
@@ -204,45 +220,68 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
 
   if (tid == 0) {
     tmem_holder[2] = 0;
-    for (uint32_t s = 0; s < kStages; ++s) { mbar_init(&w_full[s], 1); mbar_init(&w_empty[s], kSplitK ? 1 : 2); }
+    // Arrival counts.  Pair launches: barriers the even CTA's MMAs wait on also take one arrival forwarded by the odd
+    // CTA (its half of the weight stage / its tile has landed, its epilogue has drained its accumulator); the MMA
+    // commits (w_empty, mma_done) are multicast to both CTAs, so those counts are the same in both.
+    const uint32_t fwd = (kPair && rank == 0) ? 1u : 0u;
+    for (uint32_t s = 0; s < kStages; ++s) {
+      mbar_init(&w_full[s], 1 + fwd);                 // own producer (+ the odd CTA's forwarder)
+      mbar_init(&w_empty[s], kSplitK ? 1 : 2);        // a commit per MMA warp that used the stage
+    }
     for (int b = 0; b < 2; ++b) {
-      mbar_init(&a_full[b], 1); mbar_init(&mma_done[b], 2); mbar_init(&acc_empty[b], kEpiThreads);
+      mbar_init(&a_full[b], 1 + fwd);                 // own tile loader (+ the odd CTA's forwarder)
+      mbar_init(&mma_done[b], 2);                     // a commit per MMA warp
+      mbar_init(&acc_empty[b], kEpiThreads + fwd);    // own epilogue threads (+ one arrival for the odd CTA's)
       mbar_init(&a_ready[2 * b], kEpiThreads); mbar_init(&a_ready[2 * b + 1], kEpiThreads);
     }
     fence_mbar_init();
   }
-  if (warp == 1) tmem_alloc(tmem_holder, 512);
+  if (warp == 1) {
+    if (kPair) tmem_alloc_pair(tmem_holder, 512);
+    else tmem_alloc(tmem_holder, 512);
+  }
   tc_fence_before();
-  __syncthreads();
+  if (kPair) cluster_sync();           // the peer's barriers are initialised before anything arrives on them
+  else __syncthreads();
   tc_fence_after();
   const uint32_t tmem = *tmem_holder;
   // tmem_holder[2]: number of items whose RESIDUAL producer (layer res_layer, same tile, possibly another CTA) the
   // weight-producer lane has seen published (dataflow launches); read by the epilogue before it requests residual rows
   const uint32_t s_res_a = smem_u32(tmem_holder + 2);
 
-  // every role walks the same (layer, tile) item sequence of this CTA
-  const int G = (int)gridDim.x;
-  auto first_tile = [&](int l) { int t0 = ((int)blockIdx.x - l * p.rot) % G; return t0 < 0 ? t0 + G : t0; };
+  // every role walks the same (layer, unit) item sequence of this CTA; a unit is a tile, or (pair) a tile pair, and
+  // BOTH CTAs of a pair walk the same sequence
+  const int G = kPair ? (int)gridDim.x >> 1 : (int)gridDim.x;          // CTAs, or clusters
+  const int me = kPair ? (int)blockIdx.x >> 1 : (int)blockIdx.x;
+  const int num_units = kPair ? (p.num_tiles + 1) >> 1 : p.num_tiles;
+  auto first_unit = [&](int l) { int t0 = (me - l * p.rot) % G; return t0 < 0 ? t0 + G : t0; };
+  auto tile_of = [&](int u) { return kPair ? 2 * u + (int)rank : u; };
   const bool dbg = p.dbg != nullptr;
+  // pair launches: the MMA-side role timing is the even CTA's
+  const bool dbg_mma = dbg && (!kPair || rank == 0);
 
   if (warp == 0) {
     // ------------------------------------------------ weight producer
     if (lane == 0) {
       const int per_tile = 9 * chunks_tap;
       uint32_t it = 0, res_items = 0;
-      long long t_wait = 0;
+      long long t_wait = 0, t_gate = 0;
       const long long t_begin = clock64();
+      // pair: a stage of the pair layout is two contiguous halves, this CTA's is at rank * stage_bytes
+      const uint32_t full_stage = (uint32_t)chunk_g * p.N * 16, own = rank * stage_bytes;
       for (int l = 0; l < p.num_layers; ++l) {
-        const unsigned char* wl = reinterpret_cast<const unsigned char*>(p.L[l].w);
-        for (int tile = first_tile(l); tile < p.num_tiles; tile += G) {
-          if (!p.resident && p.flags) {
+        const unsigned char* wl = reinterpret_cast<const unsigned char*>(kPair ? p.L[l].w_pair : p.L[l].w);
+        for (int u = first_unit(l); u < num_units; u += G) {
+          const int tile = tile_of(u);
+          if (!resident && p.flags) {
+            const long long tg = dbg ? clock64() : 0;
             // The epilogue prefetches this item's residual rows (written by layer res_layer, same tile, in general by
             // ANOTHER CTA two layers ago) before its MMAs finish, i.e. possibly before this CTA's loader has acquired
             // the item's dependency flags -- nothing would order that write before the prefetch.  This lane, which
             // runs a few weight stages ahead of everything else, acquires the producer's flag (it is practically
             // always set already: 0 misses in 10^4 items measured) and publishes an item counter at CTA scope.
             const LayerDesc& Lr = p.L[l];
-            if (Lr.residual && Lr.res_layer >= 0) {
+            if (Lr.residual && Lr.res_layer >= 0 && (!kPair || tile < p.num_tiles)) {
               const unsigned* f = p.flags + (size_t)Lr.res_layer * p.num_tiles + tile;
               unsigned spins = 0;
               while (ld_acquire(f) == 0u) {
@@ -250,6 +289,7 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
               }
             }
             ++res_items;
+            if (dbg) t_gate += clock64() - tg;
             asm volatile("st.release.cta.shared.u32 [%0], %1;" ::"r"(s_res_a), "r"(res_items) : "memory");
           }
           for (int c = 0; c < per_tile; ++c, ++it) {
@@ -261,52 +301,85 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
             // taps are consumed centre first (kTapOrder): the centre tap is the one no edge mask applies to, so it is
             // the MMA that initialises every row of the accumulator
             // (khalf: all taps of the low 64 input channels first, then the high ones -- the order the MMA warps use)
-            const int ti = p.khalf ? c % 9 : c / chunks_tap, chs = p.khalf ? c / 9 : c - ti * chunks_tap;
+            const int ti = khalf ? c % 9 : c / chunks_tap, chs = khalf ? c / 9 : c - ti * chunks_tap;
             const int src_stage = kTapOrder[ti] * chunks_tap + chs;
-            bulk_g2s(sW + (size_t)s * stage_bytes, wl + (size_t)src_stage * stage_bytes, stage_bytes, &w_full[s]);
+            bulk_g2s(sW + (size_t)s * stage_bytes, wl + (size_t)src_stage * full_stage + own, stage_bytes, &w_full[s]);
           }
         }
       }
-      if (dbg) { p.dbg[blockIdx.x * 16 + 0] = clock64() - t_begin; p.dbg[blockIdx.x * 16 + 1] = t_wait; }
+      if (dbg) { long long* d = p.dbg + blockIdx.x * 16; d[0] = clock64() - t_begin; d[1] = t_wait; d[15] = t_gate; }
     }
+  } else if (kPair && rank == 1 && (warp == 1 || warp == 3)) {
+    // ------------------------------------------------ odd CTA of a pair: no MMAs to issue.  Its MMA warps forward the
+    // completion of its own barriers to the even CTA, whose MMAs read this CTA's shared memory: a 1-D bulk copy can
+    // only signal a barrier in the CTA it writes to.  Warp 1 forwards a_full once per item as a release at cluster
+    // scope after the observed phase completion: besides TMA bytes it carries the edge masks the loader stored with
+    // st.shared, which the even CTA reads with ld.shared::cluster after its cluster-scope acquire.  Warp 3 forwards
+    // w_full once per weight stage as a RELAXED arrival: the only payload is bulk-copy bytes in this CTA's shared
+    // memory, read by this SM's own tensor pipe, and they have landed when the local phase completes; the arrival is
+    // issued only after that completion, and the MMA only after the even CTA sees the arrival.  A release at cluster
+    // scope there compiles to MEMBAR.ALL.GPU per stage and measured 1.71 M instead of 1.03 M cycles per 33-layer
+    // Gomoku launch.
+    if (lane == 0) {
+      const int per_tile = 9 * chunks_tap;
+      uint32_t it = 0;
+      int i = 0;
+      for (int l = 0; l < p.num_layers; ++l)
+        for (int u = first_unit(l); u < num_units; u += G, ++i) {
+          if (warp == 1) {
+            mbar_wait(&a_full[i & 1], (uint32_t)(i >> 1) & 1);
+            mbar_arrive_remote(&a_full[i & 1], 0);
+          } else {
+            for (int c = 0; c < per_tile; ++c, ++it) {
+              const uint32_t s = it % kStages, ph = (it / kStages) & 1;
+              mbar_wait(&w_full[s], ph);
+              mbar_arrive_remote_relaxed(&w_full[s], 0);
+            }
+          }
+        }
+    }
+    __syncwarp();
   } else if (warp == 1 || warp == 3) {
     // ------------------------------------------------ MMA issuers: warp 1 drives accumulator 0 (tile rows 0-127),
     // warp 3 accumulator 1 (rows 128-255); a weight stage / a tile is released when BOTH have committed.
+    // (Pair launches: the even CTA's warp 1 covers rows 0-127 of both CTAs' tiles, warp 3 rows 128-255.)
     // The WHOLE warp walks the loop and one lane is elected inside each tcgen05 asm statement, so
     // ptxas emits straight-line predicated UTCHMMAs (an `if (lane == 0)` around them costs a convergence
     // loop per MMA, ~100 cycles).  Descriptors are built once; only their 14-bit start-address field
     // (16-byte units) is stepped.
     const uint32_t mhalf = warp == 1 ? 0u : 1u;
-    const uint32_t idesc = instr_desc_f16(128, (uint32_t)p.N);
+    const uint32_t idesc = instr_desc_f16(kPair ? 256 : 128, (uint32_t)p.N);
     const uint64_t a_tmpl = smem_desc(0, (uint32_t)TP * 16, 128);
-    const uint64_t b_tmpl = smem_desc(0, (uint32_t)p.N * 16, 128);
+    const uint64_t b_tmpl = smem_desc(0, half_rows * 16, 128);
     const uint32_t a_hi = (uint32_t)(a_tmpl >> 32), a_lo0 = (uint32_t)a_tmpl;
     const uint32_t b_hi = (uint32_t)(b_tmpl >> 32), b_lo0 = (uint32_t)b_tmpl;
-    const uint32_t a_kstep = 2u * (uint32_t)TP, b_kstep = 2u * (uint32_t)p.N;   // 16-byte units per K=16 step
+    const uint32_t a_kstep = 2u * (uint32_t)TP, b_kstep = 2u * half_rows;   // 16-byte units per K=16 step
     const uint32_t sA16 = smem_u32(sA) >> 4, sW16 = smem_u32(sW) >> 4, stage16 = stage_bytes >> 4;
     const int ksteps = chunk_g / 2;
     auto desc64 = [](uint32_t lo, uint32_t hi) { return ((uint64_t)hi << 32) | lo; };
+    // barriers that also count an arrival from the odd CTA are acquired at cluster scope
+    auto wait_bar = [&](uint64_t* b, uint32_t ph) { if (kPair) mbar_wait_cluster(b, ph); else mbar_wait(b, ph); };
     uint32_t st = 0, st_ph = 0;                 // weight ring slot and its phase parity
     uint32_t b_slot = b_lo0 + sW16;             // descriptor low word of ring slot `st`
     const uint32_t b_first = b_slot;
-    long long t_acc = 0, t_a = 0, t_a_pos[3] = {0, 0, 0};
+    long long t_acc = 0, t_a = 0, t_w = 0, t_a_pos[3] = {0, 0, 0};
     const long long t_begin = clock64();
     int i = 0;
     for (int l = 0; l < p.num_layers; ++l)
-    for (int tile = first_tile(l); tile < p.num_tiles; tile += G, ++i) {
+    for (int u = first_unit(l); u < num_units; u += G, ++i) {
       const int buf = i & 1;
       const uint32_t uph = (i >> 1) & 1;
-      const int pos_in_layer = (tile - first_tile(l)) / G;
+      const int pos_in_layer = (u - first_unit(l)) / G;
       long long tw = dbg ? clock64() : 0;
-      mbar_wait(&acc_empty[buf], uph ^ 1);
+      wait_bar(&acc_empty[buf], uph ^ 1);
       long long tw2 = dbg ? clock64() : 0;
       t_acc += tw2 - tw;
-      mbar_wait(&a_full[buf], uph);
+      wait_bar(&a_full[buf], uph);
       // resident launch (item i == layer i): the tile of layer i >= 1 was written by the epilogue of layer i - 1
       const uint32_t rdy_ph = (uint32_t)(((i >> 1) - (buf == 0 ? 1 : 0)) & 1);
-      if (p.resident && i > 0) {
+      if (resident && i > 0) {
         mbar_wait(&a_ready[2 * buf], rdy_ph);                         // low 64 channels of the tile
-        if (!p.khalf) mbar_wait(&a_ready[2 * buf + 1], rdy_ph);       // khalf: the high half is awaited before its K chunk
+        if (!khalf) mbar_wait(&a_ready[2 * buf + 1], rdy_ph);         // khalf: the high half is awaited before its K chunk
       }
       if (dbg) { const long long dt = clock64() - tw2; t_a += dt; t_a_pos[pos_in_layer < 2 ? pos_in_layer : 2] += dt; }
       tc_fence_after();
@@ -315,10 +388,13 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
       uint32_t acc = 0;
       uint32_t stage_no = 0;                    // weight stage within the tile (split-K: stage s belongs to warp s & 1)
       // rows of this accumulator that sit on a board edge (left / right column, top / bottom row), from the loader
+      // (pair: also the odd CTA's, which its loader stored before the a_full arrival forwarded above)
       const uint4* em = reinterpret_cast<const uint4*>(s_mask + (buf * 2 + (kSplitK ? 0 : (int)mhalf)) * 16);
       const uint4 eL = em[0], eR = em[1], eT = em[2], eB = em[3];
+      uint4 pL = make_uint4(0, 0, 0, 0), pR = pL, pT = pL, pB = pL;
+      if (kPair) { pL = ld_shared_peer_v4(em, 1); pR = ld_shared_peer_v4(em + 1, 1); pT = ld_shared_peer_v4(em + 2, 1); pB = ld_shared_peer_v4(em + 3, 1); }
       // one weight stage (a 64-channel K chunk of one tap): wait for it, issue its MMAs, release it, step the ring
-      auto run_stage = [&](uint32_t a_lo, uint32_t m0, uint32_t m1, uint32_t m2, uint32_t m3) {
+      auto run_stage = [&](uint32_t a_lo, const uint4& m, const uint4& pm) {
         if (kSplitK && (stage_no & 1u) != mhalf) {       // the other warp's stage: just step the ring
           ++stage_no;
           ++st; b_slot += stage16;
@@ -326,56 +402,69 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
           return;
         }
         ++stage_no;
-        mbar_wait(&w_full[st], st_ph);
+        const long long tws = (kPair && dbg) ? clock64() : 0;
+        mbar_wait(&w_full[st], st_ph);      // see the odd CTA's w_full forwarder
+        if (kPair && dbg) t_w += clock64() - tws;
         tc_fence_after();
         uint32_t b_lo = b_slot;
-        if (ksteps == 4) {
+        if (kPair || ksteps == 4) {                       // pair launches always have 64-channel stages (flush)
           // the common case (64-channel stage) fully unrolled
           uint32_t al[4], bl[4];
 #pragma unroll
           for (int ks = 0; ks < 4; ++ks) { al[ks] = a_lo + (uint32_t)ks * a_kstep; bl[ks] = b_lo + (uint32_t)ks * b_kstep; }
-          mma4_f16_elect_masked(dacc, desc64(al[0], a_hi), desc64(al[1], a_hi), desc64(al[2], a_hi), desc64(al[3], a_hi),
-                                desc64(bl[0], b_hi), desc64(bl[1], b_hi), desc64(bl[2], b_hi), desc64(bl[3], b_hi), idesc,
-                                acc, m0, m1, m2, m3);
+          if (kPair)
+            mma4_f16_pair_elect_masked(dacc, desc64(al[0], a_hi), desc64(al[1], a_hi), desc64(al[2], a_hi),
+                                       desc64(al[3], a_hi), desc64(bl[0], b_hi), desc64(bl[1], b_hi), desc64(bl[2], b_hi),
+                                       desc64(bl[3], b_hi), idesc, acc, m, pm);
+          else
+            mma4_f16_elect_masked(dacc, desc64(al[0], a_hi), desc64(al[1], a_hi), desc64(al[2], a_hi), desc64(al[3], a_hi),
+                                  desc64(bl[0], b_hi), desc64(bl[1], b_hi), desc64(bl[2], b_hi), desc64(bl[3], b_hi), idesc,
+                                  acc, m.x, m.y, m.z, m.w);
           acc = 1;
         } else {
           for (int ks = 0; ks < ksteps; ++ks) {
-            mma_f16_elect_masked(dacc, desc64(a_lo, a_hi), desc64(b_lo, b_hi), idesc, acc, m0, m1, m2, m3);
+            mma_f16_elect_masked(dacc, desc64(a_lo, a_hi), desc64(b_lo, b_hi), idesc, acc, m.x, m.y, m.z, m.w);
             acc = 1;
             a_lo += a_kstep;
             b_lo += b_kstep;
           }
         }
-        commit_elect(&w_empty[st]);
+        if (kPair) commit_pair_elect(&w_empty[st]);
+        else commit_elect(&w_empty[st]);
         ++st; b_slot += stage16;
         if (st == kStages) { st = 0; st_ph ^= 1; b_slot = b_first; }
       };
       // taps centre first (kTapOrder); K chunks inside a tap -- or, khalf, all taps of the low 64 input channels, then
       // (once the epilogue of the previous layer has handed them over) all taps of the high 64
-      const int outer = p.khalf ? 2 : 1;
+      const int outer = khalf ? 2 : 1;
+      // output rows whose (y + ky - 1, x + kx - 1) neighbour is across a board edge take no part in a tap
+      auto tap_mask = [](int ky, int kx, const uint4& L, const uint4& R, const uint4& T, const uint4& B) {
+        auto w = [&](uint32_t l, uint32_t r, uint32_t t, uint32_t b) {
+          return (kx == 0 ? l : 0u) | (kx == 2 ? r : 0u) | (ky == 0 ? t : 0u) | (ky == 2 ? b : 0u);
+        };
+        return make_uint4(w(L.x, R.x, T.x, B.x), w(L.y, R.y, T.y, B.y), w(L.z, R.z, T.z, B.z), w(L.w, R.w, T.w, B.w));
+      };
       for (int ko = 0; ko < outer; ++ko) {
-        if (p.khalf && ko == 1 && i > 0) { mbar_wait(&a_ready[2 * buf + 1], rdy_ph); tc_fence_after(); }
+        if (khalf && ko == 1 && i > 0) { mbar_wait(&a_ready[2 * buf + 1], rdy_ph); tc_fence_after(); }
         for (int ti = 0; ti < 9; ++ti) {
           const int tap = ti == 0 ? 4 : (ti <= 4 ? ti - 1 : ti);
           const int ky = tap / 3, kx = tap - 3 * ky;
           const uint32_t a_tap = a_tile + (uint32_t)((ky - 1) * p.W + (kx - 1));   // wraps correctly: the shift may be negative
-          // output rows whose (y + ky - 1, x + kx - 1) neighbour is across a board edge take no part in this tap
-          const uint32_t m0 = (kx == 0 ? eL.x : 0u) | (kx == 2 ? eR.x : 0u) | (ky == 0 ? eT.x : 0u) | (ky == 2 ? eB.x : 0u);
-          const uint32_t m1 = (kx == 0 ? eL.y : 0u) | (kx == 2 ? eR.y : 0u) | (ky == 0 ? eT.y : 0u) | (ky == 2 ? eB.y : 0u);
-          const uint32_t m2 = (kx == 0 ? eL.z : 0u) | (kx == 2 ? eR.z : 0u) | (ky == 0 ? eT.z : 0u) | (ky == 2 ? eB.z : 0u);
-          const uint32_t m3 = (kx == 0 ? eL.w : 0u) | (kx == 2 ? eR.w : 0u) | (ky == 0 ? eT.w : 0u) | (ky == 2 ? eB.w : 0u);
-          if (p.khalf) {
-            run_stage(a_tap + (uint32_t)(ko * ksteps) * a_kstep, m0, m1, m2, m3);
+          const uint4 m = tap_mask(ky, kx, eL, eR, eT, eB);
+          const uint4 pm = kPair ? tap_mask(ky, kx, pL, pR, pT, pB) : m;
+          if (khalf) {
+            run_stage(a_tap + (uint32_t)(ko * ksteps) * a_kstep, m, pm);
           } else {
-            for (int ch = 0; ch < chunks_tap; ++ch) run_stage(a_tap + (uint32_t)(ch * ksteps) * a_kstep, m0, m1, m2, m3);
+            for (int ch = 0; ch < chunks_tap; ++ch) run_stage(a_tap + (uint32_t)(ch * ksteps) * a_kstep, m, pm);
           }
         }
       }
-      commit_elect(&mma_done[buf]);
+      if (kPair) commit_pair_elect(&mma_done[buf]);
+      else commit_elect(&mma_done[buf]);
     }
-    if (dbg && lane == 0 && warp == 1) {
+    if (dbg_mma && lane == 0 && warp == 1) {
       long long* d = p.dbg + blockIdx.x * 16;
-      d[2] = clock64() - t_begin; d[3] = t_acc; d[4] = t_a; d[6] = i;
+      d[2] = clock64() - t_begin; d[3] = t_acc; d[4] = t_a; d[5] = t_w; d[6] = i;
       d[12] = t_a_pos[0]; d[13] = t_a_pos[1]; d[14] = t_a_pos[2];
     }
   } else if (warp == 2) {
@@ -387,14 +476,18 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
     const long long t_begin = clock64();
     int i = 0, bias_layer = -1;
     for (int l = 0; l < p.num_layers; ++l)
-    for (int tile = first_tile(l); tile < p.num_tiles; tile += G, ++i) {
+    for (int u = first_unit(l); u < num_units; u += G, ++i) {
+      const int tile = tile_of(u);
       const LayerDesc& L = p.L[l];
       const int buf = i & 1;
       const int r0 = tile * p.tile_stride - halo, r1 = r0 + kRows + 2 * halo;       // tile rows [r0, r1)
-      const bool handed_over = p.resident && l > 0;     // the epilogue of layer l - 1 writes this tile into shared memory
+      const bool handed_over = resident && l > 0;       // the epilogue of layer l - 1 writes this tile into shared memory
+      // pair launches with an odd tile count: the odd CTA's last item is a null tile; it loads nothing but still
+      // arrives, so that the pair's MMAs run (its accumulator rows are never stored)
+      const bool null_tile = kPair && tile >= p.num_tiles;
       // dataflow dependency: the three tiles of the previous layer whose rows this tile reads
       long long tw = dbg ? clock64() : 0;
-      if (L.dep0 >= 0 && !p.resident) {
+      if (L.dep0 >= 0 && !resident && !null_tile) {
         if (lane < 6) {
           const int tt = tile - 1 + lane % 3;
           const int dl = lane < 3 ? L.dep0 : L.dep1;
@@ -436,17 +529,17 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
           }
         }
       const uint32_t dst0 = smem_u32(sA) + (uint32_t)buf * a_bytes;
-      if (handed_over) {          // nothing to load: bias and masks are staged, tell the MMA warps
+      if (handed_over || null_tile) {   // nothing to load: bias and masks are staged, tell the MMA warps
         __syncwarp();
         if (lane == 0) mbar_arrive(&a_full[buf]);
         continue;
       }
       // resident: exactly the tile's own boards (every tap that leaves them is masked); else the tile and its halo
-      const int lo = p.resident ? tile * p.tile_stride : (r0 > 0 ? r0 : 0);
+      const int lo = resident ? tile * p.tile_stride : (r0 > 0 ? r0 : 0);
       int hi = L.in_slots ? p.Ptot : p.plane_rows;
-      if (p.resident) { const int e = lo + p.tile_stride; hi = e < p.Ptot ? e : p.Ptot; }
+      if (resident) { const int e = lo + p.tile_stride; hi = e < p.Ptot ? e : p.Ptot; }
       else hi = r1 < hi ? r1 : hi;
-      if (r0 < 0 && !p.resident) {
+      if (r0 < 0 && !resident) {
         // rows before the first board are read by valid outputs (top-left taps of board 0): zeros
         const int nz = -r0;
         for (int k = lane; k < nz * cg; k += 32) {
@@ -491,7 +584,8 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
     const long long t_begin = clock64();
     int k = 0;
     for (int l = 0; l < p.num_layers; ++l)
-    for (int tile = first_tile(l); tile < p.num_tiles; tile += G, ++k) {
+    for (int u = first_unit(l); u < num_units; u += G, ++k) {
+      const int tile = tile_of(u);
       const LayerDesc& L = p.L[l];
       const bool norm = (L.out_norm != nullptr) || (L.out_slots != nullptr);
       const int buf = k & 1;
@@ -499,7 +593,7 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
       const bool fast = !norm && L.tab == nullptr && L.out != nullptr;
       // resident launch: this layer's output rows also go straight into the OTHER tile buffer in shared memory, in the
       // operand layout ([channel group][row][16 B], rows offset by the halo), where the next layer's MMAs read them
-      const int hand = (p.resident && l + 1 < p.num_layers) ? L.fwd : 0;
+      const int hand = (resident && l + 1 < p.num_layers) ? L.fwd : 0;
       bool lo_done = false;
       const uint32_t next_a = smem_u32(sA) + (uint32_t)(buf ^ 1) * a_bytes + (uint32_t)halo * 16;
       const uint32_t tbase = tmem + ((uint32_t)(quad * 32) << 16) + (uint32_t)(buf * 256);
@@ -534,7 +628,7 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
         int4 ring[3][4];
         // step t of this warp -> (row half j, 32-column chunk c).  khalf: low 64 channels (chunks 0, 1 across the two
         // column-half warps) of every row first, so that they can be handed to the next layer's first K chunk early
-        const bool kh = p.khalf && NCW == 2;
+        const bool kh = khalf && NCW == 2;
         auto jof = [&](int t) { return kh ? t % NJ : t / NCW; };
         auto cof = [&](int t) { return kh ? 2 * (t / NJ) + chalf : chalf * NCW + t % NCW; };
         // j is a run-time value under khalf: select, do not index (indexing would move the arrays to local memory)
@@ -545,7 +639,7 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
 #pragma unroll
           for (int u = 0; u < 4; ++u) dst[u] = ld ? __ldcg(resp + (size_t)(g0 + u) * PR + pick(Pj, j)) : make_int4(0, 0, 0, 0);
         };
-        if (!p.resident && has_res && p.flags && L.res_layer >= 0) {
+        if (!resident && has_res && p.flags && L.res_layer >= 0) {
           // ordered behind the residual producer's flag, see the weight-producer warp (a counter that is ahead of us)
           uint32_t seen;
           do { asm volatile("ld.acquire.cta.shared.u32 %0, [%1];" : "=r"(seen) : "r"(s_res_a) : "memory"); } while (seen < (uint32_t)(k + 1));
@@ -700,12 +794,17 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
         mbar_arrive(&a_ready[2 * (buf ^ 1) + 1]);
       }
       tc_fence_before();
-      mbar_arrive(&acc_empty[buf]);
-      if (p.flags) {
+      if (!kPair || rank == 0) mbar_arrive(&acc_empty[buf]);
+      if (kPair || p.flags) {
         // publish the tile: the barrier orders every epilogue thread's stores before thread 0, whose gpu-scope
-        // release is cumulative over them (the CUTLASS semaphore pattern) -- no per-thread MEMBAR on the chain
+        // release is cumulative over them (the CUTLASS semaphore pattern) -- no per-thread MEMBAR on the chain.
+        // (A null tile publishes nothing.)  Pair launches: the odd CTA's accumulator is drained as well, which
+        // thread 0 tells the even CTA's MMA warps with one cluster-scope arrival.
         asm volatile("bar.sync 1, 256;" ::: "memory");
-        if (et == 0) st_release(p.flags + (size_t)l * p.num_tiles + tile, 1u);
+        if (et == 0) {
+          if (p.flags && (!kPair || tile < p.num_tiles)) st_release(p.flags + (size_t)l * p.num_tiles + tile, 1u);
+          if (kPair && rank == 1) mbar_arrive_remote(&acc_empty[buf], 0);
+        }
       }
     }
     if (dbg && et == 0) {
@@ -713,9 +812,16 @@ __global__ void __maxnreg__(128) conv3x3_kernel(const __grid_constant__ ConvPara
       d[10] = clock64() - t_begin; d[11] = t_wait;
     }
   }
+  // pair launches: neither CTA leaves (or frees TMEM) while its peer may still arrive on its barriers, read its
+  // shared memory or run MMAs into its TMEM
   tc_fence_before();
-  __syncthreads();
-  if (warp == 1) tmem_dealloc(tmem, 512);
+  if (kPair) cluster_sync();
+  else __syncthreads();
+  if (warp == 1) {
+    if (kPair) tmem_dealloc_pair(tmem, 512);
+    else tmem_dealloc(tmem, 512);
+  }
+  if (kPair) cluster_sync();
 }
 
 // ---------------------------------------------------------------------------
@@ -883,17 +989,20 @@ __global__ void bn_fold_kernel(const float* g, const float* beta, const float* m
 }
 
 // conv weight [N][cin_total][3][3] (first `cin` input channels) * scale[n] -> packed fp16
-// [9 taps][chunks][chunk_g][N][8]
+// [9 taps][chunks][chunk_g][N][8], or (pair) [9 taps][chunks][half][chunk_g][N/2][8]: each weight stage as two
+// contiguous halves of its N rows, one per CTA of an SM pair
 // (N rows packed; rows >= n_real are zero: the padding of num_planes up to 32, or past the end of a column pass)
 __global__ void pack_conv_kernel(const float* __restrict__ w, const float* __restrict__ scale,
-                                 act_t* __restrict__ out, int N, int n_real, int cin, int cin_total, int cg) {
+                                 act_t* __restrict__ out, int N, int n_real, int cin, int cin_total, int cg, int pair) {
   const int chunk_g = cg < 8 ? cg : 8;
+  const int nh = pair ? N / 2 : N;
   const size_t total = (size_t)9 * cg * N * 8;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
     const int e = (int)(i % 8);
     size_t r = i / 8;
-    const int n = (int)(r % N); r /= N;
+    int n = (int)(r % nh); r /= nh;
     const int gl = (int)(r % chunk_g); r /= chunk_g;
+    if (pair) { n += (int)(r % 2) * nh; r /= 2; }
     const int ch = (int)(r % (cg / chunk_g));
     const int tap = (int)(r / (cg / chunk_g));
     const int c = (ch * chunk_g + gl) * 8 + e;
@@ -1062,6 +1171,7 @@ __global__ void normalise_rows_kernel(const act_t* __restrict__ raw, act_t* __re
 // ---------------------------------------------------------------------------
 struct ConvLayer {
   const act_t* w[2];      // packed weights per 128-column pass
+  const act_t* w_pair;    // single-pass convs of >= 64 channels in and out: the pair layout (SM-pair launches), else null
   const float* bias[2];
   int cg;                 // input channel groups of 8 (padded)
   int n_out;              // output channels incl. padding: 32, 64, 128 or 256
@@ -1101,6 +1211,9 @@ struct ConvNet : NetImpl {
   unsigned* flags;
   size_t flags_cap;
   int* err_flag;
+  // 2-CTA clusters of conv3x3_kernel<128 / 64, 256, true> the device can hold at once (at the largest shared memory a
+  // launch may ask for, so a bound for every launch)
+  int pair_clusters[2] = {0, 0};
 
   static int tp_of(const Geo& g, int rows = kTileM) { return (rows + 2 * (g.W + 1)) | 1; }
   // rows of one channel-group plane of a contiguous activation buffer holding `batch` boards of grid g
@@ -1108,22 +1221,25 @@ struct ConvNet : NetImpl {
     return (batch * g.PB() + kTileM - 1) / kTileM * kTileM + kPlaneSlack;
   }
   // n = output channels of one pass (the width of a weight stage and of the bias slots)
-  static size_t conv_fixed_smem(const Geo& g, int cg, int n, int rows) {
+  // pair: SM-pair launch, whose ring slots hold half a weight stage
+  static size_t conv_fixed_smem(const Geo& g, int cg, int n, int rows, bool pair = false) {
     const int TP = tp_of(g, rows);
     size_t a = (((size_t)2 * cg * TP * 16) + 127) & ~(size_t)127;
-    return a + (2 * kMaxStages + 10) * 8 + 16 + (size_t)4 * n * 4 + 2048 + 256 + 64;
+    return a + (2 * (pair ? kMaxPairStages : kMaxStages) + 10) * 8 + 16 + (size_t)4 * n * 4 + 2048 + 256 + 64;
   }
-  static int conv_stages(const Geo& g, int cg, int n, int rows) {
-    const int chunk_g = cg < 8 ? cg : 8;
-    const size_t stage = (size_t)chunk_g * n * 16;
-    const size_t fixed = conv_fixed_smem(g, cg, n, rows);
+  static size_t slot_bytes(int cg, int n, bool pair) { return (size_t)(cg < 8 ? cg : 8) * (pair ? n / 2 : n) * 16; }
+  // Ring depth: as many slots as shared memory holds, at most kMaxStages (kMaxPairStages).  A pair launch's half-size
+  // slots double what fits: the Gomoku tower (9x9, 128 channels) goes from 5 x 16 KB to 10 x 8 KB, i.e. the same
+  // bytes in flight ahead of the MMAs, but in finer steps; the 48x48 Atari blocks go from 2 to 5 slots.
+  static int conv_stages(const Geo& g, int cg, int n, int rows, bool pair = false) {
+    const size_t stage = slot_bytes(cg, n, pair);
+    const size_t fixed = conv_fixed_smem(g, cg, n, rows, pair);
     if (fixed + 2 * stage > 227 * 1024) return 0;
-    const int s = (int)((227 * 1024 - fixed) / stage);
-    return s > kMaxStages ? kMaxStages : s;
+    const int s = (int)((227 * 1024 - fixed) / stage), cap = pair ? kMaxPairStages : kMaxStages;
+    return s > cap ? cap : s;
   }
-  static size_t conv_smem(const Geo& g, int cg, int n, int rows) {
-    const int chunk_g = cg < 8 ? cg : 8;
-    return conv_fixed_smem(g, cg, n, rows) + (size_t)conv_stages(g, cg, n, rows) * chunk_g * n * 16;
+  static size_t conv_smem(const Geo& g, int cg, int n, int rows, bool pair = false) {
+    return conv_fixed_smem(g, cg, n, rows, pair) + (size_t)conv_stages(g, cg, n, rows, pair) * slot_bytes(cg, n, pair);
   }
   // tile rows a conv with `cg` input groups can use at all: 256-row tiles need 2 x cg x TP x 16 bytes of activations
   static bool fits(const Geo& g, int cg, int n, int rows) { return conv_stages(g, cg, n, rows) >= 2; }
@@ -1163,7 +1279,7 @@ struct ConvNet : NetImpl {
     for (int h = 0; h < np; ++h) {
       LayerDesc& d = pend.L[pend.num_layers];
       const size_t goff = (size_t)h * 16;                    // channel groups before this pass
-      d.in = in; d.in_index = in_index; d.w = L.w[h]; d.bias = L.bias[h];
+      d.in = in; d.in_index = in_index; d.w = L.w[h]; d.w_pair = L.w_pair; d.bias = L.bias[h];
       d.tab = tab_ ? tab_ + goff * g.PB() * 8 : nullptr;
       d.action = action;
       d.residual = residual ? residual + goff * PR * 8 : nullptr;
@@ -1249,13 +1365,27 @@ struct ConvNet : NetImpl {
     }
     p.num_tiles = p.resident ? (p.Ptot + p.tile_stride - 1) / p.tile_stride : (p.Ptot + rows - 1) / rows;
     p.TP = tp_of(g, rows);
-    p.stages = conv_stages(g, cg, N, rows);
+    const int sm_cap = (cta_limit > 0 && cta_limit < num_sms) ? cta_limit : num_sms;
+    // SM-pair launch (see kPair): the 256-row dataflow launch of several stride-1 single-pass layers with 64-channel
+    // weight stages.  Pairs rotate over pair items as CTAs rotate over tiles; as many pairs as there are pair items,
+    // as fit beside whatever else holds SMs (cta_limit, rounded down to an even CTA count) and as the device can
+    // place at once.  No pair fits (cta_limit 1): the single-CTA form.
+    const int units = (p.num_tiles + 1) / 2;
+    int pairs = 0;
+    bool pair_w = true;
+    for (int i = 0; i < nl; ++i) pair_w = pair_w && p.L[i].w_pair != nullptr;
+    if (rows == kTileM && nl > 1 && !p.resident && !p.sub && !multi_pass && pair_w) {
+      pairs = units < sm_cap / 2 ? units : sm_cap / 2;
+      const int mc = pair_clusters[N == 128 ? 0 : 1];
+      if (pairs > mc) pairs = mc;
+    }
+    const bool pair = pairs > 0;
+    p.stages = conv_stages(g, cg, N, rows, pair);
     p.err = err_flag;
     if (p.stages < 2) { reset_pending(); set_error("conv tile does not fit shared memory for a %dx%d grid", g.H, g.W); return MZ_EINVAL; }
-    const size_t smem = conv_smem(g, cg, N, rows);
-    const int sm_cap = (cta_limit > 0 && cta_limit < num_sms) ? cta_limit : num_sms;
-    const int grid = p.num_tiles < sm_cap ? p.num_tiles : sm_cap;
-    p.rot = nl > 1 ? p.num_tiles % grid : 0;
+    const size_t smem = conv_smem(g, cg, N, rows, pair);
+    const int grid = pair ? 2 * pairs : (p.num_tiles < sm_cap ? p.num_tiles : sm_cap);
+    p.rot = nl > 1 ? (pair ? units % pairs : p.num_tiles % grid) : 0;
     p.flags = nullptr;
     if (nl > 1 && !p.resident) {
       if ((size_t)nl * p.num_tiles > flags_cap) { reset_pending(); set_error("internal: flag buffer too small"); return MZ_EINVAL; }
@@ -1273,12 +1403,17 @@ struct ConvNet : NetImpl {
       // each grab part of the SMs and wait for the rest forever).
       cudaLaunchConfig_t lc = {};
       lc.gridDim = dim3((unsigned)grid); lc.blockDim = dim3(kConvThreads); lc.dynamicSmemBytes = smem; lc.stream = st;
-      cudaLaunchAttribute at[1];
+      cudaLaunchAttribute at[2];
       at[0].id = cudaLaunchAttributeCooperative;
       at[0].val.cooperative = nl > 1 ? 1 : 0;
-      lc.attrs = at; lc.numAttrs = 1;
+      at[1].id = cudaLaunchAttributeClusterDimension;
+      at[1].val.clusterDim.x = 2; at[1].val.clusterDim.y = 1; at[1].val.clusterDim.z = 1;
+      lc.attrs = at; lc.numAttrs = pair ? 2 : 1;
       cudaError_t le;
-      if (rows == 256) {
+      if (pair) {
+        if (N == 128) le = cudaLaunchKernelEx(&lc, conv3x3_kernel<128, 256, true>, p);
+        else le = cudaLaunchKernelEx(&lc, conv3x3_kernel<64, 256, true>, p);
+      } else if (rows == 256) {
         if (N == 128) le = cudaLaunchKernelEx(&lc, conv3x3_kernel<128, 256>, p);
         else if (N == 64) le = cudaLaunchKernelEx(&lc, conv3x3_kernel<64, 256>, p);
         else le = cudaLaunchKernelEx(&lc, conv3x3_kernel<32, 256>, p);
@@ -1297,12 +1432,16 @@ struct ConvNet : NetImpl {
       std::vector<long long> h((size_t)grid * 16);
       cudaMemcpy(h.data(), p.dbg, h.size() * sizeof(long long), cudaMemcpyDeviceToHost);
       cudaFree(p.dbg);
+      // the MMA fields (2-6, 12-14) of a pair launch are written by the even CTAs only; items/cta is then per pair
       double a[16] = {0};
-      for (int c = 0; c < grid; ++c) for (int k = 0; k < 16; ++k) a[k] += (double)h[(size_t)c * 16 + k] / grid;
-      fprintf(stderr, "[conv dbg] %dx%d cg=%d layers=%d items/cta=%.1f | producer total %.0f wait_empty %.0f | mma total %.0f wait_acc %.0f "
-              "wait_a %.0f (1st / 2nd / 3rd tile of a layer: %.0f / %.0f / %.0f) | loader total %.0f wait_mma %.0f wait_dep %.0f | "
-              "epilogue total %.0f wait_mma %.0f\n",
-              g.H, g.W, cg, nl, a[6], a[0], a[1], a[2], a[3], a[4], a[12], a[13], a[14], a[7], a[8], a[9], a[10], a[11]);
+      const bool mma_field[16] = {0, 0, 1, 1, 1, 1, 1, 0, 0, 0, 0, 0, 1, 1, 1, 0};
+      for (int c = 0; c < grid; ++c)
+        for (int k = 0; k < 16; ++k) a[k] += (double)h[(size_t)c * 16 + k] / (pair && mma_field[k] ? grid / 2 : grid);
+      fprintf(stderr, "[conv dbg] %dx%d cg=%d layers=%d %s items/cta=%.1f | producer total %.0f wait_empty %.0f "
+              "residual_gate %.0f | mma total %.0f wait_acc %.0f wait_a %.0f (1st / 2nd / 3rd tile of a layer: %.0f / %.0f / "
+              "%.0f) wait_w %.0f | loader total %.0f wait_mma %.0f wait_dep %.0f | epilogue total %.0f wait_mma %.0f\n",
+              g.H, g.W, cg, nl, pair ? "pair" : "single", a[6], a[0], a[1], a[15], a[2], a[3], a[4], a[12], a[13], a[14],
+              a[5], a[7], a[8], a[9], a[10], a[11]);
     }
     return MZ_OK;
   }
@@ -1531,6 +1670,9 @@ int conv_hidden_bytes(const mz_net_config& c, int32_t* bytes) {
 }
 
 static size_t conv_w_bytes(int cg, int N) { return align_up((size_t)9 * cg * N * 16, 256); }
+// convs that can run in SM-pair launches (64-channel weight stages, one pass of >= 64 columns) also keep their weights
+// in the pair layout
+static bool pair_layout(int cg, int n_out) { return cg >= 8 && n_out >= 64 && n_out <= 128; }
 static int obs_cg(int cin) { return ((cin + 15) / 16) * 2; }
 
 // An upper bound on what conv_create takes: its grids are sized (H+1)(W+1), more than the H*W rows a board uses.
@@ -1543,6 +1685,7 @@ int conv_arena_bytes(const mz_net_config& c, int max_batch, size_t* bytes) {
   size_t t = 0;
   const int nconv_main = 1 + 6 * c.num_res_blocks + (atari ? 12 : 0);   // dyn0 + 2 per block x 3 towers (+ Atari rep)
   t += conv_w_bytes(obs_cg(c.in_channels), N) + (size_t)nconv_main * (conv_w_bytes(N / 8, N) + 512);
+  t += (size_t)(nconv_main + 1) * conv_w_bytes(N / 8, N);                             // pair layouts (+ rep0)
   t += (size_t)(2 + 6 * c.num_res_blocks + 12) * 2 * align_up((size_t)N * 4, 256);     // scale + bias per conv
   t += 2 * align_up((size_t)9 * 128 * 256 * 2, 256);                                    // stride-2 conv weights
   t += align_up((size_t)A * PB * N * 4, 256);                                           // action table
@@ -1604,9 +1747,16 @@ int conv_create(const mz_net_config& c, const float* const* w, int nw, int max_b
       act_t* wp = (act_t*)take((size_t)9 * cg * npass * 16);
       const int rows_real = n_real - h * 128 < npass ? n_real - h * 128 : npass;
       pack_conv_kernel<<<256, 256>>>(cw + (size_t)h * 128 * cin_total * 9, scale + h * 128, wp, npass, rows_real, cin,
-                                     cin_total, cg);
+                                     cin_total, cg, 0);
       MZ_LAUNCH_CHECK("pack_conv_kernel");
       L->w[h] = wp; L->bias[h] = bias + h * 128;
+    }
+    L->w_pair = nullptr;
+    if (pair_layout(cg, n_out)) {
+      act_t* wp = (act_t*)take((size_t)9 * cg * n_out * 16);
+      pack_conv_kernel<<<256, 256>>>(cw, scale, wp, n_out, n_real, cin, cin_total, cg, 1);
+      MZ_LAUNCH_CHECK("pack_conv_kernel");
+      L->w_pair = wp;
     }
     return MZ_OK;
   };
@@ -1733,8 +1883,21 @@ int conv_create(const mz_net_config& c, const float* const* w, int nw, int max_b
   if (e == cudaSuccess) e = cudaFuncSetAttribute(conv3x3_kernel<128, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(conv3x3_kernel<64, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(conv3x3_kernel<32, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(conv3x3_kernel<128, 256, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(conv3x3_kernel<64, 256, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(head_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared);
   if (e != cudaSuccess) { set_error("cudaFuncSetAttribute: %s", cudaGetErrorString(e)); delete net; return MZ_ECUDA; }
+  {
+    cudaLaunchConfig_t lc = {};
+    lc.gridDim = dim3(2 * (unsigned)net->num_sms); lc.blockDim = dim3(kConvThreads); lc.dynamicSmemBytes = smem_max;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeClusterDimension;
+    at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+    lc.attrs = at; lc.numAttrs = 1;
+    e = cudaOccupancyMaxActiveClusters(&net->pair_clusters[0], conv3x3_kernel<128, 256, true>, &lc);
+    if (e == cudaSuccess) e = cudaOccupancyMaxActiveClusters(&net->pair_clusters[1], conv3x3_kernel<64, 256, true>, &lc);
+    if (e != cudaSuccess) { set_error("cudaOccupancyMaxActiveClusters: %s", cudaGetErrorString(e)); delete net; return MZ_ECUDA; }
+  }
   *out = net;
   return MZ_OK;
 }

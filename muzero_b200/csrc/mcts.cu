@@ -623,10 +623,10 @@ extern "C" int mz_expand_backup_select(mz_pool* pool, const float* reward, const
   }
   if (pool->tree_ctas > 0 && A <= 128) {
     const dim3 cgrid(pool->tree_ctas), cblock(kConfinedThreads);
-    if (A <= 32) launch_pdl(pdl_ok(pool), backup_select_confined_kernel<1>, cgrid, cblock, (size_t)kConfinedSmem, st, d, r, v);
-    else if (A <= 64) launch_pdl(pdl_ok(pool), backup_select_confined_kernel<2>, cgrid, cblock, (size_t)kConfinedSmem, st, d, r, v);
-    else if (A <= 96) launch_pdl(pdl_ok(pool), backup_select_confined_kernel<3>, cgrid, cblock, (size_t)kConfinedSmem, st, d, r, v);
-    else launch_pdl(pdl_ok(pool), backup_select_confined_kernel<4>, cgrid, cblock, (size_t)kConfinedSmem, st, d, r, v);
+    if (A <= 32) launch_pdl_pairs(pdl_ok(pool), backup_select_confined_kernel<1>, cgrid, cblock, (size_t)kConfinedSmem, st, d, r, v);
+    else if (A <= 64) launch_pdl_pairs(pdl_ok(pool), backup_select_confined_kernel<2>, cgrid, cblock, (size_t)kConfinedSmem, st, d, r, v);
+    else if (A <= 96) launch_pdl_pairs(pdl_ok(pool), backup_select_confined_kernel<3>, cgrid, cblock, (size_t)kConfinedSmem, st, d, r, v);
+    else launch_pdl_pairs(pdl_ok(pool), backup_select_confined_kernel<4>, cgrid, cblock, (size_t)kConfinedSmem, st, d, r, v);
     MZ_LAUNCH_CHECK("backup_select_confined_kernel");
     pool->selected = 1;
     return MZ_OK;

@@ -50,6 +50,53 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
   }
 }
 
+// ---- CTA pairs (2-CTA clusters, tcgen05 .cta_group::2) ------------------------------
+__device__ __forceinline__ uint32_t cluster_ctarank() {
+  uint32_t r;
+  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+  return r;
+}
+// every thread of both CTAs; orders each CTA's earlier shared-memory writes (barrier inits included) before the
+// peer's later accesses
+__device__ __forceinline__ void cluster_sync() {
+  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+// the wait of a barrier that also receives arrivals from the peer CTA: acquire at cluster scope
+__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
+  uint32_t ok;
+  do {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
+        "selp.u32 %0, 1, 0, p;\n\t}"
+        : "=r"(ok)
+        : "r"(smem_u32(bar)), "r"(parity)
+        : "memory");
+  } while (!ok);
+}
+// arrive on the barrier at the same shared-memory offset in CTA `cta` of the cluster; release at cluster scope makes
+// everything this thread has observed (a completed local barrier phase included) visible to the peer's acquire
+__device__ __forceinline__ void mbar_arrive_remote(uint64_t* bar, uint32_t cta) {
+  uint32_t r;
+  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_u32(bar)), "r"(cta));
+  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(r) : "memory");
+}
+// the same without release semantics (no MEMBAR): forwards the completion of a barrier whose only payload is
+// bulk-copy bytes in the forwarding CTA's own shared memory (conv.cu, w_full of SM-pair launches)
+__device__ __forceinline__ void mbar_arrive_remote_relaxed(uint64_t* bar, uint32_t cta) {
+  uint32_t r;
+  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_u32(bar)), "r"(cta));
+  asm volatile("mbarrier.arrive.relaxed.cluster.shared::cluster.b64 _, [%0];" ::"r"(r) : "memory");
+}
+// 16 bytes at the same shared-memory offset in CTA `cta` of the cluster
+__device__ __forceinline__ uint4 ld_shared_peer_v4(const void* p, uint32_t cta) {
+  uint32_t r;
+  uint4 v;
+  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_u32(p)), "r"(cta));
+  asm volatile("ld.shared::cluster.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(r) : "memory");
+  return v;
+}
+
 // ---- proxies / fences ---------------------------------------------------------
 // generic-proxy writes to smem (st.shared) -> visible to the async proxy (tcgen05.mma, TMA)
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
@@ -66,6 +113,16 @@ __device__ __forceinline__ void tmem_alloc(uint32_t* smem_dst, uint32_t ncols) {
 }
 __device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
   asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
+}
+// CTA-pair forms: one warp in EACH CTA of the pair
+__device__ __forceinline__ void tmem_alloc_pair(uint32_t* smem_dst, uint32_t ncols) {
+  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_dst)),
+               "r"(ncols)
+               : "memory");
+  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+}
+__device__ __forceinline__ void tmem_dealloc_pair(uint32_t taddr, uint32_t ncols) {
+  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
 }
 // 32 lanes x 32 consecutive fp32 columns: thread i of the warp gets lane (base lane + i)
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
@@ -182,6 +239,36 @@ __device__ __forceinline__ void mma4_f16_elect(uint32_t d_tmem, uint64_t a0, uin
       "@q tcgen05.mma.cta_group::1.kind::f16 [%0], %3, %7, %9, t;\n\t"
       "@q tcgen05.mma.cta_group::1.kind::f16 [%0], %4, %8, %9, t;\n\t}"
       ::"r"(d_tmem), "l"(a0), "l"(a1), "l"(a2), "l"(a3), "l"(b0), "l"(b1), "l"(b2), "l"(b3), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+// The SM-pair form (cta_group::2, M = 256, issued by the even CTA of a 2-CTA cluster only): rows 0-127 of D are
+// the issuing CTA's, rows 128-255 the peer's, each in its own TMEM at d_tmem; each CTA supplies its 128 rows of A and
+// half of the N rows of B from its own shared memory at the descriptors' addresses.  Mask words 0-3 are the issuing
+// CTA's TMEM lanes, words 4-7 the peer's.
+__device__ __forceinline__ void mma4_f16_pair_elect_masked(uint32_t d_tmem, uint64_t a0, uint64_t a1, uint64_t a2,
+                                                           uint64_t a3, uint64_t b0, uint64_t b1, uint64_t b2, uint64_t b3,
+                                                           uint32_t idesc, uint32_t accumulate, const uint4& m,
+                                                           const uint4& n) {
+  asm volatile(
+      "{\n\t.reg .pred p, q, t;\n\t"
+      "setp.ne.b32 p, %10, 0;\n\t"
+      "setp.eq.b32 t, 0, 0;\n\t"
+      "elect.sync _|q, 0xffffffff;\n\t"
+      "@q tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %5, %9, {%11, %12, %13, %14, %15, %16, %17, %18}, p;\n\t"
+      "@q tcgen05.mma.cta_group::2.kind::f16 [%0], %2, %6, %9, {%11, %12, %13, %14, %15, %16, %17, %18}, t;\n\t"
+      "@q tcgen05.mma.cta_group::2.kind::f16 [%0], %3, %7, %9, {%11, %12, %13, %14, %15, %16, %17, %18}, t;\n\t"
+      "@q tcgen05.mma.cta_group::2.kind::f16 [%0], %4, %8, %9, {%11, %12, %13, %14, %15, %16, %17, %18}, t;\n\t}"
+      ::"r"(d_tmem), "l"(a0), "l"(a1), "l"(a2), "l"(a3), "l"(b0), "l"(b1), "l"(b2), "l"(b3), "r"(idesc),
+        "r"(accumulate), "r"(m.x), "r"(m.y), "r"(m.z), "r"(m.w), "r"(n.x), "r"(n.y), "r"(n.z), "r"(n.w)
+      : "memory");
+}
+// arrive on `bar` in BOTH CTAs of the pair once every MMA this thread issued before has completed
+__device__ __forceinline__ void commit_pair_elect(uint64_t* bar) {
+  asm volatile(
+      "{\n\t.reg .pred q;\n\t"
+      "elect.sync _|q, 0xffffffff;\n\t"
+      "@q tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;\n\t}" ::"r"(
+          smem_u32(bar)), "h"((unsigned short)3)
       : "memory");
 }
 __device__ __forceinline__ void commit_elect(uint64_t* bar) {

@@ -15,9 +15,6 @@ __device__ __forceinline__ void mma2(uint32_t d, uint64_t a, uint64_t b, uint32_
                "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d), "l"(a), "l"(b), "r"(idesc), "r"(acc)
                : "memory");
 }
-__device__ __forceinline__ void cluster_sync() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
 
 template <bool kTwo>
 __global__ void __launch_bounds__(384) bench(int N, int a_rows, int b_rows, int iters, long long* out, int writer, int data) {
