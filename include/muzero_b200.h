@@ -251,6 +251,42 @@ int mz_net_set_cta_limit(mz_net* net, int32_t max_ctas);
 int mz_net_profile_begin(mz_net* net);
 int mz_net_profile_end(mz_net* net, double* ms_by_class /* [5] */, int64_t* launches_by_class /* [5] */);
 
+/* ---- test aid of the conv nets: keep every intermediate tensor of an inference call ----
+ * The towers reuse their activation buffers (ping-pong, residual blocks write over their input), so the layers of a
+ * call are gone when it returns.  With capture on (buf != NULL, device memory of at least mz_net_debug_capture_bytes),
+ * every conv output and every pool output of the next calls goes to a region of its own in `buf`, and the last layer
+ * of a normalising tower also stores its raw output.  The launches are grouped and take the same forms as without
+ * capture, and compute the same values.  Each call starts a new record of
+ *   tensors: the packed observation, every conv / pool output, and the normalised state the prediction tower reads
+ *            (planes [groups][plane_rows][8] fp16, board b at rows b*h*w ...);
+ *   launches: one per conv3x3_kernel launch, with the form the host chose for it.
+ * buf = NULL turns capture off.  MLP nets: MZ_EINVAL. */
+#define MZ_DEBUG_MAX_LAYERS 34
+enum mz_debug_kind { MZ_DEBUG_OBS = 0, MZ_DEBUG_CONV = 1, MZ_DEBUG_POOL = 2, MZ_DEBUG_NORM = 3 };
+typedef struct {
+  void* ptr;
+  int32_t kind;            /* mz_debug_kind */
+  int32_t stage;           /* 0 representation, 1 dynamics, 2 prediction */
+  int32_t index;           /* conv (or pool) number within the stage, in execution order from 0 */
+  int32_t plane_rows, groups, h, w, batch;
+  int32_t src;             /* tensor read: conv input (-1: the hidden-state slots), pool input, or the raw tensor a
+                              NORM was normalised from */
+  int32_t residual;        /* conv: tensor added after the conv (-1: none) */
+} mz_debug_tensor;
+typedef struct {
+  int32_t num_layers, tile_rows, resident, khalf, pair, sub, multi_pass, grid, num_tiles, cg, n, h, w, batch;
+  /* per layer (LayerDesc) of the launch: the tensor it writes (-1: none), its 128-column pass, whether it normalises
+   * (bit 0: contiguous copy, bit 1: slots) or adds the action table (bit 2), its in-launch producer and residual
+   * producer (-1: an earlier launch) and the resident hand-over (1: raw output, 2: normalised) */
+  int32_t out[MZ_DEBUG_MAX_LAYERS], pass[MZ_DEBUG_MAX_LAYERS], flags[MZ_DEBUG_MAX_LAYERS];
+  int32_t dep0[MZ_DEBUG_MAX_LAYERS], res_layer[MZ_DEBUG_MAX_LAYERS], fwd[MZ_DEBUG_MAX_LAYERS];
+} mz_debug_launch;
+int mz_net_debug_capture_bytes(mz_net* net, int32_t batch, size_t* bytes);
+int mz_net_debug_capture(mz_net* net, void* buf, size_t bytes);
+/* index < 0: only *count (tensors / launches of the last call) */
+int mz_net_debug_tensor(mz_net* net, int32_t index, mz_debug_tensor* out, int32_t* count);
+int mz_net_debug_launch(mz_net* net, int32_t index, mz_debug_launch* out, int32_t* count);
+
 /* ------------------------------------------------------------------------
  * Callers of the search path, device-resident (SURVEY.md 8f: f-1, f-3)
  * ---------------------------------------------------------------------- */

@@ -40,6 +40,22 @@ class NetConfig(C.Structure):
                 ('hidden_dim', C.c_int32), ('value_support', C.c_int32), ('reward_support', C.c_int32)]
 
 
+class DebugTensor(C.Structure):
+    _fields_ = [('ptr', C.c_void_p), ('kind', C.c_int32), ('stage', C.c_int32), ('index', C.c_int32),
+                ('plane_rows', C.c_int32), ('groups', C.c_int32), ('h', C.c_int32), ('w', C.c_int32),
+                ('batch', C.c_int32), ('src', C.c_int32), ('residual', C.c_int32)]
+
+
+MZ_DEBUG_MAX_LAYERS = 34
+MZ_DEBUG_OBS, MZ_DEBUG_CONV, MZ_DEBUG_POOL, MZ_DEBUG_NORM = 0, 1, 2, 3
+
+
+class DebugLaunch(C.Structure):
+    _fields_ = ([(k, C.c_int32) for k in ('num_layers', 'tile_rows', 'resident', 'khalf', 'pair', 'sub', 'multi_pass',
+                                          'grid', 'num_tiles', 'cg', 'n', 'h', 'w', 'batch')] +
+                [(k, C.c_int32 * MZ_DEBUG_MAX_LAYERS) for k in ('out', 'pass_', 'flags', 'dep0', 'res_layer', 'fwd')])
+
+
 _P = C.c_void_p
 # name -> (restype, argtypes); every symbol include/muzero_b200.h declares
 PROTOTYPES = {
@@ -78,6 +94,10 @@ PROTOTYPES = {
     'mz_net_set_fused_search': (C.c_int, [_P, C.c_int32]),
     'mz_net_set_cta_limit': (C.c_int, [_P, C.c_int32]),
     'mz_net_profile_begin': (C.c_int, [_P]),
+    'mz_net_debug_capture_bytes': (C.c_int, [_P, C.c_int32, C.POINTER(C.c_size_t)]),
+    'mz_net_debug_capture': (C.c_int, [_P, _P, C.c_size_t]),
+    'mz_net_debug_tensor': (C.c_int, [_P, C.c_int32, C.POINTER(DebugTensor), C.POINTER(C.c_int32)]),
+    'mz_net_debug_launch': (C.c_int, [_P, C.c_int32, C.POINTER(DebugLaunch), C.POINTER(C.c_int32)]),
     'mz_net_profile_end': (C.c_int, [_P, C.POINTER(C.c_double), C.POINTER(C.c_int64)]),
     'mz_env_arena_bytes': (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_size_t)]),
     'mz_env_create': (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P, C.c_size_t, C.POINTER(_P)]),

@@ -49,6 +49,7 @@ constexpr int kMaxPairStages = 12;   // SM-pair launches: a ring slot holds half
 constexpr int kPlaneSlack = 64; // rows allocated past the last tile of every plane (>= the widest halo)
 
 constexpr int kMaxLayers = 34;   // one launch runs up to a whole recurrent inference: 1 + 16 + 16 convs
+static_assert(kMaxLayers == MZ_DEBUG_MAX_LAYERS, "mz_debug_launch holds one entry per LayerDesc of a launch");
 
 // One convolution layer of a launch.  Layers of a launch share geometry, channel counts and the
 // persistent CTAs; layer l+1's tile t starts as soon as tiles t-1, t, t+1 of layer l are published
@@ -1215,6 +1216,82 @@ struct ConvNet : NetImpl {
   // launch may ask for, so a bound for every launch)
   int pair_clusters[2] = {0, 0};
 
+  // ---- test aid (mz_net_debug_capture): every conv / pool output of a call in a region of its own ----
+  char* cap_buf = nullptr;
+  size_t cap_size = 0, cap_used = 0;
+  int cap_stage = 0, cap_conv = 0, cap_pool = 0;
+  std::vector<mz_debug_tensor> cap_tensors;
+  std::vector<mz_debug_launch> cap_launches;
+  bool capturing() const { return cap_buf != nullptr; }
+  void cap_begin() { cap_used = 0; cap_tensors.clear(); cap_launches.clear(); cap_set_stage(0); }
+  void cap_set_stage(int s) { cap_stage = s; cap_conv = 0; cap_pool = 0; }
+  size_t act_bytes(int batch) const {
+    auto rows = [&](size_t pb) { return ((size_t)batch * pb + kTileM - 1) / kTileM * kTileM + kPlaneSlack; };
+    const size_t mid_pb = atari ? (size_t)(cfg.in_h / 4 + 1) * (cfg.in_w / 4 + 1) : (size_t)lat.PB();
+    const size_t big_pb = atari ? (size_t)(cfg.in_h / 2 + 1) * (cfg.in_w / 2 + 1) : (size_t)lat.PB();
+    size_t a = rows(mid_pb) * C * 2;
+    if (atari && rows(big_pb) * 128 * 2 > a) a = rows(big_pb) * 128 * 2;
+    return align_up(a, 256);
+  }
+  // index of the recorded tensor whose planes contain p (a column pass points inside its conv's tensor), -1: none
+  int cap_find(const void* p) const {
+    for (size_t i = 0; i < cap_tensors.size(); ++i) {
+      const mz_debug_tensor& t = cap_tensors[i];
+      const char* b = (const char*)t.ptr;
+      if ((const char*)p >= b && (const char*)p < b + (size_t)t.plane_rows * t.groups * 16) return (int)i;
+    }
+    return -1;
+  }
+  int cap_add(void* ptr, int kind, const Geo& g, int batch, int groups, int src, int residual) {
+    mz_debug_tensor t;
+    t.ptr = ptr; t.kind = kind; t.stage = cap_stage;
+    t.index = kind == MZ_DEBUG_CONV ? cap_conv++ : (kind == MZ_DEBUG_POOL ? cap_pool++ : 0);
+    t.plane_rows = plane_rows_of(g, batch); t.groups = groups; t.h = g.H; t.w = g.W; t.batch = batch;
+    t.src = src; t.residual = residual;
+    cap_tensors.push_back(t);
+    return (int)cap_tensors.size() - 1;
+  }
+  // a fresh region of the capture buffer for a conv / pool output (nullptr: the buffer is full, error set)
+  act_t* cap_take(int kind, const Geo& g, int batch, int groups, const void* src, const void* residual) {
+    const size_t bytes = align_up((size_t)plane_rows_of(g, batch) * groups * 16, 256);
+    if (cap_used + bytes > cap_size) {
+      // the call fails here: drop the layers it already queued, which point into this call's buffers
+      reset_pending();
+      num_pend_heads = 0; pend_heads_smem = 0;
+      set_error("mz_net_debug_capture: buffer of %zu bytes too small", cap_size);
+      return nullptr;
+    }
+    act_t* r = (act_t*)(cap_buf + cap_used);
+    cap_used += bytes;
+    cap_add(r, kind, g, batch, groups, src ? cap_find(src) : -1, residual ? cap_find(residual) : -1);
+    return r;
+  }
+  int debug_capture_bytes(int batch, size_t* bytes) override {
+    // more regions than any call takes: board 1 + 4 blocks convs, Atari 14 + 2 blocks convs and one pool
+    *bytes = (size_t)(16 + 4 * blocks) * act_bytes(batch);
+    return MZ_OK;
+  }
+  int debug_capture(void* buf, size_t bytes) override {
+    reset_pending();                 // every call flushes what it queued; nothing of an earlier buffer may stay queued
+    cap_buf = (char*)buf; cap_size = buf ? bytes : 0;
+    cap_begin();
+    return MZ_OK;
+  }
+  int debug_tensor(int index, mz_debug_tensor* out, int32_t* count) override {
+    *count = (int32_t)cap_tensors.size();
+    if (index < 0) return MZ_OK;
+    MZ_CHECK_ARG(index < *count, "tensor %d of %d", index, *count);
+    *out = cap_tensors[index];
+    return MZ_OK;
+  }
+  int debug_launch(int index, mz_debug_launch* out, int32_t* count) override {
+    *count = (int32_t)cap_launches.size();
+    if (index < 0) return MZ_OK;
+    MZ_CHECK_ARG(index < *count, "launch %d of %d", index, *count);
+    *out = cap_launches[index];
+    return MZ_OK;
+  }
+
   static int tp_of(const Geo& g, int rows = kTileM) { return (rows + 2 * (g.W + 1)) | 1; }
   // rows of one channel-group plane of a contiguous activation buffer holding `batch` boards of grid g
   static int plane_rows_of(const Geo& g, int batch) {
@@ -1424,6 +1501,20 @@ struct ConvNet : NetImpl {
       }
       if (le != cudaSuccess) { reset_pending(); set_error("conv3x3_kernel launch: %s", cudaGetErrorString(le)); cudaGetLastError(); return MZ_ECUDA; }
     }
+    if (capturing()) {
+      mz_debug_launch r = {};
+      r.num_layers = nl; r.tile_rows = rows; r.resident = p.resident; r.khalf = p.khalf; r.pair = pairs; r.sub = p.sub;
+      r.multi_pass = multi_pass ? 1 : 0; r.grid = grid; r.num_tiles = p.num_tiles; r.cg = cg; r.n = N; r.h = g.H;
+      r.w = g.W; r.batch = batch;
+      for (int i = 0; i < nl; ++i) {
+        const LayerDesc& d = p.L[i];
+        r.out[i] = d.out ? cap_find(d.out) : -1;
+        r.pass[i] = pend_pass[i];
+        r.flags[i] = (d.out_norm ? 1 : 0) | (d.out_slots ? 2 : 0) | (d.tab ? 4 : 0);
+        r.dep0[i] = d.dep0; r.res_layer[i] = d.res_layer; r.fwd[i] = d.fwd;
+      }
+      cap_launches.push_back(r);
+    }
     prof_mark(-1, st);
     reset_pending();
     MZ_LAUNCH_CHECK("conv3x3_kernel");
@@ -1487,18 +1578,30 @@ struct ConvNet : NetImpl {
     const ConvLayer& last_layer = nblk > 0 ? blk[2 * nblk - 1] : *first;
     const bool late_norm = normalise && last_layer.passes() > 1;
     const bool keep_raw = want_raw || late_norm;
+    // Capture (mz_net_debug_capture): every conv writes a region of its own instead of b0 / b1 / b2 / raw_dst, and the
+    // last layer of a normalising tower also stores its raw output.  The launches stay as they are: add_conv groups
+    // convs on (cg, grid, N, n_real, batch, layer count, sub) only, flush() chooses the form from those, `fits()` and
+    // cta_limit, and the pointer tests it makes still hold -- each layer reads its producer's `out` (or the `out_norm`
+    // b3, which is not moved) so the resident hand-over `fwd` is the same, and a residual is still the `out` / `out_norm`
+    // of the layer that res_layer names.  Only the in-place block output (over its input) becomes a separate store.
+    const bool cap = capturing();
     if (first) {
       const bool last = (nblk == 0);
       act_t* dst = (last && raw_dst) ? raw_dst : pp[which];
-      rc = add_conv(*first, g, cur, cur_index, cur_slots, batch, tab_, action, nullptr,
-                    (last && normalise && !keep_raw) ? nullptr : dst, (last && !late_norm) ? norm_out : nullptr,
-                    (last && !late_norm) ? slots : nullptr, out_index, st);
+      act_t* out = (last && normalise && !keep_raw) ? nullptr : dst;
+      if (cap && !(dst = out = cap_take(MZ_DEBUG_CONV, g, batch, first->n_out / 8, cur_slots ? nullptr : cur, nullptr)))
+        return MZ_ENOMEM;
+      rc = add_conv(*first, g, cur, cur_index, cur_slots, batch, tab_, action, nullptr, out,
+                    (last && !late_norm) ? norm_out : nullptr, (last && !late_norm) ? slots : nullptr, out_index, st);
       if (rc) return rc;
       cur = dst; cur_index = nullptr; cur_slots = false; which ^= 1;
     }
     for (int i = 0; i < nblk; ++i) {
       const bool last = (i == nblk - 1);
-      rc = add_conv(blk[2 * i], g, cur, cur_index, cur_slots, batch, nullptr, nullptr, nullptr, b2, nullptr, nullptr, nullptr, st);
+      act_t* mid = b2;
+      if (cap && !(mid = cap_take(MZ_DEBUG_CONV, g, batch, blk[2 * i].n_out / 8, cur_slots ? nullptr : cur, nullptr)))
+        return MZ_ENOMEM;
+      rc = add_conv(blk[2 * i], g, cur, cur_index, cur_slots, batch, nullptr, nullptr, nullptr, mid, nullptr, nullptr, nullptr, st);
       if (rc) return rc;
       if (cur_slots) { set_error("internal: residual input must be contiguous"); return MZ_EINVAL; }
       // The block's output goes back INTO the buffer its input came from: element (row, channel) of the residual is read
@@ -1510,12 +1613,15 @@ struct ConvNet : NetImpl {
       if (dst == cur) dst = pp[which ^ 1];
       if (cur == b0 || cur == b1 || cur == b3) dst = const_cast<act_t*>(cur);
       if (last && raw_dst) dst = raw_dst;
-      rc = add_conv(blk[2 * i + 1], g, b2, nullptr, false, batch, nullptr, nullptr, cur,
-                    (last && normalise && !keep_raw) ? nullptr : dst, (last && !late_norm) ? norm_out : nullptr,
-                    (last && !late_norm) ? slots : nullptr, out_index, st);
+      act_t* out = (last && normalise && !keep_raw) ? nullptr : dst;
+      if (cap && !(dst = out = cap_take(MZ_DEBUG_CONV, g, batch, blk[2 * i + 1].n_out / 8, mid, cur))) return MZ_ENOMEM;
+      rc = add_conv(blk[2 * i + 1], g, mid, nullptr, false, batch, nullptr, nullptr, cur, out,
+                    (last && !late_norm) ? norm_out : nullptr, (last && !late_norm) ? slots : nullptr, out_index, st);
       if (rc) return rc;
       cur = dst; which ^= 1;
     }
+    // the normalised state the next tower reads (b3 is not moved): one more tensor of the record
+    if (cap && norm_out) cap_add(norm_out, MZ_DEBUG_NORM, g, batch, C / 8, cap_find(cur), -1);
     if (late_norm) {
       if ((rc = flush(st))) return rc;
       const int Ptot = batch * g.PB();
@@ -1541,14 +1647,22 @@ struct ConvNet : NetImpl {
       pack_obs_kernel<<<num_sms * 8, 256, 0, st>>>(obs, xobs, batch, cfg.in_channels, Hin, Win, 16, plane_rows_of(g0, batch));
     prof_mark(-1, st);
     MZ_LAUNCH_CHECK("pack_obs_kernel");
+    if (capturing()) cap_add(xobs, MZ_DEBUG_OBS, g0, batch, 2, -1, -1);
     // stride-2 conv + ReLU: one tcgen05 launch at the input resolution whose epilogue stores the even positions on
     // the half-size grid
-    auto s2 = [&](const ConvLayer& L, const act_t* in, act_t* out, const Geo& gi) -> int {
+    // under capture the stride-2 convs and the first pool write a region of their own: `out` returns where
+    auto s2 = [&](const ConvLayer& L, const act_t* in, act_t*& out, const Geo& gi) -> int {
+      if (capturing() && !(out = cap_take(MZ_DEBUG_CONV, Geo{gi.H / 2, gi.W / 2}, batch, L.n_out / 8, in, nullptr)))
+        return MZ_ENOMEM;
       int rc2 = add_conv(L, gi, in, nullptr, false, batch, nullptr, nullptr, nullptr, out, nullptr, nullptr, nullptr, st, true);
       if (rc2) return rc2;
       return flush(st);
     };
-    auto pool = [&](const act_t* in, act_t* out, act_t* sl, const int32_t* idx, const Geo& gi, const Geo& go, int norm) -> int {
+    auto pool = [&](const act_t* in, act_t*& out, act_t* sl, const int32_t* idx, const Geo& gi, const Geo& go, int norm) -> int {
+      if (capturing()) {
+        if (out == b3) cap_add(out, MZ_DEBUG_POOL, go, batch, C / 8, cap_find(in), -1);   // the normalised state
+        else if (!(out = cap_take(MZ_DEBUG_POOL, go, batch, C / 8, in, nullptr))) return MZ_ENOMEM;
+      }
       prof_mark(kProfPack, st);
       avgpool_kernel<<<num_sms * 8, 256, 0, st>>>(in, out, sl, idx, batch, gi.H, gi.W, norm, plane_rows_of(gi, batch),
                                                   plane_rows_of(go, batch), C);
@@ -1559,8 +1673,9 @@ struct ConvNet : NetImpl {
     act_t* fin;
     int rc;
     // every writer writes every row of the grid it produces, so grids of different sizes can reuse the same buffers
-    if ((rc = s2(s2_1, xobs, b0, g0))) return rc;                                              // relu(conv_1)
-    if ((rc = tower(nullptr, at_blocks[0], 2, g1, b0, nullptr, false, nullptr, nullptr, batch, true, nullptr, nullptr,
+    act_t* c1 = b0;
+    if ((rc = s2(s2_1, xobs, c1, g0))) return rc;                                              // relu(conv_1)
+    if ((rc = tower(nullptr, at_blocks[0], 2, g1, c1, nullptr, false, nullptr, nullptr, batch, true, nullptr, nullptr,
                     nullptr, st, &fin))) return rc;
     if ((rc = flush(st))) return rc;
     act_t* nxt = (fin == b0) ? b1 : b0;
@@ -1573,12 +1688,14 @@ struct ConvNet : NetImpl {
     if ((rc = tower(nullptr, at_blocks[2], 2, g3, nxt, nullptr, false, nullptr, nullptr, batch, true, nullptr, nullptr,
                     nullptr, st, &fin))) return rc;
     if ((rc = flush(st))) return rc;
-    return pool(fin, b3, slots, dst_index, g3, lat, 1);                                        // avg_pool_2 + normalise
+    act_t* norm = b3;
+    return pool(fin, norm, slots, dst_index, g3, lat, 1);                                      // avg_pool_2 + normalise
   }
 
   int initial(int batch, const float* obs, void* hidden_out, const int32_t* dst_index, float* pi_probs, float* value,
               cudaStream_t st) override {
     int rc;
+    if (capturing()) cap_begin();
     if (atari) {
       rc = represent_atari(batch, obs, nullptr, nullptr, (act_t*)hidden_out, dst_index, st);
     } else {
@@ -1587,6 +1704,7 @@ struct ConvNet : NetImpl {
                                                    plane_rows_of(lat, batch));
       prof_mark(-1, st);
       MZ_LAUNCH_CHECK("pack_obs_kernel");
+      if (capturing()) cap_add(xobs, MZ_DEBUG_OBS, lat, batch, in_cg, -1, -1);
       act_t* fin;
       // representation: raw output is not needed, normalised goes to b3 (for the prediction tower) and the slots
       rc = tower(&rep0, rep_blocks, blocks, lat, xobs, nullptr, false, nullptr, nullptr, batch, false, b3,
@@ -1604,6 +1722,7 @@ struct ConvNet : NetImpl {
                 "with an even number of stacked planes");
       return MZ_EINVAL;
     }
+    if (capturing()) cap_begin();
     int rc = represent_atari(batch, nullptr, frames, plane_values, (act_t*)hidden_out, dst_index, st);
     if (rc) return rc;
     if ((rc = predict(batch, pi_probs, value, st))) return rc;
@@ -1612,6 +1731,7 @@ struct ConvNet : NetImpl {
 
   int predict(int batch, float* pi_probs, float* value, cudaStream_t st) {
     act_t* fin;
+    if (capturing()) cap_set_stage(2);
     int rc = tower(nullptr, pred_blocks, blocks, lat, b3, nullptr, false, nullptr, nullptr, batch, true, nullptr, nullptr,
                    nullptr, st, &fin);
     if (rc) return rc;
@@ -1625,6 +1745,7 @@ struct ConvNet : NetImpl {
                 const int32_t* dst_index, float* reward_out, float* value_out, float* pi_probs,
                 cudaStream_t st) override {
     act_t* fin;
+    if (capturing()) { cap_begin(); cap_set_stage(1); }
     // dynamics: raw output (for the reward head) in a ping-pong buffer, normalised copy in b3 + the slots
     // The dynamics tower and the prediction tower run as ONE launch; the dynamics' raw output goes to b4,
     // which the prediction tower never touches, so the reward head can read it afterwards.

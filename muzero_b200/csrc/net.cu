@@ -153,6 +153,28 @@ extern "C" int mz_net_set_cta_limit(mz_net* net, int32_t max_ctas) {
   return MZ_OK;
 }
 
+extern "C" int mz_net_debug_capture_bytes(mz_net* net, int32_t batch, size_t* bytes) {
+  MZ_CHECK_ARG(net && bytes, "NULL argument");
+  MZ_CHECK_ARG(batch > 0 && batch <= net->max_batch, "batch %d outside (0, %d]", batch, net->max_batch);
+  return net->impl->debug_capture_bytes(batch, bytes);
+}
+
+extern "C" int mz_net_debug_capture(mz_net* net, void* buf, size_t bytes) {
+  MZ_CHECK_ARG(net, "NULL argument");
+  MZ_CHECK_ARG(((uintptr_t)buf & 255) == 0, "capture buffer must be 256-byte aligned");
+  return net->impl->debug_capture(buf, bytes);
+}
+
+extern "C" int mz_net_debug_tensor(mz_net* net, int32_t index, mz_debug_tensor* out, int32_t* count) {
+  MZ_CHECK_ARG(net && count && (index < 0 || out), "NULL argument");
+  return net->impl->debug_tensor(index, out, count);
+}
+
+extern "C" int mz_net_debug_launch(mz_net* net, int32_t index, mz_debug_launch* out, int32_t* count) {
+  MZ_CHECK_ARG(net && count && (index < 0 || out), "NULL argument");
+  return net->impl->debug_launch(index, out, count);
+}
+
 extern "C" int mz_net_profile_begin(mz_net* net) {
   MZ_CHECK_ARG(net, "NULL argument");
   NetImpl* n = net->impl;
