@@ -177,7 +177,10 @@ int mz_net_arena_bytes(const mz_net_config* cfg, int32_t max_batch, size_t* byte
 /* weights: array of `num_weights` device pointers to float32 tensors in the
  * reference's state_dict order and PyTorch layouts (see muzero_b200/network.py);
  * they are repacked (transposed / BatchNorm folded / converted) into the arena
- * synchronously, so the caller may free them afterwards. */
+ * synchronously, so the caller may free them afterwards.
+ * MLP nets: recurrent inference runs on tensor cores (tcgen05) for hidden_dim 64, num_planes 256 or 512 and supports
+ * up to 32 (with a policy: up to 64 actions), on the fp32 SIMT kernel otherwise; a net whose SIMT kernel would need
+ * more than 227 KB of shared memory (e.g. num_planes 2048 at hidden_dim 64) is refused with MZ_EINVAL. */
 int mz_net_create(const mz_net_config* cfg, const float* const* weights, int32_t num_weights,
                   int32_t max_batch, void* arena_dev, size_t arena_bytes, mz_net** out);
 int mz_net_destroy(mz_net* net);
@@ -251,7 +254,7 @@ int mz_net_set_cta_limit(mz_net* net, int32_t max_ctas);
 int mz_net_profile_begin(mz_net* net);
 int mz_net_profile_end(mz_net* net, double* ms_by_class /* [5] */, int64_t* launches_by_class /* [5] */);
 
-/* ---- test aid of the conv nets: keep every intermediate tensor of an inference call ----
+/* ---- test aid: keep every intermediate tensor of an inference call ----
  * The towers reuse their activation buffers (ping-pong, residual blocks write over their input), so the layers of a
  * call are gone when it returns.  With capture on (buf != NULL, device memory of at least mz_net_debug_capture_bytes),
  * every conv output and every pool output of the next calls goes to a region of its own in `buf`, and the last layer
@@ -260,9 +263,23 @@ int mz_net_profile_end(mz_net* net, double* ms_by_class /* [5] */, int64_t* laun
  *   tensors: the packed observation, every conv / pool output, and the normalised state the prediction tower reads
  *            (planes [groups][plane_rows][8] fp16, board b at rows b*h*w ...);
  *   launches: one per conv3x3_kernel launch, with the form the host chose for it.
- * buf = NULL turns capture off.  MLP nets: MZ_EINVAL. */
+ * buf = NULL turns capture off.  A buffer too small for a call fails that call with MZ_ENOMEM and queues nothing.
+ *
+ * MLP nets record tensors of kind MZ_DEBUG_MLP, row i of a region holding batch row i, and read the fields as:
+ *   stage = net (0 representation, 1 transition, 2 reward, 3 value, 4 policy), index = layer (0 the hidden layer after
+ *   bias, action column and ReLU; 1 the second Linear + bias before its transform: raw state or logits; 2 the
+ *   normalised state), plane_rows = rows, groups = columns, h = row stride in elements, w = bytes per element (2 fp16,
+ *   4 fp32), batch = the CTA part that wrote it (1: the second CTA of a tile in the split form, else 0), src = the
+ *   tensor read (-1: observation or hidden-state slots; value and policy layer 0 of the tcgen05 kernel: the transition
+ *   output whose normalisation they read), residual = -1.
+ * The tcgen05 kernel records per net and CTA part the fp16 hidden layer as its first epilogue stores it (P columns:
+ * chunk c at columns 256 c ..) and the fp32 second-layer output; the SIMT kernels every dense output and the normalised
+ * state, fp32.  One launch record per kernel launch: tile_rows = rows per tile (32: SIMT kernel, 128: tcgen05),
+ * pair = CTAs per tile (2: the split form), grid, num_tiles, multi_pass = 256-column chunks (tcgen05, else 0),
+ * n = 1 if the policy net ran, resident = 1 if the action table was in shared memory, sub = 0 initial / 1 recurrent,
+ * num_layers = nets run, h = num_planes, w = num_actions, batch; the rest 0. */
 #define MZ_DEBUG_MAX_LAYERS 34
-enum mz_debug_kind { MZ_DEBUG_OBS = 0, MZ_DEBUG_CONV = 1, MZ_DEBUG_POOL = 2, MZ_DEBUG_NORM = 3 };
+enum mz_debug_kind { MZ_DEBUG_OBS = 0, MZ_DEBUG_CONV = 1, MZ_DEBUG_POOL = 2, MZ_DEBUG_NORM = 3, MZ_DEBUG_MLP = 4 };
 typedef struct {
   void* ptr;
   int32_t kind;            /* mz_debug_kind */

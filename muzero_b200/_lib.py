@@ -47,7 +47,7 @@ class DebugTensor(C.Structure):
 
 
 MZ_DEBUG_MAX_LAYERS = 34
-MZ_DEBUG_OBS, MZ_DEBUG_CONV, MZ_DEBUG_POOL, MZ_DEBUG_NORM = 0, 1, 2, 3
+MZ_DEBUG_OBS, MZ_DEBUG_CONV, MZ_DEBUG_POOL, MZ_DEBUG_NORM, MZ_DEBUG_MLP = 0, 1, 2, 3, 4
 
 
 class DebugLaunch(C.Structure):

@@ -9,6 +9,7 @@
 #include "common.cuh"
 #include "net.cuh"
 #include "umma.cuh"
+#include <algorithm>
 #include <type_traits>
 #include "tree_thread.cuh"
 #include "tree_warp.cuh"
@@ -198,15 +199,17 @@ __device__ void normalise_and_store(const float* hraw, float* hn, int HD, float*
 struct Smem {
   float *x, *h1, *hraw, *hn, *lg;
   int *arow;
-  int ldx, ldl;
+  int ldx, ldh, ldl;
 };
+// row strides are multiples of 4 floats: dense_cols reads its input rows as float4
 __device__ Smem carve(const MlpDev& n, float* base) {
   Smem s;
   s.ldx = max(n.in_pad, n.HD);
+  s.ldh = (n.P + 3) & ~3;
   s.ldl = (max(max(n.A, n.Sv), n.Sr) + 3) & ~3;
   s.x = base;
   s.h1 = s.x + kRows * s.ldx;
-  s.hraw = s.h1 + kRows * n.P;
+  s.hraw = s.h1 + kRows * s.ldh;
   s.hn = s.hraw + kRows * n.HD;
   s.lg = s.hn + kRows * n.HD;
   s.arow = reinterpret_cast<int*>(s.lg + kRows * s.ldl);
@@ -217,21 +220,43 @@ size_t smem_bytes(const MlpDev& n) {
   int m = n.A > n.Sv ? n.A : n.Sv;
   m = m > n.Sr ? m : n.Sr;
   const int ldl = (m + 3) & ~3;
-  return sizeof(float) * ((size_t)kRows * ldx + (size_t)kRows * n.P + 2 * (size_t)kRows * n.HD + (size_t)kRows * ldl) +
+  const int ldh = (n.P + 3) & ~3;
+  return sizeof(float) * ((size_t)kRows * ldx + (size_t)kRows * ldh + 2 * (size_t)kRows * n.HD + (size_t)kRows * ldl) +
          sizeof(int) * kRows;
 }
 
 extern __shared__ __align__(16) float mlp_smem[];
 
+// Test aid (mz_net_debug_capture): where the SIMT kernels copy every dense output and the normalised state, each to a
+// [batch][columns] fp32 region of its own (nullptr: not captured).  Every captured shared-memory tensor is next written
+// at least one dense() -- and so one barrier -- later, so the copy needs no barrier of its own.
+enum SimtCapSlot { kCapNet0L0 = 0, kCapNet0L1, kCapNorm, kCapRewL0, kCapRewL1, kCapPolL0, kCapPolL1, kCapValL0, kCapValL1,
+                   kCapSlots };
+struct MlpSimtCap {
+  float* t[kCapSlots];
+};
+__device__ void cap_rows(float* dst, const float* src, int ld, int cols, int row0, int batch) {
+  if (dst == nullptr) return;
+  for (int i = threadIdx.x; i < kRows * cols; i += blockDim.x) {
+    const int r = i / cols, j = i % cols;
+    if (row0 + r < batch) dst[(size_t)(row0 + r) * cols + j] = src[(size_t)r * ld + j];
+  }
+}
+
 // prediction heads on the normalised state in s.hn (network.py:223-233)
-__device__ void prediction_heads(const MlpDev& n, const Smem& s, float* pi_probs, float* value, int row0, int batch) {
+__device__ void prediction_heads(const MlpDev& n, const Smem& s, float* pi_probs, float* value, int row0, int batch,
+                                 const MlpSimtCap& cap) {
   if (pi_probs != nullptr) {
-    dense(n.pol1_wt, nullptr, n.pol1_b, s.hn, n.HD, n.HD, n.P, true, s.h1, n.P);
-    dense(n.pol2_wt, n.pol2_w, n.pol2_b, s.h1, n.P, n.P, n.A, false, s.lg, s.ldl);
+    dense(n.pol1_wt, nullptr, n.pol1_b, s.hn, n.HD, n.HD, n.P, true, s.h1, s.ldh);
+    cap_rows(cap.t[kCapPolL0], s.h1, s.ldh, n.P, row0, batch);
+    dense(n.pol2_wt, n.pol2_w, n.pol2_b, s.h1, s.ldh, n.P, n.A, false, s.lg, s.ldl);
+    cap_rows(cap.t[kCapPolL1], s.lg, s.ldl, n.A, row0, batch);
     softmax_rows(s.lg, s.ldl, n.A, pi_probs, row0, batch);
   }
-  dense(n.val1_wt, nullptr, n.val1_b, s.hn, n.HD, n.HD, n.P, true, s.h1, n.P);
-  dense(n.val2_wt, n.val2_w, n.val2_b, s.h1, n.P, n.P, n.Sv, false, s.lg, s.ldl);
+  dense(n.val1_wt, nullptr, n.val1_b, s.hn, n.HD, n.HD, n.P, true, s.h1, s.ldh);
+  cap_rows(cap.t[kCapValL0], s.h1, s.ldh, n.P, row0, batch);
+  dense(n.val2_wt, n.val2_w, n.val2_b, s.h1, s.ldh, n.P, n.Sv, false, s.lg, s.ldl);
+  cap_rows(cap.t[kCapValL1], s.lg, s.ldl, n.Sv, row0, batch);
   support_to_scalar(s.lg, s.ldl, n.Sv, value, row0, batch);
 }
 
@@ -240,7 +265,7 @@ __device__ void prediction_heads(const MlpDev& n, const Smem& s, float* pi_probs
 __global__ void __launch_bounds__(kInitThreads)
 mlp_initial_kernel(MlpDev n, int batch, const float* __restrict__ obs, float* __restrict__ hidden_out,
                    const int32_t* __restrict__ dst_index, float* __restrict__ pi_probs, float* __restrict__ value,
-                   const __grid_constant__ RootSetup rs) {
+                   const __grid_constant__ RootSetup rs, const __grid_constant__ MlpSimtCap cap) {
   const Smem s = carve(n, mlp_smem);
   const int row0 = blockIdx.x * kRows;
   for (int i = threadIdx.x; i < kRows * s.ldx; i += blockDim.x) {
@@ -248,10 +273,13 @@ mlp_initial_kernel(MlpDev n, int batch, const float* __restrict__ obs, float* __
     s.x[i] = (row0 + r < batch && k < n.in_dim) ? obs[(size_t)(row0 + r) * n.in_dim + k] : 0.0f;
   }
   __syncthreads();
-  dense(n.rep1_wt, nullptr, n.rep1_b, s.x, s.ldx, n.in_dim, n.P, true, s.h1, n.P);
-  dense(n.rep2_wt, nullptr, n.rep2_b, s.h1, n.P, n.P, n.HD, false, s.hraw, n.HD);
+  dense(n.rep1_wt, nullptr, n.rep1_b, s.x, s.ldx, n.in_dim, n.P, true, s.h1, s.ldh);
+  cap_rows(cap.t[kCapNet0L0], s.h1, s.ldh, n.P, row0, batch);
+  dense(n.rep2_wt, nullptr, n.rep2_b, s.h1, s.ldh, n.P, n.HD, false, s.hraw, n.HD);
+  cap_rows(cap.t[kCapNet0L1], s.hraw, n.HD, n.HD, row0, batch);
   normalise_and_store(s.hraw, s.hn, n.HD, hidden_out, dst_index, row0, batch);
-  prediction_heads(n, s, pi_probs, value, row0, batch);
+  cap_rows(cap.t[kCapNorm], s.hn, n.HD, n.HD, row0, batch);
+  prediction_heads(n, s, pi_probs, value, row0, batch, cap);
   if (rs.enabled) {
     // fused root preparation (mz_net_initial_search): the warp that wrote row r's softmax (softmax_rows: warp r % 8,
     // lane i -> actions i, i + 32, ...) draws the tree's Dirichlet noise, mixes, masks, renormalises and resets the tree
@@ -265,7 +293,7 @@ __global__ void __launch_bounds__(kThreads)
 mlp_recurrent_kernel(MlpDev n, int batch, const float* __restrict__ hidden_in, const int32_t* __restrict__ src_index,
                      const int32_t* __restrict__ action, float* __restrict__ hidden_out,
                      const int32_t* __restrict__ dst_index, float* __restrict__ reward, float* __restrict__ value,
-                     float* __restrict__ pi_probs) {
+                     float* __restrict__ pi_probs, const __grid_constant__ MlpSimtCap cap) {
   const Smem s = carve(n, mlp_smem);
   const int row0 = blockIdx.x * kRows;
   // leaf gather: parent hidden state by slot index + the action as a weight-row index
@@ -285,14 +313,19 @@ mlp_recurrent_kernel(MlpDev n, int batch, const float* __restrict__ hidden_in, c
     s.arow[r] = n.HD + a;      // one-hot(action) concatenated after the state (network.py:191-193)
   }
   __syncthreads();
-  dense(n.dyn1_wt, nullptr, n.dyn1_b, s.x, s.ldx, n.HD, n.P, true, s.h1, n.P, s.arow);
-  dense(n.dyn2_wt, nullptr, n.dyn2_b, s.h1, n.P, n.P, n.HD, false, s.hraw, n.HD);
+  dense(n.dyn1_wt, nullptr, n.dyn1_b, s.x, s.ldx, n.HD, n.P, true, s.h1, s.ldh, s.arow);
+  cap_rows(cap.t[kCapNet0L0], s.h1, s.ldh, n.P, row0, batch);
+  dense(n.dyn2_wt, nullptr, n.dyn2_b, s.h1, s.ldh, n.P, n.HD, false, s.hraw, n.HD);
+  cap_rows(cap.t[kCapNet0L1], s.hraw, n.HD, n.HD, row0, batch);
   // reward head reads the UN-normalised state (network.py:195-196)
-  dense(n.rew1_wt, nullptr, n.rew1_b, s.hraw, n.HD, n.HD, n.P, true, s.h1, n.P);
-  dense(n.rew2_wt, n.rew2_w, n.rew2_b, s.h1, n.P, n.P, n.Sr, false, s.lg, s.ldl);
+  dense(n.rew1_wt, nullptr, n.rew1_b, s.hraw, n.HD, n.HD, n.P, true, s.h1, s.ldh);
+  cap_rows(cap.t[kCapRewL0], s.h1, s.ldh, n.P, row0, batch);
+  dense(n.rew2_wt, n.rew2_w, n.rew2_b, s.h1, s.ldh, n.P, n.Sr, false, s.lg, s.ldl);
+  cap_rows(cap.t[kCapRewL1], s.lg, s.ldl, n.Sr, row0, batch);
   support_to_scalar(s.lg, s.ldl, n.Sr, reward, row0, batch);
   normalise_and_store(s.hraw, s.hn, n.HD, hidden_out, dst_index, row0, batch);
-  prediction_heads(n, s, pi_probs, value, row0, batch);
+  cap_rows(cap.t[kCapNorm], s.hn, n.HD, n.HD, row0, batch);
+  prediction_heads(n, s, pi_probs, value, row0, batch, cap);
 }
 
 __global__ void transpose_kernel(const float* __restrict__ w, float* __restrict__ wt, int out, int in) {
@@ -318,7 +351,9 @@ __global__ void transpose_kernel(const float* __restrict__ w, float* __restrict_
 // util.py:70-93, softmax).  Operands are fp16 (the hidden state is normalised to [0,1]), accumulation fp32.
 // Weights are pre-packed per (net, chunk, layer) block in exactly the shared-memory core-matrix layout and
 // streamed by a producer warp with 1-D bulk copies (TMA) through a 3-slot mbarrier ring, so the next block
-// loads while the current one is multiplied.
+// loads while the current one is multiplied.  Widths 256 and 512 only: MlpTcParams holds kTcMaxBlocks = 16 blocks, two
+// per chunk of each of the three nets a search runs (the policy's adds two more per chunk); mlp_create sends every
+// other width to the SIMT kernels.
 
 constexpr int kTcRows = 128;          // rows per tile == compute threads
 constexpr int kTcCompute = 256;       // 8 compute warps: warps 0-3 own the tile's rows (thread = row), warps 4-7 share
@@ -344,6 +379,13 @@ struct MlpTcParams {
   const float* hidden_in; const int32_t* src_index; const int32_t* action;
   float* hidden_out; const int32_t* dst_index; float* reward; float* value; float* pi;
   long long* dbg;                     // MZ_MLP_DEBUG: clock64 stamps of CTA 0 / thread 0 (measurement aid)
+};
+// Test aid (mz_net_debug_capture, read by the kCap instantiation only), per net and CTA part: the fp16 hidden layer as
+// epilogue 1 stores it ([batch][P]) and the fp32 second-layer output + bias before its transform ([batch][64 | 32 | 32 |
+// A]).  The last kernel parameter, so that the parameters before it keep their offsets in every instantiation.
+struct MlpTcCap {
+  __half* mid[4][2];
+  float* out[4][2];
 };
 
 __device__ __forceinline__ uint32_t pack_h2(float a, float b) {
@@ -412,9 +454,11 @@ struct SearchArgs {
 // so a simulation costs no launch, no prologue (TMEM allocation, bias / action-table staging, barrier set-up happen
 // once per search) and the leaf action, reward and value never leave the thread's registers.  Trees of different
 // CTAs never interact, so there is no inter-CTA synchronisation at all.
-template <bool kSearch, int TA>
+// kCap: the test instantiation that also copies every intermediate to the capture regions of MlpTcParams.
+template <bool kSearch, int TA, bool kCap = false>
 __global__ void __launch_bounds__(kTcThreads, 1) mlp_tc_kernel(const __grid_constant__ MlpTcParams p,
-                                                               const __grid_constant__ SearchArgs sa) {
+                                                               const __grid_constant__ SearchArgs sa,
+                                                               const __grid_constant__ MlpTcCap cap) {
   extern __shared__ __align__(1024) unsigned char tsm[];
   unsigned char* sIn = tsm;                       // [8][128][16]  h_in   (fp16, K-major core matrices)
   unsigned char* sRaw = sIn + 16384;              // h_raw
@@ -609,6 +653,17 @@ __global__ void __launch_bounds__(kTcThreads, 1) mlp_tc_kernel(const __grid_cons
                            "r"(pack_h2(fmaxf(w[0], 0.f), fmaxf(w[1], 0.f))), "r"(pack_h2(fmaxf(w[2], 0.f), fmaxf(w[3], 0.f))),
                            "r"(pack_h2(fmaxf(w[4], 0.f), fmaxf(w[5], 0.f))), "r"(pack_h2(fmaxf(w[6], 0.f), fmaxf(w[7], 0.f))) : "memory");
             }
+            if constexpr (kCap) {
+              if (live) {
+                uint4* dst = reinterpret_cast<uint4*>(cap.mid[net][part] + (size_t)grow * p.P + col0);
+#pragma unroll
+                for (int u = 0; u < 4; ++u) {
+                  const float* w = v + 8 * u;
+                  dst[u] = make_uint4(pack_h2(fmaxf(w[0], 0.f), fmaxf(w[1], 0.f)), pack_h2(fmaxf(w[2], 0.f), fmaxf(w[3], 0.f)),
+                                      pack_h2(fmaxf(w[4], 0.f), fmaxf(w[5], 0.f)), pack_h2(fmaxf(w[6], 0.f), fmaxf(w[7], 0.f)));
+                }
+              }
+            }
           }
           fence_proxy_async();
           tc_fence_before();
@@ -631,6 +686,13 @@ __global__ void __launch_bounds__(kTcThreads, 1) mlp_tc_kernel(const __grid_cons
             tmem_ld_wait();
 #pragma unroll
             for (int e = 0; e < 32; ++e) h[q * 32 + e] = __uint_as_float(r[e]) + __ldg(b2 + q * 32 + e);
+          }
+          if constexpr (kCap) {
+            if (live) {
+              float4* dst = reinterpret_cast<float4*>(cap.out[0][part] + (size_t)grow * 64);
+#pragma unroll
+              for (int g = 0; g < 16; ++g) dst[g] = make_float4(h[4 * g], h[4 * g + 1], h[4 * g + 2], h[4 * g + 3]);
+            }
           }
           stamp();
           float mn = INFINITY, mx = -INFINITY;
@@ -668,6 +730,13 @@ __global__ void __launch_bounds__(kTcThreads, 1) mlp_tc_kernel(const __grid_cons
           float l[32];
 #pragma unroll
           for (int e = 0; e < 32; ++e) l[e] = __uint_as_float(r[e]) + (e < S ? __ldg(b2 + e) : 0.0f);
+          if constexpr (kCap) {
+            if (live) {
+#pragma unroll
+              for (int e = 0; e < 32; ++e)
+                if (e < S) cap.out[net][part][(size_t)grow * 32 + e] = l[e];
+            }
+          }
           const float out = support_scalar_regs(l, S);
           if (kSearch) { if (net == 1) rew_reg = out; else val_reg = out; }
           else if (live) (net == 1 ? p.reward : p.value)[grow] = out;
@@ -684,6 +753,9 @@ __global__ void __launch_bounds__(kTcThreads, 1) mlp_tc_kernel(const __grid_cons
                 const int a = q * 32 + e;
                 if (a < p.A) {
                   const float lg = __uint_as_float(r[e]) + __ldg(b2 + a);
+                  if constexpr (kCap) {
+                    if (pass == 0 && live) cap.out[3][part][(size_t)grow * p.A + a] = lg;
+                  }
                   if (pass == 0) m = fmaxf(m, lg);
                   else if (pass == 1) den += expf(lg - m);
                   else if (live) p.pi[(size_t)grow * p.A + a] = expf(lg - m) / den;
@@ -1020,20 +1092,130 @@ struct MlpNet : NetImpl {
   int tc_blocks_no_policy = 0, tc_blocks_policy = 0, num_sms = 148;
   size_t tc_smem = 0;
 
+  // ---- test aid (mz_net_debug_capture): every intermediate of a call in a region of its own ----
+  // Nets of a record: 0 representation, 1 transition, 2 reward, 3 value, 4 policy.  Layers: 0 the hidden layer (bias,
+  // action column, ReLU), 1 the second Linear + bias before its transform, 2 the normalised state (SIMT kernels).
+  char* cap_buf = nullptr;
+  size_t cap_size = 0, cap_used = 0;
+  bool cap_full = false;
+  std::vector<mz_debug_tensor> cap_tensors;
+  std::vector<mz_debug_launch> cap_launches;
+  bool capturing() const { return cap_buf != nullptr; }
+  void cap_begin() { cap_used = 0; cap_full = false; cap_tensors.clear(); cap_launches.clear(); }
+  // a region [batch][stride] for one tensor and its record (nullptr and cap_full: the buffer is too small)
+  void* cap_take(int net, int layer, int batch, int cols, int stride, int ebytes, int part, int src) {
+    const size_t bytes = align_up((size_t)batch * stride * ebytes, 256);
+    if (cap_full || cap_used + bytes > cap_size) { cap_full = true; return nullptr; }
+    void* r = cap_buf + cap_used;
+    cap_used += bytes;
+    mz_debug_tensor t = {};
+    t.ptr = r; t.kind = MZ_DEBUG_MLP; t.stage = net; t.index = layer; t.plane_rows = batch; t.groups = cols;
+    t.h = stride; t.w = ebytes; t.batch = part; t.src = src; t.residual = -1;
+    cap_tensors.push_back(t);
+    return r;
+  }
+  int cap_last() const { return (int)cap_tensors.size() - 1; }
+  int cap_fail() {
+    set_error("mz_net_debug_capture: buffer of %zu bytes too small", cap_size);
+    return MZ_ENOMEM;
+  }
+  void cap_launch(int recurrent, int tile_rows, int nsplit, int grid, int tiles, int chunks, int nets, bool policy,
+                  int tab_in_smem, int batch) {
+    mz_debug_launch L = {};
+    L.num_layers = nets; L.tile_rows = tile_rows; L.pair = nsplit; L.grid = grid; L.num_tiles = tiles;
+    L.multi_pass = chunks; L.n = policy ? 1 : 0; L.resident = tab_in_smem; L.sub = recurrent;
+    L.h = d.P; L.w = d.A; L.batch = batch;
+    cap_launches.push_back(L);
+  }
+  // the regions of a SIMT call (slots of MlpSimtCap), recorded in execution order
+  MlpSimtCap cap_simt(bool recurrent, int batch, bool policy) {
+    MlpSimtCap c = {};
+    const int net0 = recurrent ? 1 : 0;
+    c.t[kCapNet0L0] = (float*)cap_take(net0, 0, batch, d.P, d.P, 4, 0, -1);
+    const int l0 = cap_last();
+    c.t[kCapNet0L1] = (float*)cap_take(net0, 1, batch, d.HD, d.HD, 4, 0, l0);
+    const int raw = cap_last();
+    if (recurrent) {
+      c.t[kCapRewL0] = (float*)cap_take(2, 0, batch, d.P, d.P, 4, 0, raw);
+      c.t[kCapRewL1] = (float*)cap_take(2, 1, batch, d.Sr, d.Sr, 4, 0, cap_last());
+    }
+    c.t[kCapNorm] = (float*)cap_take(net0, 2, batch, d.HD, d.HD, 4, 0, raw);
+    const int norm = cap_last();
+    if (policy) {
+      c.t[kCapPolL0] = (float*)cap_take(4, 0, batch, d.P, d.P, 4, 0, norm);
+      c.t[kCapPolL1] = (float*)cap_take(4, 1, batch, d.A, d.A, 4, 0, cap_last());
+    }
+    c.t[kCapValL0] = (float*)cap_take(3, 0, batch, d.P, d.P, 4, 0, norm);
+    c.t[kCapValL1] = (float*)cap_take(3, 1, batch, d.Sv, d.Sv, 4, 0, cap_last());
+    return c;
+  }
+  // the regions of a tcgen05 call: per CTA part, the nets it runs (value and policy read the normalisation of their
+  // part's transition output)
+  void cap_tc(const MlpTcParams& q, MlpTcCap& c) {
+    const int S2[4] = {64, 32, 32, q.A};
+    const int cols2[4] = {64, q.Sr, q.Sv, q.A};
+    for (int part = 0; part < q.nsplit; ++part) {
+      int raw = -1;
+      for (int n = 0; n < q.nnets; ++n) {
+        if (!(q.nsplit == 1 || n == 0 || (n == 1) == (part == 0))) continue;
+        c.mid[n][part] = (__half*)cap_take(n + 1, 0, q.batch, q.P, q.P, 2, part, n == 0 ? -1 : raw);
+        c.out[n][part] = (float*)cap_take(n + 1, 1, q.batch, cols2[n], S2[n], 4, part, cap_last());
+        if (n == 0) raw = cap_last();
+      }
+    }
+  }
+  int debug_capture_bytes(int batch, size_t* bytes) override {
+    // more than any one call takes: the SIMT kernels' nine fp32 regions, or the tcgen05 kernel's eight fp16 hidden
+    // layers and eight fp32 outputs (two CTA parts)
+    const int m = std::max(std::max(std::max(d.P, d.HD), std::max(d.A, 64)), std::max(d.Sv, d.Sr));
+    const size_t simt = (size_t)kCapSlots * align_up((size_t)batch * m * 4, 256);
+    const size_t tc_b = 8 * align_up((size_t)batch * d.P * 2, 256) + 8 * align_up((size_t)batch * std::max(d.A, 64) * 4, 256);
+    *bytes = std::max(simt, tc_b);
+    return MZ_OK;
+  }
+  int debug_capture(void* buf, size_t bytes) override {
+    cap_buf = (char*)buf; cap_size = buf ? bytes : 0;
+    cap_begin();
+    return MZ_OK;
+  }
+  int debug_tensor(int index, mz_debug_tensor* out, int32_t* count) override {
+    *count = (int32_t)cap_tensors.size();
+    if (index < 0) return MZ_OK;
+    MZ_CHECK_ARG(index < *count, "tensor %d of %d", index, *count);
+    *out = cap_tensors[index];
+    return MZ_OK;
+  }
+  int debug_launch(int index, mz_debug_launch* out, int32_t* count) override {
+    *count = (int32_t)cap_launches.size();
+    if (index < 0) return MZ_OK;
+    MZ_CHECK_ARG(index < *count, "launch %d of %d", index, *count);
+    *out = cap_launches[index];
+    return MZ_OK;
+  }
+
   int search(mz_pool* pool, cudaStream_t st) override;
   int initial(int batch, const float* obs, void* hidden_out, const int32_t* dst_index, float* pi_probs,
               float* value, cudaStream_t st) override {
+    MlpSimtCap cap = {};
+    const int grid = (batch + kRows - 1) / kRows;
+    if (capturing()) {
+      cap_begin();
+      cap = cap_simt(false, batch, pi_probs != nullptr);
+      if (cap_full) return cap_fail();
+      cap_launch(0, kRows, 1, grid, grid, 0, pi_probs ? 3 : 2, pi_probs != nullptr, 0, batch);
+    }
     prof_mark(kProfMlp, st);
     RootSetup rs;
     if (pending_root) rs = *pending_root; else rs.enabled = 0;
-    mlp_initial_kernel<<<(batch + kRows - 1) / kRows, kInitThreads, smem, st>>>(d, batch, obs, (float*)hidden_out,
-                                                                           dst_index, pi_probs, value, rs);
+    mlp_initial_kernel<<<grid, kInitThreads, smem, st>>>(d, batch, obs, (float*)hidden_out, dst_index, pi_probs, value,
+                                                         rs, cap);
     prof_mark(-1, st);
     MZ_LAUNCH_CHECK("mlp_initial_kernel");
     return MZ_OK;
   }
   int recurrent(int batch, const void* hidden_in, const int32_t* src_index, const int32_t* action, void* hidden_out,
                 const int32_t* dst_index, float* reward, float* value, float* pi_probs, cudaStream_t st) override {
+    if (capturing()) cap_begin();
     if (tc && (pi_probs == nullptr || tc_blocks_policy > 0)) {
       MlpTcParams q = tcp;
       q.batch = batch; q.hidden_in = (const float*)hidden_in; q.src_index = src_index; q.action = action;
@@ -1054,7 +1236,14 @@ struct MlpNet : NetImpl {
       // sit on their SMs spinning until the predecessor drains, and with one 208 KB CTA per SM on most of the GPU
       // (CartPole, 128 tiles) they held up the kernels they were waiting for (172 -> 120 M simulations/s)
       const int grid = q.nsplit == 2 ? 2 * ntiles : (ntiles < num_sms ? ntiles : num_sms);
-      launch_pdl(2 * grid <= num_sms, mlp_tc_kernel<false, 4>, dim3(grid), dim3(kTcThreads), tc_smem, st, q, none);
+      MlpTcCap cap = {};
+      if (capturing()) {
+        cap_tc(q, cap);
+        if (cap_full) return cap_fail();
+        cap_launch(1, kTcRows, q.nsplit, grid, ntiles, q.chunks, q.nnets, pi_probs != nullptr, q.tab_in_smem, batch);
+      }
+      launch_pdl(2 * grid <= num_sms, capturing() ? mlp_tc_kernel<false, 4, true> : mlp_tc_kernel<false, 4>, dim3(grid),
+                 dim3(kTcThreads), tc_smem, st, q, none, cap);
       prof_mark(-1, st);
       MZ_LAUNCH_CHECK("mlp_recurrent_tc_kernel");
       if (debug) {   // measurement aid: cycle stamps of CTA 0 (start, prologue, gather, then per net: MMA1, epi1, MMA2, epi2; end)
@@ -1068,9 +1257,16 @@ struct MlpNet : NetImpl {
       }
       return MZ_OK;
     }
+    MlpSimtCap cap = {};
+    const int grid = (batch + kRows - 1) / kRows;
+    if (capturing()) {
+      cap = cap_simt(true, batch, pi_probs != nullptr);
+      if (cap_full) return cap_fail();
+      cap_launch(1, kRows, 1, grid, grid, 0, pi_probs ? 4 : 3, pi_probs != nullptr, 0, batch);
+    }
     prof_mark(kProfMlp, st);
-    mlp_recurrent_kernel<<<(batch + kRows - 1) / kRows, kThreads, smem, st>>>(
-        d, batch, (const float*)hidden_in, src_index, action, (float*)hidden_out, dst_index, reward, value, pi_probs);
+    mlp_recurrent_kernel<<<grid, kThreads, smem, st>>>(d, batch, (const float*)hidden_in, src_index, action,
+                                                       (float*)hidden_out, dst_index, reward, value, pi_probs, cap);
     prof_mark(-1, st);
     MZ_LAUNCH_CHECK("mlp_recurrent_kernel");
     return MZ_OK;
@@ -1129,8 +1325,9 @@ int MlpNet::search(mz_pool* pool, cudaStream_t st) {
   const int ntiles = (pool->B + kTcRows - 1) / kTcRows;
   const int grid = ntiles < num_sms ? ntiles : num_sms;
   prof_mark(kProfMlp, st);
-  if (pool->A <= 4) mlp_tc_kernel<true, 4><<<grid, kTcThreads, smem_need, st>>>(q, sa);
-  else mlp_tc_kernel<true, 12><<<grid, kTcThreads, smem_need, st>>>(q, sa);
+  const MlpTcCap no_cap = {};
+  if (pool->A <= 4) mlp_tc_kernel<true, 4><<<grid, kTcThreads, smem_need, st>>>(q, sa, no_cap);
+  else mlp_tc_kernel<true, 12><<<grid, kTcThreads, smem_need, st>>>(q, sa, no_cap);
   prof_mark(-1, st);
   MZ_LAUNCH_CHECK("mlp_tc_kernel<search>");
   if (debug) {   // cycle stamps of CTA 0 / thread 0: start, prologue, then per simulation: sim start, tree phase + gather done, ...
@@ -1228,7 +1425,11 @@ int mlp_create(const mz_net_config& c, const float* const* w, int nw, void* aren
     const int P = d.P, A = d.A;
     const int apad = (A + 15) / 16 * 16;
     const char* simt = getenv("MZ_MLP_SIMT");
-    net->tc = d.HD == 64 && P % kTcChunk == 0 && P <= 2048 && d.Sr <= 32 && d.Sv <= 32 && !(simt && simt[0] == '1');
+    // the transition, reward and value nets' 2 blocks per chunk must fit the kTcMaxBlocks entries of MlpTcParams (so
+    // P <= 512), and the kernel's shared memory a block; wider nets run on the SIMT kernel
+    const size_t tc_smem_base = 3 * 16384 + 65536 + (size_t)kTcSlots * kTcSlotBytes + 256 + (size_t)4 * P * 4;
+    net->tc = d.HD == 64 && P % kTcChunk == 0 && 3 * (P / kTcChunk) * 2 <= kTcMaxBlocks && tc_smem_base <= 227 * 1024 &&
+              d.Sr <= 32 && d.Sv <= 32 && !(simt && simt[0] == '1');
     if (net->tc) {
       const int chunks = P / kTcChunk;
       const bool pol = apad <= 64 && 4 * chunks * 2 <= kTcMaxBlocks;
@@ -1245,6 +1446,11 @@ int mlp_create(const mz_net_config& c, const float* const* w, int nw, void* aren
         q.b1[net_i] = orig[w1_idx[net_i] + 1];
         q.b2[net_i] = orig[w1_idx[net_i] + 3];
         for (int ch = 0; ch < chunks; ++ch) {
+          if (nb + 2 > kTcMaxBlocks) {
+            set_error("internal: MLP weight block %d of at most %d", nb + 1, kTcMaxBlocks);
+            delete net;
+            return MZ_EINVAL;
+          }
           // layer 1 block: rows ch*256.., K = 64
           pack_linear_kernel<<<64, 256>>>(orig[w1_idx[net_i]], (__half*)(wp + off), P, in_tot[net_i], ch * kTcChunk,
                                           kTcChunk, 0, 64);
@@ -1266,7 +1472,7 @@ int mlp_create(const mz_net_config& c, const float* const* w, int nw, void* aren
       q.tabA = tab;
       MZ_CUDA(cudaDeviceSynchronize());
       if ((size_t)(p - (char*)arena) > arena_bytes) { set_error("internal: MLP arena overrun"); delete net; return MZ_ENOMEM; }
-      net->tc_smem = 3 * 16384 + 65536 + (size_t)kTcSlots * kTcSlotBytes + 256 + (size_t)4 * P * 4;
+      net->tc_smem = tc_smem_base;
       q.tab_in_smem = net->tc_smem + (size_t)A * (P + 4) * 4 <= 227 * 1024 ? 1 : 0;
       if (q.tab_in_smem) net->tc_smem += (size_t)A * (P + 4) * 4;
       int dev = 0;
@@ -1274,6 +1480,7 @@ int mlp_create(const mz_net_config& c, const float* const* w, int nw, void* aren
       cudaDeviceGetAttribute(&net->num_sms, cudaDevAttrMultiProcessorCount, dev);
       const int smem_cap = 227 * 1024;
       MZ_CUDA(cudaFuncSetAttribute(mlp_tc_kernel<false, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_cap));
+      MZ_CUDA(cudaFuncSetAttribute(mlp_tc_kernel<false, 4, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_cap));
       MZ_CUDA(cudaFuncSetAttribute(mlp_tc_kernel<true, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_cap));
       MZ_CUDA(cudaFuncSetAttribute(mlp_tc_kernel<true, 12>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_cap));
       MZ_CUDA(cudaFuncSetAttribute(mlp_search32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_cap));

@@ -42,11 +42,11 @@ struct NetImpl {
   virtual int recurrent(int batch, const void* hidden_in, const int32_t* src_index, const int32_t* action,
                         void* hidden_out, const int32_t* dst_index, float* reward, float* value, float* pi_probs,
                         cudaStream_t st) = 0;
-  // test aid (mz_net_debug_*): conv nets only
-  virtual int debug_capture_bytes(int, size_t*) { set_error("mz_net_debug_*: conv nets only"); return MZ_EINVAL; }
-  virtual int debug_capture(void*, size_t) { set_error("mz_net_debug_*: conv nets only"); return MZ_EINVAL; }
-  virtual int debug_tensor(int, mz_debug_tensor*, int32_t*) { set_error("mz_net_debug_*: conv nets only"); return MZ_EINVAL; }
-  virtual int debug_launch(int, mz_debug_launch*, int32_t*) { set_error("mz_net_debug_*: conv nets only"); return MZ_EINVAL; }
+  // test aid (mz_net_debug_*): every family implements it
+  virtual int debug_capture_bytes(int, size_t*) = 0;
+  virtual int debug_capture(void*, size_t) = 0;
+  virtual int debug_tensor(int, mz_debug_tensor*, int32_t*) = 0;
+  virtual int debug_launch(int, mz_debug_launch*, int32_t*) = 0;
 };
 
 int mlp_hidden_bytes(const mz_net_config& c, int32_t* bytes);

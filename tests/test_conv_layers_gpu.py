@@ -166,8 +166,22 @@ def head_ratio(Y, Fm, sd, prefix, kind, n_real):
     K = f.shape[1]
     logit = f @ w2.T + b2
     e = (math.ceil(K / 32) + 7) * U32 * (f.abs() @ w2.abs().T + b2.abs()) + df @ w2.abs().T
+    return transform_ratio(Y, logit, e, kind)
+
+
+def safe_ratio(err, bound):
+    """max err / bound, where a zero bound admits only a zero error."""
+    r = torch.where(bound > 0, err / bound.clamp_min(1e-300), torch.where(err > 0, math.inf, 0.0))
+    return float(r.max()) if r.numel() else 0.0
+
+
+def transform_ratio(Y, logit, e, kind, seq=False):
+    """Y: the engine's output (float64 [B] or [B, out]) of the output transform `kind` (0 identity, 1 support ->
+    scalar, 2 softmax) of fp32 logits known to within e (float64 [B, n], like logit).  seq: one thread sums the n
+    terms in order; else 32 lanes sum n / 32 each and a butterfly combines them (module docstring)."""
     if kind == 0:
-        return float(((Y.view(-1) - logit.view(-1)).abs() / e.view(-1)).max())
+        return safe_ratio((Y.view(-1) - logit.view(-1)).abs(), e.view(-1))
+    dev = logit.device
     n = logit.shape[1]
     lg = logit.detach().requires_grad_(True)
     if kind == 2:
@@ -181,7 +195,7 @@ def head_ratio(Y, Fm, sd, prefix, kind, n_real):
                         for j in range(n if kind == 2 else 1)], 1)          # [B, outputs, logits]
     bound = (Jabs * e.unsqueeze(1)).sum(2)
     spread = (logit - logit.amax(1, keepdim=True)).abs().amax(1, keepdim=True)
-    rel = U32 * (16 + n / 32 + 2 * spread)
+    rel = U32 * (16 + (2 * n if seq else n / 32) + 2 * spread)
     out = out.detach()
     if kind == 2:
         bound = bound + out * rel + 2.0 ** -148        # expf and the division round into fp32 subnormals (2^-149)
@@ -190,6 +204,8 @@ def head_ratio(Y, Fm, sd, prefix, kind, n_real):
         sup = torch.linspace(-hi, hi, n, dtype=torch.float64, device=dev)
         xs = (p * sup).sum(1)
         dx = rel.view(-1) * (p * sup.abs()).sum(1) + ulp32(xs)
+        if n % 2 == 0:            # support points -maxv + i * fp32(2 maxv / (n - 1)) are not integers
+            dx = dx + 4 * U32 * (hi + 1)
         a = 1 + 0.004 * (1.001 + xs.abs())
         z = a.sqrt() / 2 / 1e-3 - 500
         dsp = 2 * z.abs() * 0.004 / 2 / 1e-3 / 2 / a.sqrt()          # |d signed_parabolic / dx|
@@ -746,7 +762,8 @@ def test_debug_launch_record_matches_the_header():
 @pytest.mark.gpu
 def test_undersized_capture_buffer_fails_cleanly():
     """A capture buffer too small for a call: the call raises MemoryError and leaves nothing queued that points into
-    that buffer -- after capture is turned off, the next calls give the same bytes as a net that never captured."""
+    that buffer -- after capture is turned off, the next calls give the same bytes as a net that never captured.  For
+    a conv net and an MLP net."""
     import muzero_b200 as mz
     from muzero_b200 import _lib
     from oracle.network_oracle import randomize_batchnorm
@@ -784,3 +801,30 @@ def test_undersized_capture_buffer_fails_cleanly():
         outs.append([t.view(torch.uint8) for t in (hid, pi, v, hid2, r, pi2, v2)])
     for k, (a, b) in enumerate(zip(*outs)):
         assert torch.equal(a, b), k
+    # the same for an MLP net: its SIMT initial call and its tcgen05 recurrent call
+    torch.manual_seed(24)
+    m = mz.MuZeroMLPNet((4, 5), 2, 512, 31, 31, 64).cuda().eval()
+    mobs = torch.randn((B, 4, 5), device='cuda', generator=gen)
+    mact = torch.randint(0, 2, (B,), device='cuda', generator=gen).int()
+    ref = []
+    for capture in (True, False):
+        eh = m.engine(B)['handle']
+        if capture:
+            _lib.check(lib.mz_net_debug_capture_bytes(eh, B, C.byref(nb)))
+            small = torch.empty(nb.value // 8, dtype=torch.uint8, device='cuda')
+            base = (small.data_ptr() + 255) // 256 * 256
+            _lib.check(lib.mz_net_debug_capture(eh, base, small.numel() - 256))
+            with pytest.raises(MemoryError):
+                m.initial_inference_batch(mobs)
+            with pytest.raises(MemoryError):
+                m.recurrent_inference_batch(m.new_hidden(B), mact)
+            _lib.check(lib.mz_net_debug_capture(eh, None, 0))
+            del small
+            torch.cuda.synchronize()
+        hid, pi, v = m.initial_inference_batch(mobs)
+        hid2, r, pi2, v2 = m.recurrent_inference_batch(hid, mact)
+        torch.cuda.synchronize()
+        ref.append([t.view(torch.uint8) for t in (hid, pi, v, hid2, r, pi2, v2)])
+        m.release_engine()
+    for k, (a, b) in enumerate(zip(*ref)):
+        assert torch.equal(a, b), f'mlp output {k}'

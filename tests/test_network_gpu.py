@@ -38,12 +38,27 @@ def close_tc(got, ref, tol=TC_TOL, scale=None):
     assert np.isfinite(got).all() and err <= tol * scale, f'max err {err:.4g} > {tol * scale:.4g}'
 
 
+# random-init nets that reach the one-launch search kernel's two-chunk and global-action-table paths
+RANDOM_MLPS = {
+    'p512_a8': dict(input_shape=(4, 5), num_actions=8, num_planes=512, value_support_size=31, reward_support_size=31,
+                    hidden_dim=64),
+    'p256_a20': dict(input_shape=(4, 5), num_actions=20, num_planes=256, value_support_size=31,
+                     reward_support_size=31, hidden_dim=64),
+}
+
+
 def load_mlp(name):
     import muzero_b200 as mz
-    sd = {k: torch.from_numpy(v) for k, v in np.load(os.path.join(GOLDEN, f'ckpt_{name}.npz')).items()}
-    kw = MLPS[name]
-    net = mz.MuZeroMLPNet(**kw)
-    net.load_state_dict(sd)
+    if name in RANDOM_MLPS:
+        kw = RANDOM_MLPS[name]
+        torch.manual_seed(kw['num_planes'] + kw['num_actions'])
+        net = mz.MuZeroMLPNet(**kw)
+        sd = {k: v.detach().clone() for k, v in net.state_dict().items()}
+    else:
+        sd = {k: torch.from_numpy(v) for k, v in np.load(os.path.join(GOLDEN, f'ckpt_{name}.npz')).items()}
+        kw = MLPS[name]
+        net = mz.MuZeroMLPNet(**kw)
+        net.load_state_dict(sd)
     net = net.cuda().eval()
     orc_net = OracleNet('mlp', sd, kw['num_actions'], kw['value_support_size'], kw['reward_support_size'])
     return net, orc_net, kw
@@ -280,19 +295,20 @@ def test_fp16_networks_rarely_change_a_search():
 
 
 @pytest.mark.parametrize('name,B', [('tictactoe', 300), ('cartpole', 200), ('lunarlander', 130), ('tictactoe', 4096),
-                                    ('tictactoe', 4800)])
+                                    ('tictactoe', 4800), ('p512_a8', 200), ('p256_a20', 200)])
 @pytest.mark.parametrize('noise_mode', ['device', 'none'])
 def test_one_launch_search_kernel_equals_the_launch_chain(name, B, noise_mode):
     """mz_search_run's persistent kernels for the MLP nets -- one launch per search: 32 trees per CTA with a warp per
     tree (Tic-Tac-Toe up to 32 trees per SM), or 128 trees per CTA with a thread per tree (the other cases here, on
-    request) -- against the per-simulation launch chain (warp-per-tree / thread-per-tree tree kernels + one tcgen05
+    request; the random-init nets take the warp-per-tree kernel's two-chunk and global-action-table paths) -- against
+    the per-simulation launch chain (warp-per-tree / thread-per-tree tree kernels + one tcgen05
     launch per simulation), which the lock-step and replay tests pin to the oracle: trees, statistics, hidden states,
     RNG streams, policies and actions, byte for byte."""
     import muzero_b200 as mz
     from muzero_b200 import _lib
     net, _, kw = load_mlp(name)
-    cfg = {'tictactoe': mz.make_tictactoe_config, 'cartpole': mz.make_classic_config,
-           'lunarlander': mz.make_classic_config}[name](use_tensorboard=False)
+    cfg = {'tictactoe': mz.make_tictactoe_config, 'cartpole': mz.make_classic_config, 'lunarlander': mz.make_classic_config,
+           'p512_a8': mz.make_classic_config, 'p256_a20': mz.make_classic_config}[name](use_tensorboard=False)
     A = kw['num_actions']
     gen = np.random.RandomState(B + A)
     obs = gen.standard_normal((B,) + kw['input_shape']).astype(np.float32)
